@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the LBM time step (BASELINE.json metric: D3Q19 MLUP/s at 1/2/4/8 B200 and % of the HBM-bandwidth roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one LBM time step (stream_collide on every cell of the lattice, plus the halo exchange when N > 1).
 MLUP/s = cells of the GLOBAL lattice (solids included, halo layers excluded) x steps / seconds / 1e6, the reference's own definition
@@ -21,6 +21,10 @@ The JSON line carries, besides the contract keys: `roofline` (dominant kernel, a
 MEASURED_PEAKS.json), `cpu_baseline` (the reference's kernel text compiled for host threads -- oracle/_ref -- or the C oracle, on a bounded sample),
 `e2e` (the same steps driven through the host API one step at a time, each with a pinned-memory upload of that step's inflow boundary field
 and a read-back of a probe plane), `clocks`, `gpu_launches`.
+
+--dump-outputs DIR (N = 1): right after the K timed steps of every workload it measures, rho and u (and T on thermal workloads) as the host API returns
+them, at a fixed, seeded sample of cells, go to DIR/<workload>_<field>.npy (float32; u is (3, cells)). The inputs are seeded, so two builds run with the
+same arguments can be compared file for file.
 """
 import argparse
 import json
@@ -280,7 +284,13 @@ def main():
     ap.add_argument("--traffic", default="auto", choices=["auto", "live", "file", "off"],
                     help="roofline.traffic: re-run one step under ncu (live), read the committed capture (file), auto = live when ncu is on PATH")
     ap.add_argument("--traffic-child", action="store_true", help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="N=1: after the timed steps of each workload, write rho / u (/ T) at a fixed, seeded sample of cells to DIR/<workload>_<field>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.gpus != 1):
+        ap.error("--dump-outputs writes what the GPU arm computes on one GPU (--impl b200 --gpus 1)")
     args.warmup = max(args.warmup, 3)
     args.also_default = args.also is None
     if args.also is None:
@@ -380,6 +390,37 @@ def build_domain(Domain, cases, workload, arith, device, D=(1, 1, 1), O=(0, 0, 0
     return d
 
 
+DUMP_BYTES = 64_000_000  # all .npy data of one --dump-outputs run together
+
+
+def dump_cells(N, workloads):
+    """Local cells whose fields --dump-outputs writes: a sorted sample drawn with a fixed seed (every cell of a lattice no larger than the sample), sized
+    so that `workloads` dumps of rho + u + T (20 bytes per cell) stay within DUMP_BYTES."""
+    count = 1 << 20
+    while count * 20 * workloads > DUMP_BYTES and count > 1:
+        count //= 2
+    if N <= count:
+        return np.arange(N, dtype=np.uint64)
+    return np.sort(np.random.default_rng(2024).choice(N, count, replace=False)).astype(np.uint64)
+
+
+def dump_outputs(d, CellSet, A, workload, features, out_dir, workloads):
+    """--dump-outputs: what a caller of the host API reads after the steps that ran -- rho / u (/ T), with update_fields first where the step does not
+    store them (no UPDATE_FIELDS) -- at the cells of dump_cells(), as float32 DIR/<workload>_<field>.npy; u is (3, cells)."""
+    if not features & F_UF:
+        d.enqueue_update_fields()
+    cs = CellSet(d, dump_cells(d.N, workloads))
+    fields = [("rho", A.FIELD_RHO, 1), ("u", A.FIELD_U, 3)] + ([("T", A.FIELD_T, 1)] if features & F_TEMPERATURE else [])
+    out = {name: np.empty(comps * cs.count, np.float32) for name, _, comps in fields}
+    for name, field, _ in fields:
+        cs.download(field, out[name])
+    d.finish_queue()
+    cs.close()
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, f"{workload}_{name}.npy"), a.reshape(3, cs.count) if name == "u" else a)
+
+
 def bench_single(args, workload, arith, A, cases, Domain, CellSet, pinned_empty, peak, peak_src, headline):
     case, shape, precision, features, fset, nu, desc = WORKLOADS[workload]
     Nx, Ny, Nz = shape
@@ -398,9 +439,11 @@ def bench_single(args, workload, arith, A, cases, Domain, CellSet, pinned_empty,
         launches0 = d.launch_count()
         d.timer_begin(); d.run_steps(K); ms = d.timer_end()
         launches = d.launch_count() - launches0
+        clocks = clk.stop()
+        if args.dump_outputs:
+            dump_outputs(d, CellSet, A, workload, features, args.dump_outputs, 1 + len([w for w in args.also.split(",") if w]))
         # ---- roofline pass: the same K steps with an event pair around every main-kernel launch
         d.kernel_timing(True); d.run_steps(K); kms, kn = d.kernel_timing_read(); d.kernel_timing(False)
-        clocks = clk.stop()
         mlups = N * K / ms / 1e3
         # the step IS one launch of the step kernel (plus a 4-byte memset node for its strip counter): its average duration over the timed region is ms / K.
         # The second pass brackets every launch with its own event pair; that serialises the launches (no back-to-back overlap of tail and head) and is

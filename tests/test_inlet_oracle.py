@@ -26,9 +26,7 @@ def test_oracle_reproduces_the_reference_interpolators(k):
     hd = IO.knn_hd_eval(P, U, pos, z)
     want = GOLD[f"hd_{k}"][::STRIDE]
     assert _ulp_close(hd, want), f"{int((hd != want).any(axis=1).sum())} of {len(pos)} velocities differ by more than one unit in the last place"
-    # on the machine the fixture was made on the C library's exp is the same function: bit for bit. Elsewhere a weight may differ in its last bit.
-    if os.path.isdir("/root/reference"):
-        assert np.array_equal(hd, want)
+    assert np.array_equal(hd, want), f"{int((hd != want).any(axis=1).sum())} of {len(pos)} velocities differ in their last bit (a C library whose exp differs from the fixture's)"
     assert np.count_nonzero(want) > len(pos)
 
 
