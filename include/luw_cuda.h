@@ -210,6 +210,32 @@ int luw_stats_download(luw_stats* st, float* host_mean_u, float* host_m2_u, floa
 int luw_stats_download_temperature(luw_stats* st, float* host_mean_T);
 int luw_stats_destroy(luw_stats* st);
 
+/* Pedestrian-level wind statistics. Extends the averaging window above (FX/setup.cpp:4411-4542) and what write_avg_vtk derives from it (TKE / TI from mean and
+ * M2 per component, FX/setup.cpp:2513-2683) with quantities that cannot be rebuilt from those accumulators; the reference has NO counterpart (it would read the whole
+ * u field back per sample and loop on the host). The accumulators cover a fixed list of cells only -- typically a few layers at fixed heights above the local
+ * ground or roof -- so they stay small on any lattice.
+ * luw_column_ground: host_ground[y*Nx + x] over the local Nx*Ny columns = GLOBAL z (Oz + z) of the lowest owned cell (z halo layers skipped) whose flags are not
+ *   solid ((flags & 0x03) != TYPE_S), 0xFFFFFFFF if the column has none; read from the device flags; synchronous. Over a decomposition in z the ground of a global
+ *   column is the minimum over its blocks.
+ * luw_wind_stats_create: host_cell_index[count] = local dense cell indices (like luw_cellset_create); host_thresholds: speeds in lattice units (>= 0, at most
+ *   LUW_WIND_MAX_THRESHOLDS). Accumulators zero-filled; count may be 0.
+ * luw_wind_stats_accumulate: ++n, inv_n = 1/n; per listed cell the Welford update of the means of ux, uy, uz and of their co-moments
+ *   C_ab += (x_a - mean_a,old)*(x_b - mean_b,new), ab = uu vv ww uv uw vw (C_ab / n is the covariance, u'w' = C_uw / n), Welford mean / M2 of the speed
+ *   s = |u|, its running maximum (from 0) and, per threshold, the number of samples with s > threshold. Every product and sum is rounded separately, so the
+ *   means and C_uu / C_vv / C_ww equal luw_stats' mean_u / m2_u for the same cells bit for bit. Stream-ordered on the domain's stream, no host synchronisation;
+ *   the caller runs luw_update_fields first when the domain does not store u every step, like for luw_stats_accumulate.
+ * luw_wind_stats_download: SoA over the list [j*count + k]: mean_u 3*count (u v w), comoment 6*count (uu vv ww uv uw vw), mean_speed / m2_speed / max_speed count
+ *   each, exceed threshold_count*count; any pointer may be NULL; synchronous. */
+#define LUW_WIND_MAX_THRESHOLDS 8
+typedef struct luw_wind_stats luw_wind_stats;
+int luw_column_ground(luw_domain* dom, uint32_t* host_ground);
+int luw_wind_stats_create(luw_domain* dom, uint64_t count, const uint64_t* host_cell_index, uint32_t threshold_count, const float* host_thresholds, luw_wind_stats** out);
+int luw_wind_stats_accumulate(luw_wind_stats* st);
+int luw_wind_stats_reset(luw_wind_stats* st);
+int luw_wind_stats_download(luw_wind_stats* st, float* host_mean_u, float* host_comoment, float* host_mean_speed, float* host_m2_speed, float* host_max_speed,
+	uint32_t* host_exceed, uint64_t* samples);
+int luw_wind_stats_destroy(luw_wind_stats* st);
+
 /* page-locked host memory for the mirrors (the reference's Memory<T> owns pageable new[] buffers, FX/opencl.hpp:354) */
 int luw_host_alloc(void** host_ptr, uint64_t bytes);
 int luw_host_free(void* host_ptr);

@@ -80,6 +80,12 @@ EXPORTS = {  # name -> argtypes; every symbol include/luw_cuda.h declares
     "luw_stats_download": [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
     "luw_stats_download_temperature": [C.c_void_p, C.c_void_p],
     "luw_stats_destroy": [C.c_void_p],
+    "luw_column_ground": [C.c_void_p, C.c_void_p],
+    "luw_wind_stats_create": [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.c_void_p, C.POINTER(C.c_void_p)],
+    "luw_wind_stats_accumulate": [C.c_void_p],
+    "luw_wind_stats_reset": [C.c_void_p],
+    "luw_wind_stats_download": [C.c_void_p] + [C.c_void_p] * 6 + [C.POINTER(C.c_uint64)],
+    "luw_wind_stats_destroy": [C.c_void_p],
     "luw_host_alloc": [C.POINTER(C.c_void_p), C.c_uint64],
     "luw_host_free": [C.c_void_p],
     "luw_sync": [C.c_void_p],

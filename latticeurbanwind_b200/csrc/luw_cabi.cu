@@ -3,6 +3,7 @@
 #include "../../include/luw_cuda.h"
 #include "lbm_launch.h"
 #include "lbm_inlet.cuh"
+#include "lbm_wind_stats.cuh"
 #include "vox_bins.h"
 
 #include <cmath>
@@ -87,6 +88,14 @@ struct luw_stats {
 	uint64_t count;
 	float* mean_u; float* m2_u; float* mean_rho; // device, pitched like u / rho: [c*c.N + n]
 	float* mean_T; // LUW_TEMPERATURE domains: running mean of T (avg_T, FX/setup.cpp:4449-4451, 4481-4486); nullptr otherwise
+};
+struct luw_wind_stats {
+	luw_domain* dom;
+	uint64_t count, samples;
+	uint64_t* cell; // device indices of the listed cells
+	float* acc; // [j*count + k], j < luw::WIND_FLOAT_ACCUMULATORS (lbm_wind_stats.cuh)
+	uint32_t* exceed; // [j*count + k], j < thr.count
+	luw::WindThresholds thr;
 };
 struct luw_vk_inlet {
 	luw_domain* dom;
@@ -1125,6 +1134,116 @@ int luw_stats_destroy(luw_stats* st) {
 	DeviceGuard guard(st->dom->p.device);
 	cudaStreamSynchronize(st->dom->stream);
 	cudaFree(st->mean_u); cudaFree(st->m2_u); cudaFree(st->mean_rho); cudaFree(st->mean_T);
+	delete st;
+	return LUW_OK;
+}
+
+static int require_device() { // entry points that may be reached before any domain exists: no device -> LUW_ERR_NO_DEVICE, whatever the other arguments
+	int n = 0;
+	const cudaError_t e = cudaGetDeviceCount(&n);
+	if(e!=cudaSuccess) return cuda_fail(e, "cudaGetDeviceCount");
+	return n>0 ? LUW_OK : fail(LUW_ERR_NO_DEVICE, "no CUDA device");
+}
+int luw_column_ground(luw_domain* d, uint32_t* host_ground) {
+	if(const int rc = require_device()) return rc;
+	if(!d||!host_ground) return fail(LUW_ERR_INVALID, "null argument");
+	const luw::DomainConst& c = d->c;
+	const uint32_t Hz = c.Dz>1u ? 1u : 0u;
+	DeviceGuard guard(d->p.device);
+	DeviceBuffers mem;
+	uint32_t* g = nullptr;
+	CU(mem.get(&g, (uint64_t)c.Nx*c.Ny));
+	luw::k_column_ground<<<dim3((c.Nx+255u)/256u, c.Ny), 256, 0, d->stream>>>(c.Nx, c.Px, c.Ny, Hz, c.Nz-Hz, c.Oz, c.flags, g);
+	CU(cudaGetLastError());
+	d->launches++;
+	CU(cudaMemcpyAsync(host_ground, g, (uint64_t)c.Nx*c.Ny*4ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	return LUW_OK;
+}
+int luw_wind_stats_create(luw_domain* d, uint64_t count, const uint64_t* host_cell_index, uint32_t threshold_count, const float* host_thresholds, luw_wind_stats** out) {
+	if(const int rc = require_device()) return rc;
+	if(!d||!out||(count>0ull&&!host_cell_index)||(threshold_count>0u&&!host_thresholds)) return fail(LUW_ERR_INVALID, "null argument");
+	*out = nullptr;
+	if(threshold_count>luw::WIND_MAX_THRESHOLDS) return fail(LUW_ERR_INVALID, "at most LUW_WIND_MAX_THRESHOLDS thresholds");
+	luw::WindThresholds thr;
+	memset(&thr, 0, sizeof(thr));
+	thr.count = threshold_count;
+	for(uint32_t j=0u; j<threshold_count; j++) {
+		if(!(host_thresholds[j]>=0.0f)) return fail(LUW_ERR_INVALID, "thresholds must be non-negative numbers");
+		thr.t[j] = host_thresholds[j];
+	}
+	for(uint64_t k=0ull; k<count; k++) if(host_cell_index[k]>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
+	std::vector<uint64_t> cd(count);
+	for(uint64_t k=0ull; k<count; k++) cd[k] = device_index(d->c, host_cell_index[k]);
+	DeviceGuard guard(d->p.device);
+	luw_wind_stats* st = new(std::nothrow) luw_wind_stats();
+	if(!st) return fail(LUW_ERR_OOM, "host allocation failed");
+	memset(st, 0, sizeof(*st));
+	st->dom = d; st->count = count; st->thr = thr;
+	int rc = LUW_OK;
+	if(count>0ull) {
+		rc = dev_alloc(d, &st->cell, count);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->acc, (uint64_t)luw::WIND_FLOAT_ACCUMULATORS*count);
+		if(rc==LUW_OK&&threshold_count>0u) rc = dev_alloc(d, &st->exceed, (uint64_t)threshold_count*count);
+		if(rc==LUW_OK) {
+			cudaError_t e = cudaMemcpyAsync(st->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
+			if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // the host list may be freed by the caller afterwards
+			if(e!=cudaSuccess) rc = cuda_fail(e, "upload cell list");
+		}
+	}
+	if(rc==LUW_OK) rc = luw_wind_stats_reset(st);
+	if(rc!=LUW_OK) { const std::string keep = g_error; luw_wind_stats_destroy(st); g_error = keep; return rc; }
+	*out = st;
+	return LUW_OK;
+}
+int luw_wind_stats_reset(luw_wind_stats* st) {
+	if(!st) return fail(LUW_ERR_INVALID, "null statistics object");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	if(st->count>0ull) { // every accumulator starts at 0, the running maximum of the speed included (|u| >= 0)
+		CU(cudaMemsetAsync(st->acc, 0, (uint64_t)luw::WIND_FLOAT_ACCUMULATORS*st->count*4ull, d->stream));
+		if(st->exceed) CU(cudaMemsetAsync(st->exceed, 0, (uint64_t)st->thr.count*st->count*4ull, d->stream));
+	}
+	st->samples = 0ull;
+	return LUW_OK;
+}
+int luw_wind_stats_accumulate(luw_wind_stats* st) {
+	if(!st) return fail(LUW_ERR_INVALID, "null statistics object");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	st->samples++;
+	const float inv_n = 1.0f/(float)st->samples;
+	if(st->count==0ull) return LUW_OK;
+	const uint64_t want = (st->count+255ull)/256ull, cap = d->sm_count>0 ? 8ull*(uint64_t)d->sm_count : 1184ull;
+	luw::k_wind_stats_accumulate<<<(unsigned)(want<cap ? want : cap), 256, 0, d->stream>>>(st->count, d->c.N, inv_n, d->c.u, st->cell, st->thr, st->acc, st->exceed);
+	CU(cudaGetLastError());
+	d->launches++;
+	return LUW_OK;
+}
+int luw_wind_stats_download(luw_wind_stats* st, float* host_mean_u, float* host_comoment, float* host_mean_speed, float* host_m2_speed, float* host_max_speed,
+	uint32_t* host_exceed, uint64_t* samples) {
+	if(!st) return fail(LUW_ERR_INVALID, "null statistics object");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	const uint64_t K = st->count;
+	if(K>0ull) {
+		const auto get = [&](void* host, const void* dev, const uint64_t bytes) { return host ? cudaMemcpyAsync(host, dev, bytes, cudaMemcpyDeviceToHost, d->stream) : cudaSuccess; };
+		CU(get(host_mean_u, st->acc, 3ull*K*4ull));
+		CU(get(host_comoment, st->acc+3ull*K, 6ull*K*4ull));
+		CU(get(host_mean_speed, st->acc+9ull*K, K*4ull));
+		CU(get(host_m2_speed, st->acc+10ull*K, K*4ull));
+		CU(get(host_max_speed, st->acc+11ull*K, K*4ull));
+		if(st->exceed) CU(get(host_exceed, st->exceed, (uint64_t)st->thr.count*K*4ull));
+	}
+	CU(cudaStreamSynchronize(d->stream));
+	if(samples) *samples = st->samples;
+	return LUW_OK;
+}
+int luw_wind_stats_destroy(luw_wind_stats* st) {
+	if(!st) return LUW_OK;
+	DeviceGuard guard(st->dom->p.device);
+	cudaStreamSynchronize(st->dom->stream);
+	cudaFree(st->cell); cudaFree(st->acc); cudaFree(st->exceed);
 	delete st;
 	return LUW_OK;
 }

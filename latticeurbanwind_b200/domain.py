@@ -237,6 +237,13 @@ class Domain:
         A.check(A.lib().luw_kernel_timing_read(self._h, C.byref(ms), C.byref(n)))
         return ms.value, n.value
 
+    def column_ground(self):
+        """-> uint32 [Ny, Nx]: global z of the lowest owned non-solid cell of every local column, 0xFFFFFFFF where there is none (luw_column_ground;
+        read from the device flags, so no host mirror is touched)."""
+        g = np.empty((self.Ny, self.Nx), np.uint32)
+        A.check(A.lib().luw_column_ground(self._h, _ptr(g)))
+        return g
+
     def device_bytes(self):
         n = C.c_uint64()
         A.check(A.lib().luw_domain_bytes(self._h, C.byref(n)))
@@ -320,6 +327,40 @@ class Stats:
     def close(self):
         if self._h:
             A.lib().luw_stats_destroy(self._h)
+            self._h = C.c_void_p()
+
+
+class WindStats:
+    """Pedestrian-level wind statistics of a fixed list of local cells (luw_wind_stats_*): running means and co-moments of u, mean / M2 / peak of the speed
+    and threshold exceedance counts, accumulated on the device once per sample. `thresholds`: speeds in lattice units (at most 8)."""
+
+    def __init__(self, domain, cells, thresholds=()):
+        self.domain = domain
+        self.cells = np.ascontiguousarray(cells, np.uint64)
+        self.count = int(self.cells.size)
+        self.thresholds = np.ascontiguousarray(thresholds, np.float32)
+        self._h = C.c_void_p()
+        A.check(A.lib().luw_wind_stats_create(domain._h, self.count, _ptr(self.cells), int(self.thresholds.size), _ptr(self.thresholds), C.byref(self._h)))
+
+    def accumulate(self):
+        A.check(A.lib().luw_wind_stats_accumulate(self._h))
+
+    def reset(self):
+        A.check(A.lib().luw_wind_stats_reset(self._h))
+
+    def download(self):
+        """-> (mean_u[3, count], comoment[6, count] (uu vv ww uv uw vw), mean_speed[count], m2_speed[count], max_speed[count], exceed[thresholds, count], samples)"""
+        K, T = self.count, int(self.thresholds.size)
+        mean_u, com = np.empty((3, K), np.float32), np.empty((6, K), np.float32)
+        ms, m2, mx = np.empty(K, np.float32), np.empty(K, np.float32), np.empty(K, np.float32)
+        ex = np.empty((T, K), np.uint32)
+        n = C.c_uint64()
+        A.check(A.lib().luw_wind_stats_download(self._h, _ptr(mean_u), _ptr(com), _ptr(ms), _ptr(m2), _ptr(mx), _ptr(ex), C.byref(n)))
+        return mean_u, com, ms, m2, mx, ex, n.value
+
+    def close(self):
+        if self._h:
+            A.lib().luw_wind_stats_destroy(self._h)
             self._h = C.c_void_p()
 
 

@@ -5,9 +5,22 @@
 //   in.bin : flags[N] u8, rho[N] f32, u[3N] f32 (global images, n = x+(y+z*Ny)*Nx);  out.bin : rho[N] f32, u[3N] f32
 //   LUW_CASE_TRIANGLES=<file> (u32 n, pmin[3], pmax[3], p0[3n], p1[3n], p2[3n] f32, lattice coordinates): the geometry is voxelised on the device first, through
 //   LBM::voxelize_triangles_on_device like FX/setup.cpp:4084-4125 does with the STL, the flags of in.bin are OR-ed on top, and out.bin ends with flags[N] u8
+//   LUW_CASE_WIND=h0,h1,... (heights in cells) with LUW_CASE_WIND_THR=t0,t1,... and LUW_CASE_WIND_OUT=<file>: LBM_WindStatistics over the same sampling window as
+//   LUW_CASE_STATS; the file gets samples u64, mean_u[3M], comoment[6M], mean_speed[M], m2_speed[M], max_speed[M] f32, exceed[T*M] u32, valid[M] u8, ground[Nx*Ny] u32
 //   with LUW_TEMPERATURE in `features`: in.bin carries T[N] f32 after u, out.bin ends with T[N] f32; alpha / beta of the LBM constructor from LUW_CASE_ALPHA / LUW_CASE_BETA
 #include "lbm.hpp"
 #include <fstream>
+#include <sstream>
+
+template<typename T> static std::vector<T> env_list(const char* name) { // comma-separated numbers, empty if unset
+	std::vector<T> v;
+	const char* e = getenv(name);
+	if(!e) return v;
+	std::stringstream ss(e);
+	std::string item;
+	while(std::getline(ss, item, ',')) if(!item.empty()) v.push_back((T)atof(item.c_str()));
+	return v;
+}
 
 int main(int argc, char** argv) {
 	if(argc!=26) { fprintf(stderr, "usage: see host_case.cpp\n"); return 2; }
@@ -60,8 +73,20 @@ int main(int argc, char** argv) {
 	lbm.run(0ull); // initialise only (FX/setup.cpp:4852)
 	const ulong samples = getenv("LUW_CASE_STATS") ? (ulong)atoll(getenv("LUW_CASE_STATS")) : 0ull; // averaging window over the last `samples` steps (FX/setup.cpp:4510-4542)
 	LBM_Statistics* stats = samples>0ull ? new LBM_Statistics(lbm) : nullptr;
+	const char* wind_out = getenv("LUW_CASE_WIND_OUT");
+	LBM_WindStatistics* wind = wind_out ? new LBM_WindStatistics(lbm, env_list<uint>("LUW_CASE_WIND"), env_list<float>("LUW_CASE_WIND_THR")) : nullptr;
 	lbm.run(steps-(samples<steps ? samples : steps));
-	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); stats->accumulate(); }
+	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); stats->accumulate(); if(wind) wind->accumulate(); }
+	if(wind) {
+		std::vector<float> mean_u, comoment, mean_speed, m2_speed, max_speed; std::vector<uint> exceed; std::vector<uchar> valid;
+		const uint64_t count = (uint64_t)wind->download(mean_u, comoment, mean_speed, m2_speed, max_speed, exceed, valid);
+		std::ofstream wf(wind_out, std::ios::binary);
+		wf.write((const char*)&count, 8);
+		for(const std::vector<float>* v : { &mean_u, &comoment, &mean_speed, &m2_speed, &max_speed }) wf.write((const char*)v->data(), (std::streamsize)(4u*v->size()));
+		wf.write((const char*)exceed.data(), (std::streamsize)(4u*exceed.size())); wf.write((const char*)valid.data(), (std::streamsize)valid.size());
+		wf.write((const char*)wind->ground.data(), (std::streamsize)(4u*wind->ground.size()));
+		delete wind;
+	}
 	lbm.rho.read_from_device(); lbm.u.read_from_device();
 	for(ulong n=0ull; n<N; n++) { rho[n] = lbm.rho[n]; u[n] = lbm.u.x[n]; u[N+n] = lbm.u.y[n]; u[2ull*N+n] = lbm.u.z[n]; }
 	std::ofstream out(out_path, std::ios::binary);

@@ -15,6 +15,7 @@
 #pragma once
 #include "../../include/luw_cuda.h"
 
+#include <algorithm>
 #include <cmath>
 #include <cstdint>
 #include <cstdio>
@@ -23,6 +24,7 @@
 #include <string>
 #include <vector>
 #include <chrono>
+#include <utility>
 
 #ifndef LUW_USE_REFERENCE_UTILITIES
 typedef unsigned int uint;
@@ -538,5 +540,97 @@ public:
 				avg_T[lbm->index((uint)((int)x+dom->get_Ox()), (uint)((int)y+dom->get_Oy()), (uint)((int)z+dom->get_Oz()))] = mt[l];
 			}
 		}
+	}
+};
+
+// ---------------------------------------------------------------------------------------------------------------- pedestrian-level wind statistics (no reference counterpart)
+// Surface-following layers: for every height h_k (cells) above the local ground or roof, the running mean and co-moments of u, mean / M2 / peak of the speed |u| and
+// how many samples exceed each threshold (lattice units, at most LUW_WIND_MAX_THRESHOLDS), accumulated on the device per sample (luw_wind_stats_*). Construct it once the
+// flags are on the device (after run(0)). The ground of a global column is the lowest non-solid cell over the domains stacked in z (luw_column_ground, minimum per
+// column); each domain lists its owned plain-fluid cells ((flags & 0x03) == 0) at ground + h_k, read through a cell set, so no host mirror is materialised.
+// download() stitches the lists into global layer-major arrays [k][y][x] (Nx*Ny*K per quantity; components / thresholds outermost); slots that are not listed
+// (solid, TYPE_E, above the lattice) are NaN in the float fields, 0 in the counters and 0 in `valid`. File output (VTK, NetCDF) is the caller's business.
+class LBM_WindStatistics {
+private:
+	LBM* lbm = nullptr;
+	std::vector<uint> heights;
+	uint thresholds = 0u;
+	std::vector<luw_wind_stats*> st;
+	std::vector<std::vector<ulong>> slots; // per domain: global slot of every listed cell
+public:
+	std::vector<uint> ground; // [y*Nx + x] over the global columns: global z of the lowest non-solid cell, 0xFFFFFFFF if none
+	LBM_WindStatistics(LBM& lbm_, std::vector<uint> heights_in_cells, std::vector<float> thresholds_lattice) : lbm(&lbm_), heights(std::move(heights_in_cells)), thresholds((uint)thresholds_lattice.size()) {
+		const uint Nx = lbm->get_Nx(), Ny = lbm->get_Ny(), Nz = lbm->get_Nz(), Hx = lbm->get_Dx()>1u, Hy = lbm->get_Dy()>1u, Hz = lbm->get_Dz()>1u;
+		ground.assign((size_t)Nx*Ny, 0xFFFFFFFFu);
+		for(uint d=0u; d<lbm->get_D(); d++) { // lowest non-solid cell over the blocks stacked in z
+			const LBM_Domain* dom = lbm->lbm_domain[d];
+			std::vector<uint32_t> g((size_t)dom->get_Nx()*dom->get_Ny());
+			luw_check(luw_column_ground(dom->get_handle(), g.data()));
+			for(uint y=Hy; y<dom->get_Ny()-Hy; y++) for(uint x=Hx; x<dom->get_Nx()-Hx; x++) {
+				uint& G = ground[(size_t)(y+dom->get_Oy())*Nx+(size_t)(x+dom->get_Ox())];
+				G = std::min(G, (uint)g[(size_t)y*dom->get_Nx()+x]);
+			}
+		}
+		for(uint d=0u; d<lbm->get_D(); d++) {
+			const LBM_Domain* dom = lbm->lbm_domain[d];
+			const ulong lNx = dom->get_Nx(), lNy = dom->get_Ny();
+			std::vector<uint64_t> cand; std::vector<ulong> cand_slot;
+			for(size_t k=0u; k<heights.size(); k++) for(uint y=Hy; y<dom->get_Ny()-Hy; y++) for(uint x=Hx; x<dom->get_Nx()-Hx; x++) {
+				const ulong gx = (ulong)(x+dom->get_Ox()), gy = (ulong)(y+dom->get_Oy());
+				const uint G = ground[gy*Nx+gx];
+				if(G==0xFFFFFFFFu||(ulong)G+heights[k]>=(ulong)Nz) continue;
+				const long lz = (long)G+(long)heights[k]-(long)dom->get_Oz();
+				if(lz<(long)Hz||lz>=(long)(dom->get_Nz()-Hz)) continue; // owned by another block
+				cand.push_back((uint64_t)x+((uint64_t)y+(uint64_t)lz*lNy)*lNx);
+				cand_slot.push_back((ulong)k*Nx*Ny+gy*Nx+gx);
+			}
+			std::vector<uint8_t> fl(cand.size());
+			if(!cand.empty()) { // the candidates' flags, gathered on the device
+				luw_cellset* cs = nullptr;
+				luw_check(luw_cellset_create(dom->get_handle(), cand.size(), cand.data(), &cs));
+				luw_check(luw_cellset_download(cs, LUW_FIELD_FLAGS, fl.data()));
+				luw_check(luw_sync(dom->get_handle()));
+				luw_check(luw_cellset_destroy(cs));
+			}
+			std::vector<uint64_t> cells; std::vector<ulong> sl;
+			for(size_t i=0u; i<cand.size(); i++) if((fl[i]&0x03u)==0u) { cells.push_back(cand[i]); sl.push_back(cand_slot[i]); }
+			luw_wind_stats* h = nullptr;
+			luw_check(luw_wind_stats_create(dom->get_handle(), cells.size(), cells.data(), thresholds, thresholds_lattice.data(), &h));
+			st.push_back(h); slots.push_back(std::move(sl));
+		}
+	}
+	~LBM_WindStatistics() { for(luw_wind_stats* h : st) luw_wind_stats_destroy(h); }
+	LBM_WindStatistics(const LBM_WindStatistics&) = delete;
+	LBM_WindStatistics& operator=(const LBM_WindStatistics&) = delete;
+	void accumulate() { // like LBM_Statistics::accumulate: update_fields first when rho / u are not stored every step
+		for(uint d=0u; d<lbm->get_D(); d++) lbm->lbm_domain[d]->enqueue_update_fields();
+		for(uint d=0u; d<lbm->get_D(); d++) luw_check(luw_wind_stats_accumulate(st[d]));
+	}
+	void reset() { for(luw_wind_stats* h : st) luw_check(luw_wind_stats_reset(h)); }
+	// mean_u[c*M + m] (c = u v w), comoment[j*M + m] (j = uu vv ww uv uw vw), mean / M2 / max speed[m], exceed[j*M + m] (j < thresholds), valid[m]; m = k*Nx*Ny + y*Nx + x,
+	// M = K*Nx*Ny. Returns the sample count.
+	ulong download(std::vector<float>& mean_u, std::vector<float>& comoment, std::vector<float>& mean_speed, std::vector<float>& m2_speed, std::vector<float>& max_speed,
+		std::vector<uint>& exceed, std::vector<uchar>& valid) {
+		const ulong M = (ulong)heights.size()*lbm->get_Nx()*lbm->get_Ny();
+		const float nan = std::nanf("");
+		mean_u.assign(3ull*M, nan); comoment.assign(6ull*M, nan); mean_speed.assign(M, nan); m2_speed.assign(M, nan); max_speed.assign(M, nan);
+		exceed.assign((ulong)thresholds*M, 0u); valid.assign(M, (uchar)0);
+		uint64_t samples = 0ull;
+		for(uint d=0u; d<lbm->get_D(); d++) {
+			const std::vector<ulong>& sl = slots[d];
+			const ulong K = sl.size();
+			std::vector<float> mu(3ull*K), cm(6ull*K), ms(K), m2(K), mx(K);
+			std::vector<uint32_t> ex((ulong)thresholds*K);
+			luw_check(luw_wind_stats_download(st[d], mu.data(), cm.data(), ms.data(), m2.data(), mx.data(), ex.data(), &samples));
+			for(ulong i=0ull; i<K; i++) {
+				const ulong m = sl[i];
+				for(ulong c=0ull; c<3ull; c++) mean_u[c*M+m] = mu[c*K+i];
+				for(ulong j=0ull; j<6ull; j++) comoment[j*M+m] = cm[j*K+i];
+				mean_speed[m] = ms[i]; m2_speed[m] = m2[i]; max_speed[m] = mx[i];
+				for(ulong j=0ull; j<thresholds; j++) exceed[j*M+m] = ex[j*K+i];
+				valid[m] = 1u;
+			}
+		}
+		return (ulong)samples;
 	}
 };

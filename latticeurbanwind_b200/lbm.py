@@ -17,7 +17,7 @@ import numpy as np
 
 from . import _cabi as A
 from . import cases
-from .domain import Domain
+from .domain import CellSet, Domain, WindStats
 
 AXES = (0, 1, 2)
 
@@ -189,6 +189,92 @@ class LBM(_Base):
     def close(self):
         for dom in self.domains:
             dom.close()
+
+
+def wind_layer_cells(dom, O, Ng, D, ground, heights):
+    """The cells of one domain that pedestrian-level statistics cover: for every height h_k (cells), the OWNED cells at global z = ground + h_k whose flags are
+    plain fluid ((flags & 0x03) == 0: no TYPE_S, no TYPE_E); cells above the lattice are left out. ground: uint32 [Ng_y, Ng_x], global z of the lowest non-solid
+    cell per global column (0xFFFFFFFF: none). The flags are gathered from the device at the candidate cells (a cell set), so no host mirror is touched.
+    Returns (local dense cell indices, slots), slots[i] = k*Ng_x*Ng_y + y*Ng_x + x of the global layer-major arrays, in that order."""
+    H = tuple(1 if d > 1 else 0 for d in D)
+    xs, ys = np.arange(H[0], dom.Nx - H[0]), np.arange(H[1], dom.Ny - H[1])
+    gx, gy = xs + O[0], ys + O[1]  # owned cells never wrap
+    g = ground[np.ix_(gy, gx)].astype(np.int64)
+    cells, slots = [], []
+    for k, h in enumerate(heights):
+        zg = g + int(h)
+        lz = zg - O[2]
+        yy, xx = np.nonzero((g != 0xFFFFFFFF) & (zg < Ng[2]) & (lz >= H[2]) & (lz < dom.Nz - H[2]))
+        cells.append(xs[xx] + (ys[yy] + lz[yy, xx] * dom.Ny) * dom.Nx)
+        slots.append(k * Ng[0] * Ng[1] + gy[yy] * Ng[0] + gx[xx])
+    cells, slots = np.concatenate(cells).astype(np.uint64), np.concatenate(slots).astype(np.int64)
+    fl = np.zeros(cells.size, np.uint8)
+    if cells.size:
+        cs = CellSet(dom, cells)
+        cs.download(A.FIELD_FLAGS, fl)
+        dom.finish_queue()
+        cs.close()
+    keep = (fl & 0x03) == 0
+    return cells[keep], slots[keep]
+
+
+class WindStatistics:
+    """Pedestrian-level wind statistics of an in-process `LBM` (all domains in this process) on surface-following layers: for every height h_k (cells) above the
+    local ground or roof, the running mean and co-moments of u, mean / M2 / peak of the speed and threshold exceedance counts, accumulated on the device per sample
+    (luw_wind_stats_*). Build it after the flags are on the device (after run(0) / initialize()).
+
+    The ground of a global column is the lowest non-solid cell over the domains stacked in z (luw_column_ground per domain, minimum per column); each domain then
+    lists its owned plain-fluid cells at ground + h_k. The one-process-per-GPU DistributedLBM is not covered here; the C ABI allows the same construction there:
+    per-rank luw_column_ground, a min-reduce over the ranks stacked in z, then per-rank lists."""
+
+    def __init__(self, lbm, heights, thresholds=()):
+        self.lbm = lbm
+        self.heights = [int(h) for h in heights]
+        self.thresholds = np.ascontiguousarray(thresholds, np.float32)
+        Ng = lbm.Ng
+        H = tuple(1 if d > 1 else 0 for d in lbm.D)
+        self.ground = np.full((Ng[1], Ng[0]), 0xFFFFFFFF, np.uint32)
+        for dom, (_, O) in zip(lbm.domains, lbm._split):
+            g = dom.column_ground()[H[1]:dom.Ny - H[1], H[0]:dom.Nx - H[0]]
+            view = self.ground[O[1] + H[1]:O[1] + H[1] + g.shape[0], O[0] + H[0]:O[0] + H[0] + g.shape[1]]
+            np.minimum(view, g, out=view)
+        self._stats, self._slots = [], []
+        for dom, (_, O) in zip(lbm.domains, lbm._split):
+            cells, slots = wind_layer_cells(dom, O, Ng, lbm.D, self.ground, self.heights)
+            self._stats.append(WindStats(dom, cells, self.thresholds))
+            self._slots.append(slots)
+
+    def accumulate(self):
+        if not self.lbm.features & A.UPDATE_FIELDS:  # rho / u are not stored every step
+            self.lbm.update_fields()
+        for st in self._stats:
+            st.accumulate()
+
+    def reset(self):
+        for st in self._stats:
+            st.reset()
+
+    def download(self):
+        """-> dict of global layer-major arrays [..., k, y, x]: mean_u (3, K, Ny, Nx), comoment (6, ...: uu vv ww uv uw vw), mean_speed, m2_speed, max_speed,
+        exceed (thresholds, ...), valid (bool: the slot is a listed cell; float fields are NaN and counters 0 elsewhere) and the sample count."""
+        Ng, K, T = self.lbm.Ng, len(self.heights), int(self.thresholds.size)
+        M = K * Ng[1] * Ng[0]
+        out = {"mean_u": np.full((3, M), np.nan, np.float32), "comoment": np.full((6, M), np.nan, np.float32), "mean_speed": np.full(M, np.nan, np.float32),
+               "m2_speed": np.full(M, np.nan, np.float32), "max_speed": np.full(M, np.nan, np.float32), "exceed": np.zeros((T, M), np.uint32),
+               "valid": np.zeros(M, bool)}
+        samples = 0
+        for st, slots in zip(self._stats, self._slots):
+            mean_u, com, ms, m2, mx, ex, samples = st.download()
+            out["mean_u"][:, slots], out["comoment"][:, slots], out["exceed"][:, slots] = mean_u, com, ex
+            out["mean_speed"][slots], out["m2_speed"][slots], out["max_speed"][slots] = ms, m2, mx
+            out["valid"][slots] = True
+        out = {k: v.reshape(v.shape[:-1] + (K, Ng[1], Ng[0])) for k, v in out.items()}
+        out["samples"] = samples
+        return out
+
+    def close(self):
+        for st in self._stats:
+            st.close()
 
 
 class DistributedLBM(_Base):
