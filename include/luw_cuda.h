@@ -236,6 +236,34 @@ int luw_wind_stats_download(luw_wind_stats* st, float* host_mean_u, float* host_
 	uint32_t* host_exceed, uint64_t* samples);
 int luw_wind_stats_destroy(luw_wind_stats* st);
 
+/* Wind loads on buildings (momentum exchange). The reference's FORCE_FIELD extension (update_force_field, object_force / object_torque) keeps a 12 B-per-cell
+ * force field over the whole lattice and sums it with float atomics; here only the solid cells that touch the fluid are visited, per label (building), and
+ * every sum has a fixed order (csrc/lbm_wall_loads.cuh has the definitions).
+ * periodic_mask: bit a set = axis a (x y z) is periodic; a link whose partner lies across a GLOBAL face of a non-periodic axis does not count.
+ * luw_solid_surface: the listed cells of the domain -- owned solid cells ((flags & 0x03) == TYPE_S) with at least one counted link (partner n - c_i not solid) --
+ *   as local dense indices in ascending order, enumerated on the device from the device flags. Two calls: *count first (host_cells NULL), then the list
+ *   (capacity >= *count, else LUW_ERR_INVALID). Synchronous; meant to run once per case.
+ * luw_wall_loads_create: host_cell_index[count] local dense indices (owned, not halo) with host_label[count] < label_count, sorted by (label, index) strictly
+ *   increasing; host_ref_points[3*label_count] the reference point r0 of every label (global lattice coordinates, finite); sample_capacity >= 1 samples of
+ *   [label_count][6] doubles are kept on the device until drained. The links are classified once, here, from the device flags. count may be 0.
+ * luw_wall_loads_accumulate: one sample of the state whose DDFs are read with time step t (the t luw_update_fields would be given for it): per listed cell
+ *   F = 2 x the momentum its counted links carry into the wall (the GAUGE force of the fluid on the cell, relative to the reference pressure 1/3, lattice units),
+ *   the Welford update of the mean / M2 of F per cell, and per label the sums of F and of M = (r - r0) x F in double ([Fx Fy Fz Mx My Mz]). Stream-ordered on
+ *   the domain's stream, no host synchronisation, no luw_update_fields needed; LUW_ERR_INVALID when sample_capacity samples are pending (the host counts them).
+ * luw_wall_loads_drain: synchronous; copies the pending samples out in order, host_loads[s][label][6] (NULL: discard them), *samples = their number, and clears them.
+ * luw_wall_loads_download_cells: SoA [c*count + k] over the list, mean_F 3*count, m2_F 3*count; any pointer may be NULL; synchronous; *samples = samples since
+ *   create / reset.
+ * luw_wall_loads_reset: clears the per-cell statistics and discards the pending samples. */
+typedef struct luw_wall_loads luw_wall_loads;
+int luw_solid_surface(luw_domain* dom, uint32_t periodic_mask, uint64_t capacity, uint64_t* host_cells, uint64_t* count);
+int luw_wall_loads_create(luw_domain* dom, uint64_t count, const uint64_t* host_cell_index, const uint32_t* host_label, uint32_t label_count, const double* host_ref_points,
+	uint32_t periodic_mask, uint32_t sample_capacity, luw_wall_loads** out);
+int luw_wall_loads_accumulate(luw_wall_loads* st, uint64_t t);
+int luw_wall_loads_drain(luw_wall_loads* st, double* host_loads, uint64_t* samples);
+int luw_wall_loads_download_cells(luw_wall_loads* st, float* host_mean_F, float* host_m2_F, uint64_t* samples);
+int luw_wall_loads_reset(luw_wall_loads* st);
+int luw_wall_loads_destroy(luw_wall_loads* st);
+
 /* page-locked host memory for the mirrors (the reference's Memory<T> owns pageable new[] buffers, FX/opencl.hpp:354) */
 int luw_host_alloc(void** host_ptr, uint64_t bytes);
 int luw_host_free(void* host_ptr);

@@ -86,6 +86,13 @@ EXPORTS = {  # name -> argtypes; every symbol include/luw_cuda.h declares
     "luw_wind_stats_reset": [C.c_void_p],
     "luw_wind_stats_download": [C.c_void_p] + [C.c_void_p] * 6 + [C.POINTER(C.c_uint64)],
     "luw_wind_stats_destroy": [C.c_void_p],
+    "luw_solid_surface": [C.c_void_p, C.c_uint32, C.c_uint64, C.c_void_p, C.POINTER(C.c_uint64)],
+    "luw_wall_loads_create": [C.c_void_p, C.c_uint64, C.c_void_p, C.c_void_p, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.POINTER(C.c_void_p)],
+    "luw_wall_loads_accumulate": [C.c_void_p, C.c_uint64],
+    "luw_wall_loads_drain": [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
+    "luw_wall_loads_download_cells": [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
+    "luw_wall_loads_reset": [C.c_void_p],
+    "luw_wall_loads_destroy": [C.c_void_p],
     "luw_host_alloc": [C.POINTER(C.c_void_p), C.c_uint64],
     "luw_host_free": [C.c_void_p],
     "luw_sync": [C.c_void_p],

@@ -4,6 +4,7 @@
 #include "lbm_launch.h"
 #include "lbm_inlet.cuh"
 #include "lbm_wind_stats.cuh"
+#include "lbm_wall_loads.cuh"
 #include "vox_bins.h"
 
 #include <cmath>
@@ -96,6 +97,23 @@ struct luw_wind_stats {
 	float* acc; // [j*count + k], j < luw::WIND_FLOAT_ACCUMULATORS (lbm_wind_stats.cuh)
 	uint32_t* exceed; // [j*count + k], j < thr.count
 	luw::WindThresholds thr;
+};
+struct luw_wall_loads {
+	luw_domain* dom;
+	uint64_t count, nchunks, samples, pending, capacity;
+	uint32_t L, periodic;
+	uint64_t* cell; // device indices of the listed cells, sorted by (label, index)
+	uint32_t* links; // counted links per listed cell (lbm_wall_loads.cuh)
+	float* F; // [a*count + k]: the last sample's force per cell
+	float* acc; // [a*count + k]: mean of F (a < 3), M2 of F (3 <= a < 6)
+	uint64_t* chunk_begin; uint32_t* chunk_label; // [nchunks + 1], [nchunks]: first-level chunks of WALL_CHUNK cells of one label
+	uint64_t ngroups;
+	uint64_t* group_begin; // [ngroups + 1]: second-level groups of up to WALL_GROUP chunks of one label
+	uint64_t* label_group; // [L + 1]: the groups of label l are [label_group[l], label_group[l+1])
+	double* ref; // [3L]: reference points
+	double* partial; // [a*nchunks + h]
+	double* partial2; // [a*ngroups + g]
+	double* ring; // [capacity][L][6]: samples not drained yet
 };
 struct luw_vk_inlet {
 	luw_domain* dom;
@@ -1244,6 +1262,194 @@ int luw_wind_stats_destroy(luw_wind_stats* st) {
 	DeviceGuard guard(st->dom->p.device);
 	cudaStreamSynchronize(st->dom->stream);
 	cudaFree(st->cell); cudaFree(st->acc); cudaFree(st->exceed);
+	delete st;
+	return LUW_OK;
+}
+
+// owned range of a local axis: the halo layer at each end of a decomposed axis belongs to the neighbours
+static void owned_range(const uint32_t n, const uint32_t D, uint32_t& lo, uint32_t& hi) { lo = D>1u ? 1u : 0u; hi = n-lo; }
+static unsigned list_grid(const luw_domain* d, const uint64_t items) {
+	const uint64_t want = (items+255ull)/256ull, cap = d->sm_count>0 ? 8ull*(uint64_t)d->sm_count : 1184ull;
+	return (unsigned)(want<1ull ? 1ull : want<cap ? want : cap);
+}
+int luw_solid_surface(luw_domain* d, uint32_t periodic_mask, uint64_t capacity, uint64_t* host_cells, uint64_t* count) {
+	if(const int rc = require_device()) return rc;
+	if(!d||!count) return fail(LUW_ERR_INVALID, "null argument");
+	const luw::DomainConst& c = d->c;
+	uint32_t x0, x1, y0, y1, z0, z1;
+	owned_range(c.Nx, c.Dx, x0, x1); owned_range(c.Ny, c.Dy, y0, y1); owned_range(c.Nz, c.Dz, z0, z1);
+	const uint64_t rows = (uint64_t)(y1-y0)*(z1-z0);
+	DeviceGuard guard(d->p.device);
+	DeviceBuffers mem;
+	uint32_t* rc_dev = nullptr;
+	CU(mem.get(&rc_dev, rows));
+	luw::k_surface_rows<<<list_grid(d, rows), 256, 0, d->stream>>>(c, periodic_mask&7u, x0, x1, y0, y1, z0, z1, nullptr, rc_dev, nullptr);
+	CU(cudaGetLastError());
+	d->launches++;
+	std::vector<uint32_t> rc(rows);
+	CU(cudaMemcpyAsync(rc.data(), rc_dev, rows*4ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	std::vector<uint64_t> offset(rows);
+	uint64_t total = 0ull;
+	for(uint64_t r=0ull; r<rows; r++) { offset[r] = total; total += rc[r]; }
+	*count = total;
+	if(!host_cells) return LUW_OK;
+	if(capacity<total) return fail(LUW_ERR_INVALID, "capacity below the number of surface cells (call with host_cells == NULL for the count)");
+	if(total==0ull) return LUW_OK;
+	uint64_t* off_dev = nullptr; uint64_t* cells_dev = nullptr;
+	CU(mem.get(&off_dev, rows));
+	CU(mem.get(&cells_dev, total));
+	CU(cudaMemcpyAsync(off_dev, offset.data(), rows*8ull, cudaMemcpyHostToDevice, d->stream));
+	luw::k_surface_rows<<<list_grid(d, rows), 256, 0, d->stream>>>(c, periodic_mask&7u, x0, x1, y0, y1, z0, z1, off_dev, nullptr, cells_dev);
+	CU(cudaGetLastError());
+	d->launches++;
+	CU(cudaMemcpyAsync(host_cells, cells_dev, total*8ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	return LUW_OK;
+}
+int luw_wall_loads_create(luw_domain* d, uint64_t count, const uint64_t* host_cell_index, const uint32_t* host_label, uint32_t label_count, const double* host_ref_points,
+	uint32_t periodic_mask, uint32_t sample_capacity, luw_wall_loads** out) {
+	if(const int rc = require_device()) return rc;
+	if(!d||!out||(count>0ull&&(!host_cell_index||!host_label))||!host_ref_points) return fail(LUW_ERR_INVALID, "null argument");
+	*out = nullptr;
+	if(label_count==0u) return fail(LUW_ERR_INVALID, "label_count must be at least 1");
+	if(sample_capacity==0u) return fail(LUW_ERR_INVALID, "sample_capacity must be at least 1");
+	for(uint64_t q=0ull; q<3ull*label_count; q++) if(!std::isfinite(host_ref_points[q])) return fail(LUW_ERR_INVALID, "reference points must be finite");
+	const luw::DomainConst& c = d->c;
+	uint32_t x0, x1, y0, y1, z0, z1;
+	owned_range(c.Nx, c.Dx, x0, x1); owned_range(c.Ny, c.Dy, y0, y1); owned_range(c.Nz, c.Dz, z0, z1);
+	std::vector<uint64_t> cd(count), chunk_begin;
+	std::vector<uint32_t> chunk_label;
+	std::vector<uint64_t> label_group(label_count+1ull, 0ull);
+	for(uint64_t k=0ull; k<count; k++) {
+		const uint64_t n = host_cell_index[k];
+		const uint32_t l = host_label[k];
+		if(n>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
+		const uint32_t x = (uint32_t)(n%c.Nx), y = (uint32_t)((n/c.Nx)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Nx*c.Ny));
+		if(x<x0||x>=x1||y<y0||y>=y1||z<z0||z>=z1) return fail(LUW_ERR_INVALID, "cell index in a halo layer");
+		if(l>=label_count) return fail(LUW_ERR_INVALID, "label outside [0, label_count)");
+		if(k>0ull&&!(l>host_label[k-1ull]||(l==host_label[k-1ull]&&n>host_cell_index[k-1ull]))) return fail(LUW_ERR_INVALID, "the list must be sorted by (label, cell index), strictly increasing");
+		if(k==0ull||l!=host_label[k-1ull]||k-chunk_begin.back()==(uint64_t)luw::WALL_CHUNK) { chunk_begin.push_back(k); chunk_label.push_back(l); }
+		cd[k] = device_index(c, n);
+	}
+	const uint64_t nchunks = chunk_label.size();
+	chunk_begin.push_back(count);
+	std::vector<uint64_t> group_begin;
+	for(uint64_t h=0ull; h<nchunks; h++) if(h==0ull||chunk_label[h]!=chunk_label[h-1ull]||h-group_begin.back()==(uint64_t)luw::WALL_GROUP) {
+		group_begin.push_back(h);
+		label_group[chunk_label[h]+1ull] = group_begin.size(); // label l's groups: [label_group[l], label_group[l+1])
+	} else {
+		label_group[chunk_label[h]+1ull] = group_begin.size();
+	}
+	const uint64_t ngroups = group_begin.size();
+	group_begin.push_back(nchunks);
+	for(uint32_t l=1u; l<=label_count; l++) if(label_group[l]<label_group[l-1u]) label_group[l] = label_group[l-1u]; // labels without cells: empty ranges
+	DeviceGuard guard(d->p.device);
+	luw_wall_loads* st = new(std::nothrow) luw_wall_loads();
+	if(!st) return fail(LUW_ERR_OOM, "host allocation failed");
+	memset(st, 0, sizeof(*st));
+	st->dom = d; st->count = count; st->nchunks = nchunks; st->ngroups = ngroups; st->L = label_count; st->capacity = sample_capacity; st->periodic = periodic_mask&7u;
+	int rc = dev_alloc(d, &st->ref, 3ull*label_count);
+	if(rc==LUW_OK) rc = dev_alloc(d, &st->label_group, label_count+1ull);
+	if(rc==LUW_OK) rc = dev_alloc(d, &st->ring, (uint64_t)sample_capacity*label_count*luw::WALL_COMPONENTS);
+	if(rc==LUW_OK&&count>0ull) {
+		rc = dev_alloc(d, &st->cell, count);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->links, count);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->F, 3ull*count);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->acc, 6ull*count);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->chunk_begin, nchunks+1ull);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->chunk_label, nchunks);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->partial, luw::WALL_COMPONENTS*nchunks);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->group_begin, ngroups+1ull);
+		if(rc==LUW_OK) rc = dev_alloc(d, &st->partial2, luw::WALL_COMPONENTS*ngroups);
+	}
+	if(rc==LUW_OK) {
+		cudaError_t e = cudaMemcpyAsync(st->ref, host_ref_points, 3ull*label_count*8ull, cudaMemcpyHostToDevice, d->stream);
+		if(e==cudaSuccess) e = cudaMemcpyAsync(st->label_group, label_group.data(), (label_count+1ull)*8ull, cudaMemcpyHostToDevice, d->stream);
+		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->group_begin, group_begin.data(), (ngroups+1ull)*8ull, cudaMemcpyHostToDevice, d->stream);
+		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
+		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->chunk_begin, chunk_begin.data(), (nchunks+1ull)*8ull, cudaMemcpyHostToDevice, d->stream);
+		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->chunk_label, chunk_label.data(), nchunks*4ull, cudaMemcpyHostToDevice, d->stream);
+		if(e==cudaSuccess&&count>0ull) { // the links are classified once, from the device flags as they are now
+			luw::k_wall_links<<<list_grid(d, count), 256, 0, d->stream>>>(c, st->periodic, count, st->cell, st->links);
+			e = cudaGetLastError();
+			d->launches++;
+		}
+		if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // the host arrays may be freed by the caller afterwards
+		if(e!=cudaSuccess) rc = cuda_fail(e, "set up the wall-load list");
+	}
+	if(rc==LUW_OK) rc = luw_wall_loads_reset(st);
+	if(rc!=LUW_OK) { const std::string keep = g_error; luw_wall_loads_destroy(st); g_error = keep; return rc; }
+	*out = st;
+	return LUW_OK;
+}
+int luw_wall_loads_reset(luw_wall_loads* st) {
+	if(!st) return fail(LUW_ERR_INVALID, "null wall-loads object");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	if(st->count>0ull) CU(cudaMemsetAsync(st->acc, 0, 6ull*st->count*4ull, d->stream));
+	st->samples = 0ull;
+	st->pending = 0ull;
+	return LUW_OK;
+}
+int luw_wall_loads_accumulate(luw_wall_loads* st, uint64_t t) {
+	if(!st) return fail(LUW_ERR_INVALID, "null wall-loads object");
+	if(st->pending>=st->capacity) return fail(LUW_ERR_INVALID, "the sample ring is full: drain it first");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	const float inv_n = 1.0f/(float)(st->samples+1ull);
+	const uint32_t odd = (uint32_t)(t&1ull);
+	if(st->count>0ull) {
+		const unsigned g = list_grid(d, st->count);
+		switch(d->c.precision) {
+			case luw::P_FP32: luw::k_wall_cells<luw::P_FP32><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); break;
+			case luw::P_FP16S: luw::k_wall_cells<luw::P_FP16S><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); break;
+			default: luw::k_wall_cells<luw::P_FP16C><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); break;
+		}
+		CU(cudaGetLastError());
+		luw::k_wall_chunks<<<list_grid(d, st->nchunks), 256, 0, d->stream>>>(d->c, st->count, st->nchunks, st->chunk_begin, st->chunk_label, st->cell, st->F, st->ref, st->partial);
+		CU(cudaGetLastError());
+		luw::k_wall_segments<<<list_grid(d, st->ngroups*luw::WALL_COMPONENTS), 256, 0, d->stream>>>(st->ngroups, st->group_begin, st->nchunks, st->partial, 1ull, st->ngroups, st->partial2);
+		CU(cudaGetLastError());
+		d->launches += 3ull;
+	}
+	luw::k_wall_segments<<<list_grid(d, (uint64_t)st->L*luw::WALL_COMPONENTS), 256, 0, d->stream>>>(st->L, st->label_group, st->ngroups, st->partial2, luw::WALL_COMPONENTS, 1ull,
+		st->ring+st->pending*st->L*luw::WALL_COMPONENTS);
+	CU(cudaGetLastError());
+	d->launches++;
+	st->samples++;
+	st->pending++;
+	return LUW_OK;
+}
+int luw_wall_loads_drain(luw_wall_loads* st, double* host_loads, uint64_t* samples) {
+	if(!st) return fail(LUW_ERR_INVALID, "null wall-loads object");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	if(host_loads&&st->pending>0ull) CU(cudaMemcpyAsync(host_loads, st->ring, st->pending*st->L*luw::WALL_COMPONENTS*8ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	if(samples) *samples = st->pending;
+	st->pending = 0ull;
+	return LUW_OK;
+}
+int luw_wall_loads_download_cells(luw_wall_loads* st, float* host_mean_F, float* host_m2_F, uint64_t* samples) {
+	if(!st) return fail(LUW_ERR_INVALID, "null wall-loads object");
+	luw_domain* d = st->dom;
+	DeviceGuard guard(d->p.device);
+	const uint64_t K = st->count;
+	if(K>0ull) {
+		if(host_mean_F) CU(cudaMemcpyAsync(host_mean_F, st->acc, 3ull*K*4ull, cudaMemcpyDeviceToHost, d->stream));
+		if(host_m2_F) CU(cudaMemcpyAsync(host_m2_F, st->acc+3ull*K, 3ull*K*4ull, cudaMemcpyDeviceToHost, d->stream));
+	}
+	CU(cudaStreamSynchronize(d->stream));
+	if(samples) *samples = st->samples;
+	return LUW_OK;
+}
+int luw_wall_loads_destroy(luw_wall_loads* st) {
+	if(!st) return LUW_OK;
+	DeviceGuard guard(st->dom->p.device);
+	cudaStreamSynchronize(st->dom->stream);
+	cudaFree(st->cell); cudaFree(st->links); cudaFree(st->F); cudaFree(st->acc); cudaFree(st->chunk_begin); cudaFree(st->chunk_label);
+	cudaFree(st->group_begin); cudaFree(st->label_group); cudaFree(st->ref); cudaFree(st->partial); cudaFree(st->partial2); cudaFree(st->ring);
 	delete st;
 	return LUW_OK;
 }

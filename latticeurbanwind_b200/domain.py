@@ -244,6 +244,15 @@ class Domain:
         A.check(A.lib().luw_column_ground(self._h, _ptr(g)))
         return g
 
+    def solid_surface(self, periodic_mask=0):
+        """-> uint64 local dense indices, ascending, of the owned solid cells with at least one counted link (luw_solid_surface; enumerated on the device).
+        periodic_mask: bit a set = axis a is periodic (links across a global face of a non-periodic axis do not count)."""
+        n = C.c_uint64()
+        A.check(A.lib().luw_solid_surface(self._h, int(periodic_mask), 0, None, C.byref(n)))
+        cells = np.empty(n.value, np.uint64)
+        A.check(A.lib().luw_solid_surface(self._h, int(periodic_mask), cells.size, _ptr(cells), C.byref(n)))
+        return cells
+
     def device_bytes(self):
         n = C.c_uint64()
         A.check(A.lib().luw_domain_bytes(self._h, C.byref(n)))
@@ -361,6 +370,49 @@ class WindStats:
     def close(self):
         if self._h:
             A.lib().luw_wind_stats_destroy(self._h)
+            self._h = C.c_void_p()
+
+
+class WallLoads:
+    """Wind loads of a list of local solid cells (luw_wall_loads_*): per sample and label the sums of the momentum-exchange force F and of its moment
+    (r - r0) x F in double, kept in a device ring of `capacity` samples until drained, and per cell the running mean / M2 of F. `cells` / `labels` sorted by
+    (label, index); ref_points [L, 3] (global lattice coordinates)."""
+
+    def __init__(self, domain, cells, labels, label_count, ref_points, periodic_mask=0, capacity=256):
+        self.domain = domain
+        self.cells = np.ascontiguousarray(cells, np.uint64)
+        self.labels = np.ascontiguousarray(labels, np.uint32)
+        self.count, self.L, self.capacity = int(self.cells.size), int(label_count), int(capacity)
+        self.ref_points = np.ascontiguousarray(ref_points, np.float64)
+        assert self.labels.size == self.count and self.ref_points.size == 3 * self.L
+        self._h = C.c_void_p()
+        A.check(A.lib().luw_wall_loads_create(domain._h, self.count, _ptr(self.cells), _ptr(self.labels), self.L, _ptr(self.ref_points), int(periodic_mask),
+                                              self.capacity, C.byref(self._h)))
+
+    def accumulate(self, t=None):
+        """One sample of the current state (t: the domain's time step by default). Stream-ordered, no synchronisation."""
+        A.check(A.lib().luw_wall_loads_accumulate(self._h, self.domain.t if t is None else int(t)))
+
+    def drain(self):
+        """-> float64 [samples, L, 6] (Fx Fy Fz Mx My Mz) of the pending samples, in order; synchronous; clears them."""
+        out = np.empty((self.capacity, self.L, 6), np.float64)
+        n = C.c_uint64()
+        A.check(A.lib().luw_wall_loads_drain(self._h, _ptr(out), C.byref(n)))
+        return out[:n.value].copy()
+
+    def download_cells(self):
+        """-> (mean_F [3, count], m2_F [3, count], samples since create / reset)"""
+        mean, m2 = np.empty((3, self.count), np.float32), np.empty((3, self.count), np.float32)
+        n = C.c_uint64()
+        A.check(A.lib().luw_wall_loads_download_cells(self._h, _ptr(mean), _ptr(m2), C.byref(n)))
+        return mean, m2, n.value
+
+    def reset(self):
+        A.check(A.lib().luw_wall_loads_reset(self._h))
+
+    def close(self):
+        if self._h:
+            A.lib().luw_wall_loads_destroy(self._h)
             self._h = C.c_void_p()
 
 

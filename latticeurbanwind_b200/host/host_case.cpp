@@ -7,6 +7,8 @@
 //   LBM::voxelize_triangles_on_device like FX/setup.cpp:4084-4125 does with the STL, the flags of in.bin are OR-ed on top, and out.bin ends with flags[N] u8
 //   LUW_CASE_WIND=h0,h1,... (heights in cells) with LUW_CASE_WIND_THR=t0,t1,... and LUW_CASE_WIND_OUT=<file>: LBM_WindStatistics over the same sampling window as
 //   LUW_CASE_STATS; the file gets samples u64, mean_u[3M], comoment[6M], mean_speed[M], m2_speed[M], max_speed[M] f32, exceed[T*M] u32, valid[M] u8, ground[Nx*Ny] u32
+//   LUW_CASE_WALL_OUT=<file> (with LUW_CASE_WALL_GROUND=<ground_z>, default 0): LBM_WallLoads over the same sampling window as LUW_CASE_STATS; the file gets
+//   samples u64, L u32, K u64, series[samples*L*6] f64, ref_points[3L] f64, column_labels[Nx*Ny] u32, cell[K] u64, label[K] u32, mean_F[3K], m2_F[3K] f32
 //   with LUW_TEMPERATURE in `features`: in.bin carries T[N] f32 after u, out.bin ends with T[N] f32; alpha / beta of the LBM constructor from LUW_CASE_ALPHA / LUW_CASE_BETA
 #include "lbm.hpp"
 #include <fstream>
@@ -76,7 +78,20 @@ int main(int argc, char** argv) {
 	const char* wind_out = getenv("LUW_CASE_WIND_OUT");
 	LBM_WindStatistics* wind = wind_out ? new LBM_WindStatistics(lbm, env_list<uint>("LUW_CASE_WIND"), env_list<float>("LUW_CASE_WIND_THR")) : nullptr;
 	lbm.run(steps-(samples<steps ? samples : steps));
-	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); stats->accumulate(); if(wind) wind->accumulate(); }
+	const char* wall_out = getenv("LUW_CASE_WALL_OUT");
+	LBM_WallLoads* wall = wall_out ? new LBM_WallLoads(lbm, getenv("LUW_CASE_WALL_GROUND") ? (uint)atoi(getenv("LUW_CASE_WALL_GROUND")) : 0u) : nullptr;
+	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); stats->accumulate(); if(wind) wind->accumulate(); if(wall) wall->accumulate(); }
+	if(wall) {
+		std::vector<double> series; std::vector<ulong> cell; std::vector<uint> label; std::vector<float> mean_F, m2_F;
+		const uint64_t count = (uint64_t)wall->series(series), K = (uint64_t)(wall->surface(cell, label, mean_F, m2_F), cell.size());
+		std::ofstream wf(wall_out, std::ios::binary);
+		wf.write((const char*)&count, 8); wf.write((const char*)&wall->L, 4); wf.write((const char*)&K, 8);
+		wf.write((const char*)series.data(), (std::streamsize)(8u*series.size())); wf.write((const char*)wall->ref_points.data(), (std::streamsize)(8u*wall->ref_points.size()));
+		wf.write((const char*)wall->column_labels.data(), (std::streamsize)(4u*wall->column_labels.size()));
+		wf.write((const char*)cell.data(), (std::streamsize)(8u*K)); wf.write((const char*)label.data(), (std::streamsize)(4u*K));
+		wf.write((const char*)mean_F.data(), (std::streamsize)(4u*mean_F.size())); wf.write((const char*)m2_F.data(), (std::streamsize)(4u*m2_F.size()));
+		delete wall;
+	}
 	if(wind) {
 		std::vector<float> mean_u, comoment, mean_speed, m2_speed, max_speed; std::vector<uint> exceed; std::vector<uchar> valid;
 		const uint64_t count = (uint64_t)wind->download(mean_u, comoment, mean_speed, m2_speed, max_speed, exceed, valid);

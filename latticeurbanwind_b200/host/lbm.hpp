@@ -543,6 +543,23 @@ public:
 	}
 };
 
+// [y*Nx + x] over the global columns: global z of the lowest non-solid cell over the blocks stacked in z (luw_column_ground per domain, minimum per column),
+// 0xFFFFFFFF if none
+inline std::vector<uint> luw_global_column_ground(LBM& lbm) {
+	const uint Nx = lbm.get_Nx(), Ny = lbm.get_Ny(), Hx = lbm.get_Dx()>1u, Hy = lbm.get_Dy()>1u;
+	std::vector<uint> ground((size_t)Nx*Ny, 0xFFFFFFFFu);
+	for(uint d=0u; d<lbm.get_D(); d++) {
+		const LBM_Domain* dom = lbm.lbm_domain[d];
+		std::vector<uint32_t> g((size_t)dom->get_Nx()*dom->get_Ny());
+		luw_check(luw_column_ground(dom->get_handle(), g.data()));
+		for(uint y=Hy; y<dom->get_Ny()-Hy; y++) for(uint x=Hx; x<dom->get_Nx()-Hx; x++) {
+			uint& G = ground[(size_t)(y+dom->get_Oy())*Nx+(size_t)(x+dom->get_Ox())];
+			G = std::min(G, (uint)g[(size_t)y*dom->get_Nx()+x]);
+		}
+	}
+	return ground;
+}
+
 // ---------------------------------------------------------------------------------------------------------------- pedestrian-level wind statistics (no reference counterpart)
 // Surface-following layers: for every height h_k (cells) above the local ground or roof, the running mean and co-moments of u, mean / M2 / peak of the speed |u| and
 // how many samples exceed each threshold (lattice units, at most LUW_WIND_MAX_THRESHOLDS), accumulated on the device per sample (luw_wind_stats_*). Construct it once the
@@ -561,16 +578,7 @@ public:
 	std::vector<uint> ground; // [y*Nx + x] over the global columns: global z of the lowest non-solid cell, 0xFFFFFFFF if none
 	LBM_WindStatistics(LBM& lbm_, std::vector<uint> heights_in_cells, std::vector<float> thresholds_lattice) : lbm(&lbm_), heights(std::move(heights_in_cells)), thresholds((uint)thresholds_lattice.size()) {
 		const uint Nx = lbm->get_Nx(), Ny = lbm->get_Ny(), Nz = lbm->get_Nz(), Hx = lbm->get_Dx()>1u, Hy = lbm->get_Dy()>1u, Hz = lbm->get_Dz()>1u;
-		ground.assign((size_t)Nx*Ny, 0xFFFFFFFFu);
-		for(uint d=0u; d<lbm->get_D(); d++) { // lowest non-solid cell over the blocks stacked in z
-			const LBM_Domain* dom = lbm->lbm_domain[d];
-			std::vector<uint32_t> g((size_t)dom->get_Nx()*dom->get_Ny());
-			luw_check(luw_column_ground(dom->get_handle(), g.data()));
-			for(uint y=Hy; y<dom->get_Ny()-Hy; y++) for(uint x=Hx; x<dom->get_Nx()-Hx; x++) {
-				uint& G = ground[(size_t)(y+dom->get_Oy())*Nx+(size_t)(x+dom->get_Ox())];
-				G = std::min(G, (uint)g[(size_t)y*dom->get_Nx()+x]);
-			}
-		}
+		ground = luw_global_column_ground(*lbm);
 		for(uint d=0u; d<lbm->get_D(); d++) {
 			const LBM_Domain* dom = lbm->lbm_domain[d];
 			const ulong lNx = dom->get_Nx(), lNy = dom->get_Ny();
@@ -630,6 +638,139 @@ public:
 				for(ulong j=0ull; j<thresholds; j++) exceed[j*M+m] = ex[j*K+i];
 				valid[m] = 1u;
 			}
+		}
+		return (ulong)samples;
+	}
+};
+
+// ---------------------------------------------------------------------------------------------------------------- wind loads on buildings (momentum exchange)
+// Per sample and label (building): the force of the fluid on the label's surface cells and its moment about the label's reference point r0, [Fx Fy Fz Mx My Mz]
+// in double, lattice units, GAUGE (relative to the reference pressure 1/3); per surface cell the running mean / M2 of the force (luw_solid_surface,
+// luw_wall_loads_*; definitions in csrc/lbm_wall_loads.cuh). Construct it once the flags are on the device (after run(0)); call accumulate() after a step --
+// no update_fields is needed. The same labels and r0 as lbm.WallLoads in Python: a building column is one whose global column ground (luw_global_column_ground)
+// lies above ground_z + 1; building columns form 4-connected footprints (no wrap across the lattice edges) numbered 1..B in row-major (y, x) order of first
+// appearance; a listed cell takes its column's label above z = ground_z, 0 (terrain) at or below it; r0 = the footprint's column-centre centroid at
+// z = ground_z + 0.5 (overturning moment), the origin for label 0. column_labels[y*Nx + x] / ref_points[3*l + a] replace the defaults when not empty.
+// The samples stay on the device until `capacity` are pending; then they are drained (the only host synchronisation). This class does not add the
+// reference's FORCE_FIELD names (lbm.F, object_force, object_torque).
+class LBM_WallLoads {
+private:
+	LBM* lbm = nullptr;
+	uint capacity = 256u;
+	ulong pending = 0ull;
+	std::vector<luw_wall_loads*> st;
+	std::vector<std::vector<ulong>> global; // per domain: global cell index of every listed cell, in list order
+	std::vector<std::vector<uint>> labels_of; // per domain: label of every listed cell, in list order
+	std::vector<double> loads; // drained samples [s][L][6], summed over the domains in domain order
+	void drain() {
+		const ulong S6 = (ulong)L*6ull;
+		std::vector<double> total, part((ulong)capacity*S6);
+		uint64_t n = 0ull;
+		for(uint d=0u; d<st.size(); d++) {
+			luw_check(luw_wall_loads_drain(st[d], part.data(), &n));
+			if(d==0u) total.assign(part.begin(), part.begin()+(long)(n*S6));
+			else for(ulong q=0ull; q<n*S6; q++) total[q] += part[q];
+		}
+		loads.insert(loads.end(), total.begin(), total.end());
+		pending = 0ull;
+	}
+public:
+	uint L = 0u; // labels
+	std::vector<uint> ground; // [y*Nx + x]: global column ground
+	std::vector<uint> column_labels; // [y*Nx + x]
+	std::vector<double> ref_points; // [3*l + a]
+	LBM_WallLoads(LBM& lbm_, const uint ground_z=0u, std::vector<uint> column_labels_in={}, std::vector<double> ref_points_in={}, const bool periodic_x=false,
+		const bool periodic_y=false, const bool periodic_z=false, const uint capacity_=256u) : lbm(&lbm_), capacity(capacity_) {
+		const uint Nx = lbm->get_Nx(), Ny = lbm->get_Ny();
+		const uint periodic = (periodic_x ? 1u : 0u)|(periodic_y ? 2u : 0u)|(periodic_z ? 4u : 0u);
+		ground = luw_global_column_ground(*lbm);
+		if(column_labels_in.empty()) { // breadth-first flood fill, started in row-major order
+			column_labels.assign((size_t)Nx*Ny, 0u);
+			uint next = 0u;
+			std::vector<ulong> queue;
+			for(ulong s=0ull; s<(ulong)Nx*Ny; s++) {
+				if(!((ulong)ground[s]>(ulong)ground_z+1ull)||column_labels[s]!=0u) continue;
+				column_labels[s] = ++next;
+				queue.assign(1u, s);
+				for(size_t q=0u; q<queue.size(); q++) {
+					const ulong c = queue[q], x = c%Nx, y = c/Nx;
+					const ulong nb[4] = { y>0ull ? c-Nx : c, y+1ull<Ny ? c+Nx : c, x>0ull ? c-1ull : c, x+1ull<Nx ? c+1ull : c };
+					for(const ulong m : nb) if(m!=c&&(ulong)ground[m]>(ulong)ground_z+1ull&&column_labels[m]==0u) { column_labels[m] = next; queue.push_back(m); }
+				}
+			}
+		} else {
+			column_labels = std::move(column_labels_in);
+		}
+		L = 1u;
+		for(const uint l : column_labels) L = std::max(L, l+1u);
+		if(ref_points_in.empty()) {
+			std::vector<ulong> cnt(L, 0ull), sx(L, 0ull), sy(L, 0ull);
+			for(ulong s=0ull; s<(ulong)Nx*Ny; s++) { const uint l = column_labels[s]; cnt[l]++; sx[l] += s%Nx; sy[l] += s/Nx; }
+			ref_points.assign(3ull*L, 0.0);
+			for(uint l=1u; l<L; l++) if(cnt[l]>0ull) {
+				ref_points[3u*l] = (double)sx[l]/(double)cnt[l]; ref_points[3u*l+1u] = (double)sy[l]/(double)cnt[l]; ref_points[3u*l+2u] = (double)ground_z+0.5;
+			}
+		} else {
+			ref_points = std::move(ref_points_in);
+		}
+		for(uint d=0u; d<lbm->get_D(); d++) {
+			const LBM_Domain* dom = lbm->lbm_domain[d];
+			const ulong lNx = dom->get_Nx(), lNy = dom->get_Ny();
+			uint64_t count = 0ull;
+			luw_check(luw_solid_surface(dom->get_handle(), periodic, 0ull, nullptr, &count));
+			std::vector<uint64_t> cells(count);
+			luw_check(luw_solid_surface(dom->get_handle(), periodic, count, cells.data(), &count));
+			std::vector<uint> lab(count);
+			std::vector<ulong> gidx(count), order(count);
+			for(ulong k=0ull; k<count; k++) {
+				const ulong n = cells[k];
+				const ulong gx = (ulong)((long)(n%lNx)+dom->get_Ox()), gy = (ulong)((long)((n/lNx)%lNy)+dom->get_Oy()), gz = (ulong)((long)(n/(lNx*lNy))+dom->get_Oz());
+				lab[k] = gz>(ulong)ground_z ? column_labels[gy*Nx+gx] : 0u;
+				gidx[k] = gx+(gy+gz*Ny)*(ulong)Nx;
+				order[k] = k;
+			}
+			std::sort(order.begin(), order.end(), [&](const ulong a, const ulong b) { return lab[a]!=lab[b] ? lab[a]<lab[b] : cells[a]<cells[b]; });
+			std::vector<uint64_t> sc(count); std::vector<uint32_t> sl(count); std::vector<ulong> sg(count); std::vector<uint> slab(count);
+			for(ulong k=0ull; k<count; k++) { sc[k] = cells[order[k]]; sl[k] = lab[order[k]]; sg[k] = gidx[order[k]]; slab[k] = lab[order[k]]; }
+			luw_wall_loads* h = nullptr;
+			luw_check(luw_wall_loads_create(dom->get_handle(), count, sc.data(), sl.data(), L, ref_points.data(), periodic, capacity, &h));
+			st.push_back(h); global.push_back(std::move(sg)); labels_of.push_back(std::move(slab));
+		}
+	}
+	~LBM_WallLoads() { for(luw_wall_loads* h : st) luw_wall_loads_destroy(h); }
+	LBM_WallLoads(const LBM_WallLoads&) = delete;
+	LBM_WallLoads& operator=(const LBM_WallLoads&) = delete;
+	void accumulate() {
+		if(pending==(ulong)capacity) drain();
+		for(uint d=0u; d<lbm->get_D(); d++) luw_check(luw_wall_loads_accumulate(st[d], lbm->lbm_domain[d]->get_t()));
+		pending++;
+	}
+	void reset() { for(luw_wall_loads* h : st) luw_check(luw_wall_loads_reset(h)); pending = 0ull; loads.clear(); }
+	// series[(s*L + l)*6 + a], a = Fx Fy Fz Mx My Mz, since construction / reset. Returns the sample count.
+	ulong series(std::vector<double>& out) {
+		drain();
+		out = loads;
+		return (ulong)(loads.size()/((ulong)L*6ull));
+	}
+	// all listed cells in ascending global index n = x+(y+z*Ny)*Nx: cell[k], label[k], mean_F[a*K + k], m2_F[a*K + k]. Returns the sample count.
+	ulong surface(std::vector<ulong>& cell, std::vector<uint>& label, std::vector<float>& mean_F, std::vector<float>& m2_F) {
+		std::vector<ulong> all; std::vector<uint> lab; std::vector<float> mean[3], m2[3];
+		uint64_t samples = 0ull;
+		for(uint d=0u; d<st.size(); d++) {
+			const ulong K = global[d].size();
+			std::vector<float> a(3ull*K), b(3ull*K);
+			luw_check(luw_wall_loads_download_cells(st[d], a.data(), b.data(), &samples));
+			all.insert(all.end(), global[d].begin(), global[d].end()); lab.insert(lab.end(), labels_of[d].begin(), labels_of[d].end());
+			for(uint c=0u; c<3u; c++) { mean[c].insert(mean[c].end(), a.begin()+(long)(c*K), a.begin()+(long)((c+1u)*K)); m2[c].insert(m2[c].end(), b.begin()+(long)(c*K), b.begin()+(long)((c+1u)*K)); }
+		}
+		const ulong K = all.size();
+		std::vector<ulong> order(K);
+		for(ulong k=0ull; k<K; k++) order[k] = k;
+		std::sort(order.begin(), order.end(), [&](const ulong a, const ulong b) { return all[a]<all[b]; });
+		cell.resize(K); label.resize(K); mean_F.resize(3ull*K); m2_F.resize(3ull*K);
+		for(ulong k=0ull; k<K; k++) {
+			cell[k] = all[order[k]]; label[k] = lab[order[k]];
+			for(uint c=0u; c<3u; c++) { mean_F[c*K+k] = mean[c][order[k]]; m2_F[c*K+k] = m2[c][order[k]]; }
 		}
 		return (ulong)samples;
 	}

@@ -18,6 +18,7 @@ import numpy as np
 from . import _cabi as A
 from . import cases
 from .domain import CellSet, Domain, WindStats
+from .domain import WallLoads as DomainWallLoads
 
 AXES = (0, 1, 2)
 
@@ -218,6 +219,19 @@ def wind_layer_cells(dom, O, Ng, D, ground, heights):
     return cells[keep], slots[keep]
 
 
+def global_column_ground(lbm):
+    """uint32 [Ng_y, Ng_x]: global z of the lowest non-solid cell of every global column over the domains stacked in z (luw_column_ground per domain, minimum
+    per column), 0xFFFFFFFF where there is none."""
+    Ng = lbm.Ng
+    H = tuple(1 if d > 1 else 0 for d in lbm.D)
+    ground = np.full((Ng[1], Ng[0]), 0xFFFFFFFF, np.uint32)
+    for dom, (_, O) in zip(lbm.domains, lbm._split):
+        g = dom.column_ground()[H[1]:dom.Ny - H[1], H[0]:dom.Nx - H[0]]
+        view = ground[O[1] + H[1]:O[1] + H[1] + g.shape[0], O[0] + H[0]:O[0] + H[0] + g.shape[1]]
+        np.minimum(view, g, out=view)
+    return ground
+
+
 class WindStatistics:
     """Pedestrian-level wind statistics of an in-process `LBM` (all domains in this process) on surface-following layers: for every height h_k (cells) above the
     local ground or roof, the running mean and co-moments of u, mean / M2 / peak of the speed and threshold exceedance counts, accumulated on the device per sample
@@ -232,12 +246,7 @@ class WindStatistics:
         self.heights = [int(h) for h in heights]
         self.thresholds = np.ascontiguousarray(thresholds, np.float32)
         Ng = lbm.Ng
-        H = tuple(1 if d > 1 else 0 for d in lbm.D)
-        self.ground = np.full((Ng[1], Ng[0]), 0xFFFFFFFF, np.uint32)
-        for dom, (_, O) in zip(lbm.domains, lbm._split):
-            g = dom.column_ground()[H[1]:dom.Ny - H[1], H[0]:dom.Nx - H[0]]
-            view = self.ground[O[1] + H[1]:O[1] + H[1] + g.shape[0], O[0] + H[0]:O[0] + H[0] + g.shape[1]]
-            np.minimum(view, g, out=view)
+        self.ground = global_column_ground(lbm)
         self._stats, self._slots = [], []
         for dom, (_, O) in zip(lbm.domains, lbm._split):
             cells, slots = wind_layer_cells(dom, O, Ng, lbm.D, self.ground, self.heights)
@@ -274,6 +283,138 @@ class WindStatistics:
 
     def close(self):
         for st in self._stats:
+            st.close()
+
+
+def footprint_labels(ground, ground_z=0):
+    """uint32 [Ny, Nx] from the global column ground: 0 outside buildings; a building column is one whose ground (lowest non-solid z) lies above ground_z + 1
+    (an all-solid column included). Building columns are grouped into 4-connected footprints (no wrap across the lattice edges), numbered 1..B in row-major
+    (y, x) order of first appearance. Minimum-index propagation with pointer jumping: every column ends with the smallest raster index of its footprint."""
+    b = np.asarray(ground).astype(np.int64) > int(ground_z) + 1
+    Ny, Nx = b.shape
+    big = Ny * Nx
+    lab = np.where(b, np.arange(big, dtype=np.int64).reshape(Ny, Nx), big)
+    while True:
+        n = lab.copy()
+        np.minimum(n[1:], lab[:-1], out=n[1:])
+        np.minimum(n[:-1], lab[1:], out=n[:-1])
+        np.minimum(n[:, 1:], lab[:, :-1], out=n[:, 1:])
+        np.minimum(n[:, :-1], lab[:, 1:], out=n[:, :-1])
+        n = np.where(b, n, big)
+        n = np.where(b, n.reshape(-1)[np.minimum(n, big - 1)], big)  # pointer jumping: the label of the column one points at
+        if np.array_equal(n, lab):
+            break
+        lab = n
+    out = np.zeros((Ny, Nx), np.uint32)
+    roots = np.unique(lab[b])  # ascending smallest raster index = order of first appearance
+    out[b] = (np.searchsorted(roots, lab[b]) + 1).astype(np.uint32)
+    return out
+
+
+def footprint_ref_points(column_labels, label_count, ground_z=0):
+    """float64 [L, 3]: per label l >= 1 the centroid of its columns' centres (x, y) -- integer sums divided by the column count -- at z = ground_z + 0.5, the
+    base of the building, so that the moment is the overturning moment; the origin for label 0 (terrain) and for a label without columns."""
+    lab = np.asarray(column_labels).astype(np.int64).reshape(-1)
+    Ny, Nx = np.asarray(column_labels).shape
+    xs, ys = np.tile(np.arange(Nx, dtype=np.int64), Ny), np.repeat(np.arange(Ny, dtype=np.int64), Nx)
+    cnt = np.bincount(lab, minlength=label_count)[:label_count]
+    sx, sy = np.bincount(lab, xs, label_count)[:label_count], np.bincount(lab, ys, label_count)[:label_count]
+    out = np.zeros((label_count, 3), np.float64)
+    has = cnt > 0
+    has[0] = False
+    out[has, 0], out[has, 1] = sx[has] / cnt[has], sy[has] / cnt[has]
+    out[has, 2] = float(ground_z) + 0.5
+    return out
+
+
+class WallLoads:
+    """Wind loads on the buildings of an in-process `LBM` (all domains in this process): per sample and label (building) the momentum-exchange force and its
+    moment about the label's reference point, and per surface cell the running mean / M2 of the force (luw_solid_surface, luw_wall_loads_*). Build it after
+    the flags are on the device (after run(0) / initialize()).
+
+    Every domain lists its solid cells that touch the fluid (luw_solid_surface; `periodic` per axis: links across a global face of a non-periodic axis do not
+    count). Labels: by default from the global column ground (as in WindStatistics) -- footprint_labels(ground, ground_z) -- or from `column_labels[Ny][Nx]`
+    (for example building ids from GIS data); a listed cell takes its column's label above z = ground_z and 0 (terrain) at or below it. Reference points:
+    `ref_points[L][3]` or footprint_ref_points (the footprint's centroid at its base; the origin for label 0).
+
+    accumulate() samples the current state without update_fields; the samples stay on the device until `capacity` of them are pending, then they are drained
+    (the only host synchronisation). Forces and moments are in lattice units and gauge (relative to the reference pressure 1/3); dividing by 1/2 rho U^2 A for
+    coefficients is the caller's business. The one-process-per-GPU DistributedLBM is not covered (it would need a cross-rank sum per sample)."""
+
+    def __init__(self, lbm, ground_z=0, column_labels=None, ref_points=None, periodic=(False, False, False), capacity=256):
+        self.lbm = lbm
+        self.ground_z = int(ground_z)
+        self.capacity = int(capacity)
+        self.periodic_mask = sum(1 << a for a in AXES if periodic[a])
+        Ng = lbm.Ng
+        self.ground = global_column_ground(lbm)
+        self.column_labels = footprint_labels(self.ground, self.ground_z) if column_labels is None else np.asarray(column_labels).astype(np.uint32).reshape(Ng[1], Ng[0])
+        self.L = int(self.column_labels.max()) + 1
+        self.ref_points = footprint_ref_points(self.column_labels, self.L, self.ground_z) if ref_points is None else \
+            np.ascontiguousarray(ref_points, np.float64).reshape(self.L, 3)
+        self._loads, self._global, self._labels = [], [], []
+        for dom, (_, O) in zip(lbm.domains, lbm._split):
+            local = dom.solid_surface(self.periodic_mask).astype(np.int64)
+            gx, gy, gz = local % dom.Nx + O[0], (local // dom.Nx) % dom.Ny + O[1], local // (dom.Nx * dom.Ny) + O[2]  # owned cells never wrap
+            lab = np.where(gz > self.ground_z, self.column_labels[gy, gx], 0).astype(np.uint32)
+            order = np.lexsort((local, lab))
+            self._loads.append(DomainWallLoads(dom, local[order], lab[order], self.L, self.ref_points, self.periodic_mask, self.capacity))
+            self._global.append((gx + (gy + gz * Ng[1]) * Ng[0])[order])
+            self._labels.append(lab[order])
+        self._pending = 0
+        self._series = []
+
+    def accumulate(self):
+        if self._pending == self.capacity:
+            self._drain()
+        for dom, st in zip(self.lbm.domains, self._loads):
+            st.accumulate(dom.t)
+        self._pending += 1
+
+    def _drain(self):
+        parts = [st.drain() for st in self._loads]
+        total = parts[0].copy()
+        for p in parts[1:]:  # domain order
+            total += p
+        if total.shape[0]:
+            self._series.append(total)
+        self._pending = 0
+
+    def series(self):
+        """-> float64 [samples, L, 6]: Fx Fy Fz Mx My Mz per sample and label since construction / reset, summed over the domains in domain order."""
+        self._drain()
+        return np.concatenate(self._series) if self._series else np.zeros((0, self.L, 6), np.float64)
+
+    def summary(self):
+        """-> dict of float64 [L, 6]: mean, std (population), min and max over the samples of the series, and the sample count."""
+        s = self.series()
+        if not s.shape[0]:
+            raise ValueError("no samples accumulated")
+        return {"mean": s.mean(0), "std": s.std(0), "min": s.min(0), "max": s.max(0), "samples": s.shape[0]}
+
+    def surface(self):
+        """-> dict over all listed cells, ascending global index n = x + (y + z*Ny)*Nx: cell, x, y, z, label, mean_F [3, K], m2_F [3, K], samples."""
+        Ng = self.lbm.Ng
+        cell = np.concatenate(self._global)
+        label = np.concatenate(self._labels)
+        mean, m2, samples = [], [], 0
+        for st in self._loads:
+            a, b, samples = st.download_cells()
+            mean.append(a)
+            m2.append(b)
+        order = np.argsort(cell, kind="stable")
+        cell = cell[order]
+        return {"cell": cell.astype(np.uint64), "x": cell % Ng[0], "y": (cell // Ng[0]) % Ng[1], "z": cell // (Ng[0] * Ng[1]), "label": label[order],
+                "mean_F": np.concatenate(mean, axis=1)[:, order], "m2_F": np.concatenate(m2, axis=1)[:, order], "samples": samples}
+
+    def reset(self):
+        for st in self._loads:
+            st.reset()
+        self._pending = 0
+        self._series = []
+
+    def close(self):
+        for st in self._loads:
             st.close()
 
 
