@@ -264,6 +264,22 @@ int luw_wall_loads_download_cells(luw_wall_loads* st, float* host_mean_F, float*
 int luw_wall_loads_reset(luw_wall_loads* st);
 int luw_wall_loads_destroy(luw_wall_loads* st);
 
+/* Probe time series. The reference reads the whole u field back per probe output (FX/setup.cpp:4498-4509), after update_fields over the whole lattice
+ * (FX/lbm.cpp:348-355); here one kernel reads the DDFs of the listed cells only, and the samples stay on the device until drained (csrc/lbm_probes.cuh).
+ * luw_probes_create: host_cell_index[count] = local dense indices (like luw_cellset_create), owned (not halo) and < Nx*Ny*Nz; duplicates allowed, count may be 0;
+ *   sample_capacity >= 1 samples of C*count floats are kept on the device, C = 4 (rho ux uy uz) or 5 (and T, LUW_TEMPERATURE domains).
+ * luw_probes_sample: the same arguments as luw_update_fields; per listed cell the rho / u (/ T) that luw_update_fields(t, ...) followed by a read of the fields
+ *   would give -- the stored fields on domains with LUW_UPDATE_FIELDS and at the cells update_fields leaves alone -- without writing into the lattice.
+ *   Stream-ordered on the domain's stream, no host synchronisation; LUW_ERR_INVALID when sample_capacity samples are pending (the host counts them).
+ * luw_probes_drain: synchronous; copies the pending samples out in order, host_values[s][c][k] (NULL: discard them), *samples = their number, and clears them.
+ * luw_probes_reset: discards the pending samples. Without a CUDA device every entry returns LUW_ERR_NO_DEVICE. */
+typedef struct luw_probes luw_probes;
+int luw_probes_create(luw_domain* dom, uint64_t count, const uint64_t* host_cell_index, uint32_t sample_capacity, luw_probes** out);
+int luw_probes_sample(luw_probes* pr, uint64_t t, float fx, float fy, float fz, float omega_x, float omega_y, float omega_z);
+int luw_probes_drain(luw_probes* pr, float* host_values, uint64_t* samples);
+int luw_probes_reset(luw_probes* pr);
+int luw_probes_destroy(luw_probes* pr);
+
 /* page-locked host memory for the mirrors (the reference's Memory<T> owns pageable new[] buffers, FX/opencl.hpp:354) */
 int luw_host_alloc(void** host_ptr, uint64_t bytes);
 int luw_host_free(void* host_ptr);

@@ -93,6 +93,11 @@ EXPORTS = {  # name -> argtypes; every symbol include/luw_cuda.h declares
     "luw_wall_loads_download_cells": [C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
     "luw_wall_loads_reset": [C.c_void_p],
     "luw_wall_loads_destroy": [C.c_void_p],
+    "luw_probes_create": [C.c_void_p, C.c_uint64, C.c_void_p, C.c_uint32, C.POINTER(C.c_void_p)],
+    "luw_probes_sample": [C.c_void_p, C.c_uint64] + [C.c_float] * 6,
+    "luw_probes_drain": [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
+    "luw_probes_reset": [C.c_void_p],
+    "luw_probes_destroy": [C.c_void_p],
     "luw_host_alloc": [C.POINTER(C.c_void_p), C.c_uint64],
     "luw_host_free": [C.c_void_p],
     "luw_sync": [C.c_void_p],

@@ -29,6 +29,8 @@ struct KernelSet { // one per arithmetic mode; every function enqueues exactly o
 	cudaError_t (*halo_gi)(const DomainConst& c, int precision, uint32_t axis, uint32_t odd, bool insert, bool xfast, void* buf_p, void* buf_m, cudaStream_t s);
 	cudaError_t (*halo_T)(const DomainConst& c, uint32_t axis, bool insert, bool xfast, void* buf_p, void* buf_m, cudaStream_t s);
 	cudaError_t (*thermal_g)(const DomainConst& c, const StepArgs& a, cudaStream_t s); // the TEMPERATURE block alone, after a tiled momentum step that filled c.upre
+	// probe sample (lbm_probes.cuh): rho, u (and T) of `count` listed cells (device indices), as update_fields + a read would give them, into out[c*count + k]
+	cudaError_t (*probe_sample)(const DomainConst& c, const StepArgs& a, uint64_t count, const uint64_t* cell, float* out, unsigned grid, cudaStream_t s);
 };
 const KernelSet& kernels_strict(); // lbm_strict.cu: -fmad=false
 const KernelSet& kernels_fast(); // lbm_fast.cu: contraction allowed

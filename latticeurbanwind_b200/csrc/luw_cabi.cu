@@ -115,6 +115,13 @@ struct luw_wall_loads {
 	double* partial2; // [a*ngroups + g]
 	double* ring; // [capacity][L][6]: samples not drained yet
 };
+struct luw_probes {
+	luw_domain* dom;
+	uint64_t count, pending, capacity;
+	uint32_t comps; // 4: rho ux uy uz; 5: and T
+	uint64_t* cell; // device indices of the listed cells
+	float* ring; // [capacity][comps][count]: samples not drained yet
+};
 struct luw_vk_inlet {
 	luw_domain* dom;
 	uint64_t P, M, V;
@@ -1451,6 +1458,82 @@ int luw_wall_loads_destroy(luw_wall_loads* st) {
 	cudaFree(st->cell); cudaFree(st->links); cudaFree(st->F); cudaFree(st->acc); cudaFree(st->chunk_begin); cudaFree(st->chunk_label);
 	cudaFree(st->group_begin); cudaFree(st->label_group); cudaFree(st->ref); cudaFree(st->partial); cudaFree(st->partial2); cudaFree(st->ring);
 	delete st;
+	return LUW_OK;
+}
+
+int luw_probes_create(luw_domain* d, uint64_t count, const uint64_t* host_cell_index, uint32_t sample_capacity, luw_probes** out) {
+	if(const int rc = require_device()) return rc;
+	if(!d||!out||(count>0ull&&!host_cell_index)) return fail(LUW_ERR_INVALID, "null argument");
+	*out = nullptr;
+	if(sample_capacity==0u) return fail(LUW_ERR_INVALID, "sample_capacity must be at least 1");
+	const luw::DomainConst& c = d->c;
+	uint32_t x0, x1, y0, y1, z0, z1;
+	owned_range(c.Nx, c.Dx, x0, x1); owned_range(c.Ny, c.Dy, y0, y1); owned_range(c.Nz, c.Dz, z0, z1);
+	std::vector<uint64_t> cd(count);
+	for(uint64_t k=0ull; k<count; k++) {
+		const uint64_t n = host_cell_index[k];
+		if(n>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
+		const uint32_t x = (uint32_t)(n%c.Nx), y = (uint32_t)((n/c.Nx)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Nx*c.Ny));
+		if(x<x0||x>=x1||y<y0||y>=y1||z<z0||z>=z1) return fail(LUW_ERR_INVALID, "cell index in a halo layer");
+		cd[k] = device_index(c, n);
+	}
+	DeviceGuard guard(d->p.device);
+	luw_probes* pr = new(std::nothrow) luw_probes();
+	if(!pr) return fail(LUW_ERR_OOM, "host allocation failed");
+	memset(pr, 0, sizeof(*pr));
+	pr->dom = d; pr->count = count; pr->capacity = sample_capacity; pr->comps = (c.features&luw::F_TEMPERATURE) ? 5u : 4u;
+	int rc = LUW_OK;
+	if(count>0ull) {
+		rc = dev_alloc(d, &pr->cell, count);
+		if(rc==LUW_OK) rc = dev_alloc(d, &pr->ring, (uint64_t)sample_capacity*pr->comps*count);
+		if(rc==LUW_OK) {
+			cudaError_t e = cudaMemcpyAsync(pr->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
+			if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // cd is freed on return
+			if(e!=cudaSuccess) rc = cuda_fail(e, "upload the probe list");
+		}
+	}
+	if(rc!=LUW_OK) { const std::string keep = g_error; luw_probes_destroy(pr); g_error = keep; return rc; }
+	*out = pr;
+	return LUW_OK;
+}
+int luw_probes_sample(luw_probes* pr, uint64_t t, float fx, float fy, float fz, float ox, float oy, float oz) {
+	if(const int rc = require_device()) return rc;
+	if(!pr) return fail(LUW_ERR_INVALID, "null probes object");
+	if(pr->pending>=pr->capacity) return fail(LUW_ERR_INVALID, "the sample ring is full: drain it first");
+	luw_domain* d = pr->dom;
+	if(pr->count>0ull) {
+		DeviceGuard guard(d->p.device);
+		const luw::StepArgs a = { t, fx, fy, fz, ox, oy, oz };
+		CU(d->ks->probe_sample(d->c, a, pr->count, pr->cell, pr->ring+pr->pending*pr->comps*pr->count, list_grid(d, pr->count), d->stream));
+		d->launches++;
+	}
+	pr->pending++;
+	return LUW_OK;
+}
+int luw_probes_drain(luw_probes* pr, float* host_values, uint64_t* samples) {
+	if(const int rc = require_device()) return rc;
+	if(!pr) return fail(LUW_ERR_INVALID, "null probes object");
+	luw_domain* d = pr->dom;
+	DeviceGuard guard(d->p.device);
+	if(host_values&&pr->pending>0ull&&pr->count>0ull) CU(cudaMemcpyAsync(host_values, pr->ring, pr->pending*pr->comps*pr->count*4ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	if(samples) *samples = pr->pending;
+	pr->pending = 0ull;
+	return LUW_OK;
+}
+int luw_probes_reset(luw_probes* pr) {
+	if(const int rc = require_device()) return rc;
+	if(!pr) return fail(LUW_ERR_INVALID, "null probes object");
+	pr->pending = 0ull;
+	return LUW_OK;
+}
+int luw_probes_destroy(luw_probes* pr) {
+	if(const int rc = require_device()) return rc;
+	if(!pr) return LUW_OK;
+	DeviceGuard guard(pr->dom->p.device);
+	cudaStreamSynchronize(pr->dom->stream);
+	cudaFree(pr->cell); cudaFree(pr->ring);
+	delete pr;
 	return LUW_OK;
 }
 

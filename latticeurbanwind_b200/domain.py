@@ -416,6 +416,39 @@ class WallLoads:
             self._h = C.c_void_p()
 
 
+class Probes:
+    """Time series of rho, u (and T) at a list of local cells (luw_probes_*): per sample the values update_fields + a read would give, read from the DDFs of
+    the listed cells only and kept in a device ring of `capacity` samples until drained. `cells`: local dense indices, owned (not halo); duplicates allowed."""
+
+    def __init__(self, domain, cells, capacity=256):
+        self.domain = domain
+        self.cells = np.ascontiguousarray(cells, np.uint64)
+        self.count, self.capacity = int(self.cells.size), int(capacity)
+        self.comps = 5 if domain.thermal else 4
+        self._h = C.c_void_p()
+        A.check(A.lib().luw_probes_create(domain._h, self.count, _ptr(self.cells), self.capacity, C.byref(self._h)))
+
+    def sample(self, t=None):
+        """One sample with the domain's t (or `t`), force and Coriolis, the arguments enqueue_update_fields passes. Stream-ordered, no synchronisation."""
+        d = self.domain
+        A.check(A.lib().luw_probes_sample(self._h, d.t if t is None else int(t), *map(float, d.f), *map(float, d.omega)))
+
+    def drain(self):
+        """-> float32 [samples, comps, count] (rho ux uy uz [T]) of the pending samples, in order; synchronous; clears them."""
+        out = np.empty((self.capacity, self.comps, self.count), np.float32)
+        n = C.c_uint64()
+        A.check(A.lib().luw_probes_drain(self._h, _ptr(out), C.byref(n)))
+        return out[:n.value].copy()
+
+    def reset(self):
+        A.check(A.lib().luw_probes_reset(self._h))
+
+    def close(self):
+        if self._h:
+            A.lib().luw_probes_destroy(self._h)
+            self._h = C.c_void_p()
+
+
 def pinned_empty(count, dtype):
     """numpy array over page-locked host memory (luw_host_alloc). The array keeps the allocation alive through its base object."""
     dtype = np.dtype(dtype)

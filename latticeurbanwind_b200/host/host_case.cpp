@@ -9,6 +9,8 @@
 //   LUW_CASE_STATS; the file gets samples u64, mean_u[3M], comoment[6M], mean_speed[M], m2_speed[M], max_speed[M] f32, exceed[T*M] u32, valid[M] u8, ground[Nx*Ny] u32
 //   LUW_CASE_WALL_OUT=<file> (with LUW_CASE_WALL_GROUND=<ground_z>, default 0): LBM_WallLoads over the same sampling window as LUW_CASE_STATS; the file gets
 //   samples u64, L u32, K u64, series[samples*L*6] f64, ref_points[3L] f64, column_labels[Nx*Ny] u32, cell[K] u64, label[K] u32, mean_F[3K], m2_F[3K] f32
+//   LUW_CASE_PROBES=x0,y0,z0,x1,y1,z1,... (global lattice points) with LUW_CASE_PROBES_OUT=<file>: LBM_Probes sampled after every step of the same window as
+//   LUW_CASE_STATS (capacity LUW_CASE_PROBES_CAP, default 256); the file gets samples u64, comps u32, P u64, t[samples] u64, values[samples*comps*P] f32
 //   with LUW_TEMPERATURE in `features`: in.bin carries T[N] f32 after u, out.bin ends with T[N] f32; alpha / beta of the LBM constructor from LUW_CASE_ALPHA / LUW_CASE_BETA
 #include "lbm.hpp"
 #include <fstream>
@@ -80,7 +82,17 @@ int main(int argc, char** argv) {
 	lbm.run(steps-(samples<steps ? samples : steps));
 	const char* wall_out = getenv("LUW_CASE_WALL_OUT");
 	LBM_WallLoads* wall = wall_out ? new LBM_WallLoads(lbm, getenv("LUW_CASE_WALL_GROUND") ? (uint)atoi(getenv("LUW_CASE_WALL_GROUND")) : 0u) : nullptr;
-	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); stats->accumulate(); if(wind) wind->accumulate(); if(wall) wall->accumulate(); }
+	const char* probes_out = getenv("LUW_CASE_PROBES_OUT");
+	LBM_Probes* probes = probes_out ? new LBM_Probes(lbm, env_list<uint>("LUW_CASE_PROBES"), getenv("LUW_CASE_PROBES_CAP") ? (uint)atoi(getenv("LUW_CASE_PROBES_CAP")) : 256u) : nullptr;
+	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); if(probes) probes->sample(); stats->accumulate(); if(wind) wind->accumulate(); if(wall) wall->accumulate(); }
+	if(probes) {
+		std::vector<float> values;
+		const uint64_t count = (uint64_t)probes->series(values), P = (uint64_t)probes->points;
+		std::ofstream pf(probes_out, std::ios::binary);
+		pf.write((const char*)&count, 8); pf.write((const char*)&probes->comps, 4); pf.write((const char*)&P, 8);
+		pf.write((const char*)probes->t.data(), (std::streamsize)(8u*probes->t.size())); pf.write((const char*)values.data(), (std::streamsize)(4u*values.size()));
+		delete probes;
+	}
 	if(wall) {
 		std::vector<double> series; std::vector<ulong> cell; std::vector<uint> label; std::vector<float> mean_F, m2_F;
 		const uint64_t count = (uint64_t)wall->series(series), K = (uint64_t)(wall->surface(cell, label, mean_F, m2_F), cell.size());

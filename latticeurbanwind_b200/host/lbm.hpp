@@ -775,3 +775,79 @@ public:
 		return (ulong)samples;
 	}
 };
+
+// ---------------------------------------------------------------------------------------------------------------- probe time series
+// rho, u (and T with LUW_TEMPERATURE) at a list of global lattice points, sampled on the device without update_fields over the lattice (luw_probes_*;
+// csrc/lbm_probes.cuh): per sample the values update_fields + a read would give, with t / f / omega taken from each LBM_Domain exactly as
+// enqueue_update_fields takes them. Each point belongs to the one block that owns it (halo layers excluded); a point outside the lattice is an error.
+// The samples stay on the device until `capacity` are pending; then they are drained (the only host synchronisation). The reference reads the whole u field
+// back per probe output instead (FX/setup.cpp:4498-4509). Same semantics as lbm.Probes in Python.
+class LBM_Probes {
+private:
+	LBM* lbm = nullptr;
+	uint capacity = 256u;
+	ulong pending = 0ull;
+	std::vector<luw_probes*> st;
+	std::vector<std::vector<ulong>> slots; // per domain: position in the caller's point list of every listed cell
+	std::vector<float> values; // drained samples [s][c][p], points in the caller's order
+	void drain() {
+		const ulong P = points, SP = (ulong)comps*P;
+		std::vector<float> total(pending*SP), part;
+		uint64_t n = 0ull;
+		for(uint d=0u; d<st.size(); d++) {
+			const ulong K = slots[d].size();
+			part.resize((ulong)capacity*comps*K);
+			luw_check(luw_probes_drain(st[d], part.data(), &n));
+			for(ulong s=0ull; s<n; s++) for(ulong c=0ull; c<comps; c++) for(ulong k=0ull; k<K; k++) total[s*SP+c*P+slots[d][k]] = part[(s*comps+c)*K+k];
+		}
+		values.insert(values.end(), total.begin(), total.end());
+		pending = 0ull;
+	}
+public:
+	ulong points = 0ull;
+	uint comps = 4u; // rho ux uy uz (and T)
+	std::vector<ulong> t; // time step of every sample
+	// xyz[3*p + a]: global lattice coordinates of point p
+	LBM_Probes(LBM& lbm_, const std::vector<uint>& xyz, const uint capacity_=256u) : lbm(&lbm_), capacity(capacity_), points((ulong)xyz.size()/3ull) {
+		comps = LBM_Domain::thermal() ? 5u : 4u;
+		const uint Hx = lbm->get_Dx()>1u, Hy = lbm->get_Dy()>1u, Hz = lbm->get_Dz()>1u;
+		std::vector<std::vector<uint64_t>> cells(lbm->get_D());
+		slots.assign(lbm->get_D(), {});
+		for(ulong p=0ull; p<points; p++) {
+			const uint x = xyz[3ull*p], y = xyz[3ull*p+1ull], z = xyz[3ull*p+2ull];
+			if(x>=lbm->get_Nx()||y>=lbm->get_Ny()||z>=lbm->get_Nz()) print_error("LBM_Probes: point outside the lattice");
+			for(uint d=0u; d<lbm->get_D(); d++) {
+				const LBM_Domain* dom = lbm->lbm_domain[d];
+				const long lx = (long)x-dom->get_Ox(), ly = (long)y-dom->get_Oy(), lz = (long)z-dom->get_Oz();
+				if(lx<(long)Hx||lx>=(long)(dom->get_Nx()-Hx)||ly<(long)Hy||ly>=(long)(dom->get_Ny()-Hy)||lz<(long)Hz||lz>=(long)(dom->get_Nz()-Hz)) continue;
+				cells[d].push_back((uint64_t)lx+((uint64_t)ly+(uint64_t)lz*dom->get_Ny())*dom->get_Nx());
+				slots[d].push_back(p);
+				break;
+			}
+		}
+		for(uint d=0u; d<lbm->get_D(); d++) {
+			luw_probes* h = nullptr;
+			luw_check(luw_probes_create(lbm->lbm_domain[d]->get_handle(), cells[d].size(), cells[d].data(), capacity, &h));
+			st.push_back(h);
+		}
+	}
+	~LBM_Probes() { for(luw_probes* h : st) luw_probes_destroy(h); }
+	LBM_Probes(const LBM_Probes&) = delete;
+	LBM_Probes& operator=(const LBM_Probes&) = delete;
+	void sample() {
+		if(pending==(ulong)capacity) drain();
+		for(uint d=0u; d<lbm->get_D(); d++) {
+			const LBM_Domain* dom = lbm->lbm_domain[d];
+			luw_check(luw_probes_sample(st[d], dom->get_t(), dom->get_fx(), dom->get_fy(), dom->get_fz(), dom->get_omega_x(), dom->get_omega_y(), dom->get_omega_z()));
+		}
+		t.push_back(lbm->lbm_domain[0]->get_t());
+		pending++;
+	}
+	void reset() { for(luw_probes* h : st) luw_check(luw_probes_reset(h)); pending = 0ull; values.clear(); t.clear(); }
+	// out[(s*comps + c)*points + p], c = rho ux uy uz (T), since construction / reset. Returns the sample count.
+	ulong series(std::vector<float>& out) {
+		drain();
+		out = values;
+		return (ulong)t.size();
+	}
+};

@@ -19,6 +19,7 @@ from . import _cabi as A
 from . import cases
 from .domain import CellSet, Domain, WindStats
 from .domain import WallLoads as DomainWallLoads
+from .domain import Probes as DomainProbes
 
 AXES = (0, 1, 2)
 
@@ -416,6 +417,103 @@ class WallLoads:
     def close(self):
         for st in self._loads:
             st.close()
+
+
+def probe_owners(Ng, D, split_offsets, Nl, points):
+    """Which block owns each global point: -> (block [P], local dense index [P]). Halo layers are never owners, so every point of the lattice has exactly one.
+    Raises ValueError for points outside the lattice [0, Ng)."""
+    p = np.asarray(points, np.int64).reshape(-1, 3)
+    if ((p < 0) | (p >= np.asarray(Ng, np.int64))).any():
+        raise ValueError("probe points must lie inside the lattice [0, Ng)")
+    H = np.array([1 if d > 1 else 0 for d in D], np.int64)
+    Nl = np.asarray(Nl, np.int64)
+    block, local = np.full(p.shape[0], -1, np.int64), np.zeros(p.shape[0], np.int64)
+    for b, O in enumerate(split_offsets):
+        q = p - np.asarray(O, np.int64)
+        own = ((q >= H) & (q < Nl - H)).all(axis=1)
+        block[own] = b
+        local[own] = q[own, 0] + (q[own, 1] + q[own, 2] * Nl[1]) * Nl[0]
+    assert (block >= 0).all()
+    return block, local
+
+
+def probe_columns(ground, xy, heights, Nz):
+    """Vertical profiles that follow terrain and roofs: the points (x, y, ground + h) for every column (x, y) of `xy` [M, 2] and height h (cells) of `heights`,
+    ground from global_column_ground (uint32 [Ny, Nx]). A column without ground (0xFFFFFFFF) or whose top point would lie at or above Nz is dropped.
+    -> (points int64 [M_kept * len(heights), 3] ordered [column][height], dropped: indices into xy of the dropped columns)."""
+    g = np.asarray(ground)
+    xy = np.asarray(xy, np.int64).reshape(-1, 2)
+    h = np.asarray(heights, np.int64).reshape(-1)
+    if ((xy < 0) | (xy >= np.array([g.shape[1], g.shape[0]]))).any():
+        raise ValueError("columns must lie inside the lattice")
+    if (h < 0).any():
+        raise ValueError("heights must be non-negative")
+    G = g[xy[:, 1], xy[:, 0]].astype(np.int64)
+    keep = (G != 0xFFFFFFFF) & (G + (h.max() if h.size else 0) < int(Nz))
+    k = np.nonzero(keep)[0]
+    pts = np.empty((k.size, h.size, 3), np.int64)
+    pts[..., 0] = xy[k, 0, None]
+    pts[..., 1] = xy[k, 1, None]
+    pts[..., 2] = G[k, None] + h[None, :]
+    return pts.reshape(-1, 3), np.nonzero(~keep)[0]
+
+
+class Probes:
+    """Time series of rho, u (and T on thermal lattices) at points of an in-process `LBM` (all domains in this process), sampled on the device without
+    update_fields over the lattice (luw_probes_*). `points` [P, 3]: global lattice coordinates (ValueError outside the lattice); each goes to the one block
+    that owns it. sample() takes the values update_fields + a read would give at the current time step; the samples stay on the device until `capacity`
+    are pending, then they are drained (the only host synchronisation). Build it after initialisation (run(0)) when the domains do not store rho / u every
+    step, as update_fields needs DDFs to read. The one-process-per-GPU DistributedLBM is not covered."""
+
+    def __init__(self, lbm, points, capacity=256):
+        self.lbm = lbm
+        self.points = np.asarray(points, np.int64).reshape(-1, 3)
+        self.P, self.capacity = self.points.shape[0], int(capacity)
+        self.comps = 5 if lbm.thermal else 4
+        block, local = probe_owners(lbm.Ng, lbm.D, [O for _, O in lbm._split], lbm.Nl, self.points)
+        self._probes, self._slots = [], []
+        for b, dom in enumerate(lbm.domains):
+            slot = np.nonzero(block == b)[0]
+            self._probes.append(DomainProbes(dom, local[slot], self.capacity))
+            self._slots.append(slot)
+        self._pending = 0
+        self._t, self._series = [], []
+
+    def sample(self):
+        if self._pending == self.capacity:
+            self._drain()
+        for pr in self._probes:
+            pr.sample()
+        self._t.append(self.lbm.domains[0].t)
+        self._pending += 1
+
+    def _drain(self):
+        out = np.empty((self._pending, self.comps, self.P), np.float32)
+        for pr, slot in zip(self._probes, self._slots):
+            out[:, :, slot] = pr.drain()
+        if out.shape[0]:
+            self._series.append(out)
+        self._pending = 0
+
+    def series(self):
+        """-> dict: t int64 [S], rho float32 [S, P], u float32 [S, 3, P] (and T [S, P] on thermal lattices), points in the caller's order, since construction /
+        reset."""
+        self._drain()
+        s = np.concatenate(self._series) if self._series else np.zeros((0, self.comps, self.P), np.float32)
+        out = {"t": np.asarray(self._t, np.int64), "rho": s[:, 0].copy(), "u": s[:, 1:4].copy()}
+        if self.comps == 5:
+            out["T"] = s[:, 4].copy()
+        return out
+
+    def reset(self):
+        for pr in self._probes:
+            pr.reset()
+        self._pending = 0
+        self._t, self._series = [], []
+
+    def close(self):
+        for pr in self._probes:
+            pr.close()
 
 
 class DistributedLBM(_Base):
