@@ -7,6 +7,7 @@
 #include "lbm_wall_loads.cuh"
 #include "vox_bins.h"
 
+#include <climits>
 #include <cmath>
 #include <cstdio>
 #include <cstdlib>
@@ -50,6 +51,7 @@ struct luw_domain {
 	bool tiled = false; // the tiled step is usable for this domain
 	int last_sched_parity = -1; // parity of the last tiled step enqueued (see enqueue_step)
 	int tile_variant = 0, sm_count = 0;
+	luw::TileShape tile_shape = {}; // box of tile_variant
 	struct HaloAxis { // transfer buffers of one decomposed axis (reference: transfer_buffer_p / _m, FX/lbm.cpp:1864-1889) and the events that order their use
 		char* send_p = nullptr; char* send_m = nullptr; char* recv_p = nullptr; char* recv_m = nullptr;
 		uint64_t bytes = 0ull;
@@ -199,35 +201,23 @@ encode_tiled_fn get_encode_tiled() {
 	}
 	return fn;
 }
-// Build the TMA descriptors of a domain for the tile shape of the selected variant. Leaves d->tiled false when the lattice cannot be
+// Build the TMA descriptors of a domain for the tile shape of the selected variant (KernelSet::choose_tile). Leaves d->tiled false when the lattice cannot be
 // described (row pitch not a multiple of 16 bytes for every array) -- the per-cell kernels are used then.
 void setup_tiles(luw_domain* d) {
 	d->tiled = false;
 	const char* off = getenv("LUW_NO_TILE");
 	if(off&&off[0]=='1') return;
 	const char* var = getenv("LUW_TILE_VARIANT");
-	// default (measured, profiles/r2_variant_sweeps.txt): FP16S and FP16C -> the lean-loop two-pass kernel, 128x4 tiles with 8 consumer warps per producer for the LES step (V5),
-	// 128x2 tiles and 5 CTAs/SM without LES (V6) -- for FP16C too since the lean loop: 55.8 (V6) / 51.4 (V5) against 48.2 GLUP/s (single-pass V3) on the channel, 38.9 against 31.2 on
-	// the urban LES step with UPDATE_FIELDS; FP32 -> single pass (V0) without LES (HBM-bound: 0.98 of the copy peak on the channel); for the LES step the two-pass kernels:
-	// the lean loop (V5) on large lattices (512 x 512 x 256 with UPDATE_FIELDS: 35.8 GLUP/s = 0.84 of the copy peak at 153 B per cell, V1 34.9, V0 30.0), its general-loop twin (V1)
-	// on small ones (C1-sized 256 x 256 x 128: 27.7, V5 27.3, V0 24.5; profiles/r2_variant_sweeps.txt calls Z / ZA).
-	// STRICT arithmetic runs k_stream_collide_tile on the same tile shapes.
-	const bool large = (uint64_t)d->c.Nx*d->c.Ny*d->c.Nz>=(1ull<<25);
-	const int want = (var&&var[0]) ? atoi(var) : d->c.precision==luw::P_FP32 ? ((d->c.features&luw::F_SUBGRID) ? (large ? 5 : 1) : 0) : ((d->c.features&luw::F_SUBGRID) ? 5 : 6);
 	const luw::DomainConst& c = d->c;
 	// odd Nx: the row's last pair holds one cell (rows are padded to Px, a multiple of 16 elements); lbm_tile.cuh `odd_end`
 	encode_tiled_fn enc = get_encode_tiled();
 	if(!enc) return;
-	luw::TileShape sh;
-	bool found = false;
-	const int fallback = d->c.precision==luw::P_FP32 ? 0 : 5; // thermal domains: the one variant per precision their momentum kernel is built for
-	// FP32 LES: the single-pass and the two-pass kernels differ in their FAST roundings, so a narrow block of a decomposition must not drop to single pass (V0 / V2) while the
-	// others run two-pass: its fallbacks are the two-pass variants (V1, 64-wide V7) first. Thermal FP32 domains have V0 only and take it on every block alike.
-	const bool fp32_les = !(var&&var[0])&&d->c.precision==luw::P_FP32&&(d->c.features&luw::F_SUBGRID)&&!(d->c.features&luw::F_TEMPERATURE);
-	for(int v : { want, fp32_les ? 1 : fallback, fp32_les ? 7 : 0, fp32_les ? 0 : 2, 2 }) { // 2: 64-wide tiles for narrow lattices // the requested variant, else one whose tile is not wider than the lattice
-		if(d->ks->tile_shape(c.precision, c.features, v, &sh)&&c.Nx>=(uint32_t)sh.tx) { d->tile_variant = v; found = true; break; }
-	}
-	if(!found) return;
+	int want = -1; // the default
+	if(var&&var[0]) want = atoi(var)>=0 ? atoi(var) : INT_MAX; // a negative request names no variant: it falls back like any other that is not built
+	const int v = d->ks->choose_tile(c.precision, c.features, c.Nx, c.Ny, c.Nz, want, &d->tile_shape);
+	if(v<0) return;
+	d->tile_variant = v;
+	const luw::TileShape& sh = d->tile_shape;
 	const cuuint64_t es = d->ddf_size;
 	const CUtensorMapDataType dt = es==4u ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_UINT16;
 	const cuuint64_t dims4[4] = { c.Nx, c.Ny, c.Nz, 19u };
@@ -810,9 +800,9 @@ __global__ void k_boundary_wait(const uint32_t* ctr, const uint32_t target) {
 }
 // Strip order of an overlapped step (DomainConst::so_*): the tile rows / planes that hold layers 0, 1, N-2, N-1 of the decomposed y / z axes. false: no interior left to overlap with.
 static bool halo_strip_order(const luw_domain* d, luw::DomainConst* o, uint32_t* per_strip) {
-	luw::TileShape sh;
-	if(!d->tiled||!d->ks->tile_shape(d->c.precision, d->c.features, d->tile_variant, &sh)) return false;
+	if(!d->tiled) return false;
 	const luw::DomainConst& c = d->c;
+	const luw::TileShape& sh = d->tile_shape;
 	const uint32_t TY = (uint32_t)sh.ty, TZ = (uint32_t)sh.tz, Tx = (c.Nx+(uint32_t)sh.tx-1u)/(uint32_t)sh.tx;
 	*o = c;
 	if(!luw::strip_order_fill(*o, TY, TZ)) return false;
@@ -1408,11 +1398,7 @@ int luw_wall_loads_accumulate(luw_wall_loads* st, uint64_t t) {
 	const uint32_t odd = (uint32_t)(t&1ull);
 	if(st->count>0ull) {
 		const unsigned g = list_grid(d, st->count);
-		switch(d->c.precision) {
-			case luw::P_FP32: luw::k_wall_cells<luw::P_FP32><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); break;
-			case luw::P_FP16S: luw::k_wall_cells<luw::P_FP16S><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); break;
-			default: luw::k_wall_cells<luw::P_FP16C><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); break;
-		}
+		luw::with_precision(d->c.precision, [&](auto p) { luw::k_wall_cells<decltype(p)::value><<<g, 256, 0, d->stream>>>(d->c, st->count, st->cell, st->links, odd, inv_n, st->F, st->acc); });
 		CU(cudaGetLastError());
 		luw::k_wall_chunks<<<list_grid(d, st->nchunks), 256, 0, d->stream>>>(d->c, st->count, st->nchunks, st->chunk_begin, st->chunk_label, st->cell, st->F, st->ref, st->partial);
 		CU(cudaGetLastError());

@@ -5,7 +5,7 @@
 #include "../../latticeurbanwind_b200/csrc/vox_bins.h"
 using namespace luw;
 
-// one "launch": grid (ceil(Nx/tx), Ny, Nz) x block tx, as cell_grid() / pick_tx() of lbm_launch.inc
+// one "launch": grid (ceil(Nx/tx), Ny, Nz) x block tx, as launch_cells() of lbm_launch.inc
 template<class K> static void for_cells(const DomainConst& c, K kernel) {
 	const unsigned tx = c.Nx>=128u ? 128u : c.Nx>=64u ? 64u : 32u, gx = (c.Nx+tx-1u)/tx;
 #pragma omp parallel for collapse(2) schedule(static)

@@ -139,7 +139,7 @@ def test_tiled_fast_within_tolerance(oracle_lib, precision, fset):
 
 # ---------------------------------------------------------------------------------------------- the instantiations bench.py times
 # bench.py's workloads: "chan" (FEAT = 4, channel case: TYPE_E x faces, TYPE_S walls) and "luwnf" / "luw" (FEAT = 14 / 15, urban case), FAST arithmetic, the tile
-# variant the dispatcher picks (csrc/luw_cabi.cu setup_tiles). Every variant the dispatcher can pick is pinned here, STRICT bit for bit and FAST within tolerance.
+# variant the dispatcher picks (csrc/lbm_launch.inc choose_tile). Every variant the dispatcher can pick is pinned here, STRICT bit for bit and FAST within tolerance.
 BENCH_CASES = {"chan": ("channel", 1.0 / 6.0), "luwnf": ("urban", 1e-6), "luw": ("urban", 1e-6)}
 BENCH_VARIANTS = [0, 1, 3, 4, 5]  # V0 / V1 two-pass 128x2, V3 single-pass, V4 two-pass 128x4, V5 the lean-loop kernel (default for FAST two-pass configurations)
 BENCH_ZONES = dict(downstream_face=2, buffer_N=5, buffer_inv_tau=0.01, buffer_nudge_vertical=1, sponge_N=4, sponge_inv_tau=0.02)
@@ -201,7 +201,7 @@ def test_fast_result_does_not_depend_on_the_tile_variant(monkeypatch, variant, s
 @pytest.mark.parametrize("variant,shape", [(5, (256, 24, 12)), (7, (256, 24, 12))], ids=["V5-lean", "V7-64wide"])
 def test_fp32_two_pass_variants_agree(monkeypatch, variant, shape):
     """The FP32 LES step runs two-pass by default (V1; the lean loop V5 on large lattices; V7 = two-pass on 64-wide tiles for blocks narrower than 128 cells,
-    csrc/luw_cabi.cu setup_tiles): all three must produce V1's bits, or a decomposed FP32 run would depend on how wide its blocks are."""
+    csrc/lbm_launch.inc choose_tile): all three must produce V1's bits, or a decomposed FP32 run would depend on how wide its blocks are."""
     flags, rho, u, w = _bench_case("luw", shape)
     res = []
     for v in (1, variant):
@@ -212,7 +212,7 @@ def test_fp32_two_pass_variants_agree(monkeypatch, variant, shape):
 
 @pytest.mark.parametrize("arith", [0, 1], ids=["strict", "fast"])
 def test_fp32_les_on_a_narrow_lattice_takes_the_64_wide_two_pass_tiles(oracle_lib, monkeypatch, arith):
-    """66 cells wide (a block of a 128-cell lattice split in x): no explicit variant, so setup_tiles falls through V1 to V7. STRICT equals the oracle bit for bit, FAST within tolerance."""
+    """66 cells wide (a block of a 128-cell lattice split in x): no explicit variant, so choose_tile falls through V1 to V7. STRICT equals the oracle bit for bit, FAST within tolerance."""
     O = oracle_lib
     monkeypatch.delenv("LUW_TILE_VARIANT", raising=False)
     shape = (66, 24, 12)
