@@ -12,6 +12,7 @@
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
+#include <memory>
 #include <new>
 #include <string>
 #include <vector>
@@ -34,6 +35,46 @@ struct DeviceGuard { // every entry point may be called with any current device;
 	~DeviceGuard() { if(prev>=0) cudaSetDevice(prev); }
 };
 
+// Owner of device arrays and events: frees all of them when it goes. While an array lives its bytes are counted in *charge (a domain's luw_domain_bytes);
+// per-call scratch has no charge. A count of 0 allocates one element.
+class DeviceMemory {
+public:
+	uint64_t* charge;
+	explicit DeviceMemory(uint64_t* charge_ = nullptr) : charge(charge_) {}
+	DeviceMemory(const DeviceMemory&) = delete;
+	DeviceMemory& operator=(const DeviceMemory&) = delete;
+	~DeviceMemory() {
+		for(const Array& a : arrays) { cudaFree(a.ptr); if(charge) *charge -= a.bytes; }
+		for(const cudaEvent_t ev : events) cudaEventDestroy(ev);
+	}
+	template<typename T> cudaError_t alloc(T** ptr, const uint64_t count) {
+		const uint64_t bytes = (count>0ull ? count : 1ull)*sizeof(T);
+		const cudaError_t e = cudaMalloc((void**)ptr, bytes);
+		if(e!=cudaSuccess) { *ptr = nullptr; return e; }
+		arrays.push_back({ (void*)*ptr, bytes });
+		if(charge) *charge += bytes;
+		return cudaSuccess;
+	}
+	template<typename T> cudaError_t upload(T** ptr, const T* host, const uint64_t count, const cudaStream_t stream) { // alloc, then an H2D copy of `count` elements
+		const cudaError_t e = alloc(ptr, count);
+		return e==cudaSuccess&&count>0ull ? cudaMemcpyAsync(*ptr, host, count*sizeof(T), cudaMemcpyHostToDevice, stream) : e;
+	}
+	cudaError_t event(cudaEvent_t* ev, const unsigned flags = cudaEventDisableTiming) {
+		const cudaError_t e = cudaEventCreateWithFlags(ev, flags);
+		if(e!=cudaSuccess) { *ev = nullptr; return e; }
+		events.push_back(*ev);
+		return cudaSuccess;
+	}
+	void take(DeviceMemory& from) { // from's arrays and events become mine; both must have the same charge
+		arrays.insert(arrays.end(), from.arrays.begin(), from.arrays.end()); from.arrays.clear();
+		events.insert(events.end(), from.events.begin(), from.events.end()); from.events.clear();
+	}
+private:
+	struct Array { void* ptr; uint64_t bytes; };
+	std::vector<Array> arrays;
+	std::vector<cudaEvent_t> events;
+};
+
 } // namespace
 
 struct luw_domain {
@@ -43,8 +84,8 @@ struct luw_domain {
 	cudaStream_t own_stream = nullptr, stream = nullptr;
 	cudaStream_t copy_stream = nullptr; // H2D / D2H of cell sets, overlapping the kernels on `stream`
 	cudaEvent_t ev0 = nullptr, ev1 = nullptr;
-	float* wbuf = nullptr; float* sigma = nullptr;
 	uint64_t bytes = 0ull, launches = 0ull;
+	DeviceMemory mem{&bytes}; // every device array and event of the domain
 	uint64_t ncells = 0ull; // Nx*Ny*Nz: cells of the lattice = elements per component of a HOST image (the device arrays have c.N = Px*Ny*Nz, see lbm_common.cuh)
 	size_t ddf_size = 4u;
 	luw::TileMaps maps; // TMA descriptors for the tiled step
@@ -75,8 +116,10 @@ struct luw_domain {
 	std::vector<cudaEvent_t> kev; // event pairs
 	size_t kev_used = 0u;
 };
+// The companion objects of a domain: each owns its device arrays and events in `mem`, charged to the domain, and is destroyed before the domain.
 struct luw_cellset {
 	luw_domain* dom;
+	DeviceMemory mem;
 	uint64_t count;
 	uint64_t* cell; // device: local cell indices
 	// Copies run on the domain's copy stream so that they overlap the step kernel; only the small scatter / gather kernels sit on the domain's stream.
@@ -88,12 +131,14 @@ struct luw_cellset {
 };
 struct luw_stats {
 	luw_domain* dom;
+	DeviceMemory mem;
 	uint64_t count;
 	float* mean_u; float* m2_u; float* mean_rho; // device, pitched like u / rho: [c*c.N + n]
 	float* mean_T; // LUW_TEMPERATURE domains: running mean of T (avg_T, FX/setup.cpp:4449-4451, 4481-4486); nullptr otherwise
 };
 struct luw_wind_stats {
 	luw_domain* dom;
+	DeviceMemory mem;
 	uint64_t count, samples;
 	uint64_t* cell; // device indices of the listed cells
 	float* acc; // [j*count + k], j < luw::WIND_FLOAT_ACCUMULATORS (lbm_wind_stats.cuh)
@@ -102,6 +147,7 @@ struct luw_wind_stats {
 };
 struct luw_wall_loads {
 	luw_domain* dom;
+	DeviceMemory mem;
 	uint64_t count, nchunks, samples, pending, capacity;
 	uint32_t L, periodic;
 	uint64_t* cell; // device indices of the listed cells, sorted by (label, index)
@@ -119,6 +165,7 @@ struct luw_wall_loads {
 };
 struct luw_probes {
 	luw_domain* dom;
+	DeviceMemory mem;
 	uint64_t count, pending, capacity;
 	uint32_t comps; // 4: rho ux uy uz; 5: and T
 	uint64_t* cell; // device indices of the listed cells
@@ -126,6 +173,7 @@ struct luw_probes {
 };
 struct luw_vk_inlet {
 	luw_domain* dom;
+	DeviceMemory mem;
 	uint64_t P, M, V;
 	uint64_t* point_cell; uint8_t* point_face; float* point_data; float* mode_data;
 	float* mode_cs; // [6*V]: A cos(phi), A sin(phi) per component, for the FAST kernel
@@ -183,10 +231,31 @@ cudaError_t copy_field(luw_domain* d, char* dev_base, const size_t elem, char* h
 uint64_t face_area(const luw::DomainConst& c, const uint32_t axis) {
 	return axis==0u ? (uint64_t)c.Ny*c.Nz : axis==1u ? (uint64_t)c.Nz*c.Nx : (uint64_t)c.Nx*c.Ny;
 }
-template<typename T> int dev_alloc(luw_domain* d, T** ptr, const uint64_t count) {
-	const cudaError_t e = cudaMalloc((void**)ptr, count*sizeof(T));
-	if(e!=cudaSuccess) { *ptr = nullptr; return cuda_fail(e, "cudaMalloc"); }
-	d->bytes += count*sizeof(T);
+// grid of the whole-lattice grid-stride kernels: 8 blocks per SM (1184 while the SM count is not known yet, which is 8 x the 148 SMs of a B200)
+unsigned lattice_grid(const luw_domain* d) { return d->sm_count>0 ? 8u*(unsigned)d->sm_count : 1184u; }
+// grid of a kernel over a list of `items`: one block of 256 threads per 256 items, at least 1 and at most the lattice grid
+unsigned list_grid(const luw_domain* d, const uint64_t items) {
+	const uint64_t want = (items+255ull)/256ull, cap = lattice_grid(d);
+	return (unsigned)(want<1ull ? 1ull : want<cap ? want : cap);
+}
+// the cells a domain owns: the halo layer at each end of a decomposed axis belongs to the neighbours
+struct Box { uint32_t x0, x1, y0, y1, z0, z1; };
+Box owned_box(const luw::DomainConst& c) {
+	const uint32_t hx = c.Dx>1u ? 1u : 0u, hy = c.Dy>1u ? 1u : 0u, hz = c.Dz>1u ? 1u : 0u;
+	return { hx, c.Nx-hx, hy, c.Ny-hy, hz, c.Nz-hz };
+}
+// Device indices of a host list of dense cell indices: each must lie in the lattice and, with `owned`, outside the halo layers.
+int device_cells(const luw_domain* d, const uint64_t* host, const uint64_t count, const bool owned, std::vector<uint64_t>& out) {
+	const luw::DomainConst& c = d->c;
+	const Box b = owned_box(c);
+	out.resize(count);
+	for(uint64_t k=0ull; k<count; k++) {
+		const uint64_t n = host[k];
+		if(n>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
+		const uint32_t x = (uint32_t)(n%c.Nx), y = (uint32_t)((n/c.Nx)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Nx*c.Ny));
+		if(owned&&(x<b.x0||x>=b.x1||y<b.y0||y>=b.y1||z<b.z0||z>=b.z1)) return fail(LUW_ERR_INVALID, "cell index in a halo layer");
+		out[k] = device_index(c, n);
+	}
 	return LUW_OK;
 }
 // cuTensorMapEncodeTiled through the runtime's driver entry point (no link-time dependency on libcuda)
@@ -245,7 +314,7 @@ cudaError_t enqueue_step(luw_domain* d, const luw::StepArgs& a, const luw::Domai
 		d->last_sched_parity = par;
 	}
 	if(d->ktiming) { // event pair around the main kernel
-		if(d->kev_used+2u>d->kev.size()) for(int k=0; k<2; k++) { cudaEvent_t ev; e = cudaEventCreate(&ev); if(e!=cudaSuccess) return e; d->kev.push_back(ev); }
+		if(d->kev_used+2u>d->kev.size()) for(int k=0; k<2; k++) { cudaEvent_t ev; e = d->mem.event(&ev, cudaEventDefault); if(e!=cudaSuccess) return e; d->kev.push_back(ev); }
 		e = cudaEventRecord(d->kev[d->kev_used], d->stream); if(e!=cudaSuccess) return e;
 	}
 	// thermal domains: momentum in the tiled kernel (which leaves the pre-force velocity in c.upre) + the TEMPERATURE block as a second kernel -- unless the buoyancy
@@ -342,11 +411,6 @@ __global__ void k_fill_f32(float* p, const uint64_t n, const float v) {
 
 // Inflow-sample searches (lbm_inlet.cuh): host buffers in, host buffers out, cells in batches so that the kept-sample table (256 B per cell) stays bounded.
 namespace {
-struct DeviceBuffers { // released on every exit path
-	std::vector<void*> p;
-	~DeviceBuffers() { for(void* q : p) cudaFree(q); }
-	template<typename T> cudaError_t get(T** out, const uint64_t count) { *out = nullptr; const cudaError_t e = cudaMalloc((void**)out, (count>0ull ? count : 1ull)*sizeof(T)); if(e==cudaSuccess) p.push_back((void*)*out); return e; }
-};
 constexpr uint64_t kInletBatch = 1ull<<20;
 uint64_t g_inlet_launches = 0ull;
 } // namespace
@@ -397,7 +461,7 @@ int luw_domain_create(const luw_domain_params* p, luw_domain** out) {
 	if(guard.err!=cudaSuccess) return cuda_fail(guard.err, "cudaSetDevice");
 
 	if(p->Dx*p->Dy*p->Dz>1u) enable_peer_access(p->device, ndev);
-	luw_domain* d = new(std::nothrow) luw_domain();
+	std::unique_ptr<luw_domain, int(*)(luw_domain*)> d(new(std::nothrow) luw_domain(), luw_domain_destroy);
 	if(!d) return fail(LUW_ERR_OOM, "host allocation failed");
 	d->p = *p;
 	d->ks = p->arith==LUW_ARITH_STRICT ? &luw::kernels_strict() : &luw::kernels_fast();
@@ -417,53 +481,58 @@ int luw_domain_create(const luw_domain_params* p, luw_domain** out) {
 	c.sponge_N = p->sponge_N;
 	c.w_T = 1.0f; c.beta = 0.0f; c.T_avg = 1.0f; // luw_thermal_params
 
-	int rc = LUW_OK;
-	cudaError_t e = cudaStreamCreateWithFlags(&d->own_stream, cudaStreamNonBlocking);
-	if(e==cudaSuccess) e = cudaStreamCreateWithFlags(&d->copy_stream, cudaStreamNonBlocking);
-	if(e==cudaSuccess) e = cudaEventCreate(&d->ev0);
-	if(e==cudaSuccess) e = cudaEventCreate(&d->ev1);
-	if(e!=cudaSuccess) rc = cuda_fail(e, "stream/event creation");
+	CU(cudaStreamCreateWithFlags(&d->own_stream, cudaStreamNonBlocking));
 	d->stream = d->own_stream;
-	if(rc==LUW_OK) rc = dev_alloc(d, (uint8_t**)&c.fi, 19ull*N*d->ddf_size);
-	if(rc==LUW_OK) rc = dev_alloc(d, &c.rho, N);
-	if(rc==LUW_OK) rc = dev_alloc(d, &c.u, 3ull*N);
-	if(rc==LUW_OK) rc = dev_alloc(d, &c.flags, N);
-	if(rc==LUW_OK) rc = dev_alloc(d, &c.sched, 4u); // [0], [1]: strip counters of the two step parities; [2]: boundary-strip counter of the overlapped halo exchange (c.bdone)
+	CU(cudaStreamCreateWithFlags(&d->copy_stream, cudaStreamNonBlocking));
+	DeviceMemory& m = d->mem;
+	CU(m.event(&d->ev0, cudaEventDefault));
+	CU(m.event(&d->ev1, cudaEventDefault));
+	CU(m.alloc((uint8_t**)&c.fi, 19ull*N*d->ddf_size));
+	CU(m.alloc(&c.rho, N));
+	CU(m.alloc(&c.u, 3ull*N));
+	CU(m.alloc(&c.flags, N));
+	CU(m.alloc(&c.sched, 4u)); // [0], [1]: strip counters of the two step parities; [2]: boundary-strip counter of the overlapped halo exchange (c.bdone)
+	c.bdone = c.sched+2;
 	const bool thermal = (p->features&LUW_TEMPERATURE)!=0u;
-	if(rc==LUW_OK&&thermal) rc = dev_alloc(d, (uint8_t**)&c.gi, 7ull*N*d->ddf_size); // gi = Memory<fpxx>(N, 7), T = Memory<float>(N, 1, .., 1.0f): FX/lbm.cpp:322-323
-	if(rc==LUW_OK&&thermal) rc = dev_alloc(d, &c.T, N);
-	if(rc==LUW_OK&&thermal) rc = dev_alloc(d, &c.upre, 3ull*N); // two-kernel thermal step: the pre-force velocity handed from the momentum kernel to k_thermal_g (+12 B per cell)
-	if(rc==LUW_OK) { // Memory<> zero-fills; rho starts at 1 (FX/lbm.cpp:283-288)
-		e = cudaMemsetAsync(c.fi, 0, 19ull*N*d->ddf_size, d->stream);
-		if(e==cudaSuccess) e = cudaMemsetAsync(c.u, 0, 3ull*N*4ull, d->stream);
-		if(e==cudaSuccess) e = cudaMemsetAsync(c.flags, 0, N, d->stream);
-		if(e==cudaSuccess) e = cudaMemsetAsync(c.sched, 0, 16u, d->stream);
-		if(e==cudaSuccess) { k_fill_f32<<<1184, 256, 0, d->stream>>>(c.rho, N, 1.0f); e = cudaGetLastError(); d->launches++; }
-		if(e==cudaSuccess&&thermal) e = cudaMemsetAsync(c.gi, 0, 7ull*N*d->ddf_size, d->stream);
-		if(e==cudaSuccess&&thermal) { k_fill_f32<<<1184, 256, 0, d->stream>>>(c.T, N, 1.0f); e = cudaGetLastError(); d->launches++; }
-		if(e!=cudaSuccess) rc = cuda_fail(e, "zero-fill");
+	if(thermal) {
+		CU(m.alloc((uint8_t**)&c.gi, 7ull*N*d->ddf_size)); // gi = Memory<fpxx>(N, 7), T = Memory<float>(N, 1, .., 1.0f): FX/lbm.cpp:322-323
+		CU(m.alloc(&c.T, N));
+		CU(m.alloc(&c.upre, 3ull*N)); // two-kernel thermal step: the pre-force velocity handed from the momentum kernel to k_thermal_g (+12 B per cell)
 	}
-	if(rc==LUW_OK&&(p->features&LUW_BUFFER_NUDGING)) { // distance -> sin^2 ramp, float arithmetic as written in FX/kernel.cpp:1579-1581
+	// Memory<> zero-fills; rho starts at 1 (FX/lbm.cpp:283-288)
+	CU(cudaMemsetAsync(c.fi, 0, 19ull*N*d->ddf_size, d->stream));
+	CU(cudaMemsetAsync(c.u, 0, 3ull*N*4ull, d->stream));
+	CU(cudaMemsetAsync(c.flags, 0, N, d->stream));
+	CU(cudaMemsetAsync(c.sched, 0, 16u, d->stream));
+	k_fill_f32<<<lattice_grid(d.get()), 256, 0, d->stream>>>(c.rho, N, 1.0f);
+	CU(cudaGetLastError());
+	d->launches++;
+	if(thermal) {
+		CU(cudaMemsetAsync(c.gi, 0, 7ull*N*d->ddf_size, d->stream));
+		k_fill_f32<<<lattice_grid(d.get()), 256, 0, d->stream>>>(c.T, N, 1.0f);
+		CU(cudaGetLastError());
+		d->launches++;
+	}
+	if(p->features&LUW_BUFFER_NUDGING) { // distance -> sin^2 ramp, float arithmetic as written in FX/kernel.cpp:1579-1581
 		std::vector<float> t(p->buffer_N+1u);
 		for(uint32_t k=0u; k<=p->buffer_N; k++) { const float xi = 1.0f-(float)k/(float)p->buffer_N; float wb = sinf(1.5707963267948966f*xi); wb *= wb; t[k] = wb; }
-		rc = dev_alloc(d, &d->wbuf, t.size());
-		if(rc==LUW_OK) { e = cudaMemcpyAsync(d->wbuf, t.data(), t.size()*4u, cudaMemcpyHostToDevice, d->stream); if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); if(e!=cudaSuccess) rc = cuda_fail(e, "upload nudging table"); }
+		float* wbuf;
+		CU(m.upload(&wbuf, t.data(), t.size(), d->stream));
+		CU(cudaStreamSynchronize(d->stream));
+		c.wbuf = wbuf;
 	}
-	if(rc==LUW_OK&&(p->features&LUW_TOP_SPONGE)) { // depth -> inv_tau*sin^2 ramp, FX/kernel.cpp:1602-1605
+	if(p->features&LUW_TOP_SPONGE) { // depth -> inv_tau*sin^2 ramp, FX/kernel.cpp:1602-1605
 		std::vector<float> t(p->sponge_N);
 		const int Ns = (int)p->sponge_N;
 		for(int k=0; k<Ns; k++) { const float xi = Ns>1 ? 1.0f-(float)k/(float)(Ns-1) : 1.0f; float sg = sinf(1.5707963267948966f*xi); sg = p->sponge_inv_tau*sg*sg; t[(size_t)k] = sg; }
-		rc = dev_alloc(d, &d->sigma, t.size());
-		if(rc==LUW_OK) { e = cudaMemcpyAsync(d->sigma, t.data(), t.size()*4u, cudaMemcpyHostToDevice, d->stream); if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); if(e!=cudaSuccess) rc = cuda_fail(e, "upload sponge table"); }
+		float* sigma;
+		CU(m.upload(&sigma, t.data(), t.size(), d->stream));
+		CU(cudaStreamSynchronize(d->stream));
+		c.sigma = sigma;
 	}
-	c.wbuf = d->wbuf; c.sigma = d->sigma;
-	c.bdone = c.sched ? c.sched+2 : nullptr;
-	if(rc==LUW_OK) {
-		cudaDeviceGetAttribute(&d->sm_count, cudaDevAttrMultiProcessorCount, p->device);
-		setup_tiles(d);
-	}
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_domain_destroy(d); g_error = keep; return rc; }
-	*out = d;
+	cudaDeviceGetAttribute(&d->sm_count, cudaDevAttrMultiProcessorCount, p->device);
+	setup_tiles(d.get());
+	*out = d.release();
 	return LUW_OK;
 }
 
@@ -471,29 +540,14 @@ int luw_domain_destroy(luw_domain* d) {
 	if(!d) return LUW_OK;
 	DeviceGuard guard(d->p.device);
 	if(d->own_stream) cudaStreamSynchronize(d->own_stream);
-	cudaFree(d->c.fi); cudaFree(d->c.rho); cudaFree(d->c.u); cudaFree(d->c.flags); cudaFree(d->c.sched); cudaFree(d->wbuf); cudaFree(d->sigma); cudaFree(d->c.gi); cudaFree(d->c.T); cudaFree(d->c.upre);
 	if(d->halo_stream) { cudaStreamSynchronize(d->halo_stream); cudaStreamDestroy(d->halo_stream); }
-	if(d->halo_done) cudaEventDestroy(d->halo_done);
-	if(d->ev0) cudaEventDestroy(d->ev0);
-	if(d->ev1) cudaEventDestroy(d->ev1);
-	for(cudaEvent_t ev : d->kev) cudaEventDestroy(ev);
-	for(int a=0; a<3; a++) {
-		luw_domain::HaloAxis& h = d->halo[a];
-		cudaFree(h.send_p); cudaFree(h.send_m); cudaFree(h.recv_p); cudaFree(h.recv_m);
-		if(h.extracted) cudaEventDestroy(h.extracted);
-		if(h.inserted) cudaEventDestroy(h.inserted);
-		if(h.got_p) cudaEventDestroy(h.got_p);
-		if(h.got_m) cudaEventDestroy(h.got_m);
-	}
-	for(int a=0; a<3; a++) {
-		luw_domain::HaloIpc& h = d->ipc[a];
+	for(const luw_domain::HaloIpc& h : d->ipc) {
 		if(h.up) cudaIpcCloseMemHandle(h.up);
 		if(h.dn&&!h.same) cudaIpcCloseMemHandle(h.dn);
-		cudaFree(h.block);
 	}
 	if(d->copy_stream) { cudaStreamSynchronize(d->copy_stream); cudaStreamDestroy(d->copy_stream); }
 	if(d->own_stream) cudaStreamDestroy(d->own_stream);
-	delete d;
+	delete d; // d->mem frees the device arrays and events
 	return LUW_OK;
 }
 
@@ -620,20 +674,21 @@ int luw_halo_extract(luw_domain* d, int payload, uint32_t axis, uint64_t t, void
 int luw_halo_insert(luw_domain* d, int payload, uint32_t axis, uint64_t t, const void* bp, const void* bm) { return halo(d, payload, axis, t, (void*)bp, (void*)bm, true); }
 
 static int halo_axis_setup(luw_domain* d, const uint32_t axis) { // buffers sized for the larger payload (rho_u_flags: 17 B per face cell >= 5 fpxx for FP16; FP32: 20 B)
-	luw_domain::HaloAxis& h = d->halo[axis];
-	if(h.send_p) return LUW_OK;
+	if(d->halo[axis].send_p) return LUW_OK;
 	DeviceGuard guard(d->p.device);
-	const uint64_t A = face_area(d->c, axis);
-	h.bytes = A*(d->ddf_size==4u ? 20ull : 17ull);
-	int rc = dev_alloc(d, &h.send_p, h.bytes);
-	if(rc==LUW_OK) rc = dev_alloc(d, &h.send_m, h.bytes);
-	if(rc==LUW_OK) rc = dev_alloc(d, &h.recv_p, h.bytes);
-	if(rc==LUW_OK) rc = dev_alloc(d, &h.recv_m, h.bytes);
-	if(rc!=LUW_OK) return rc;
-	CU(cudaEventCreateWithFlags(&h.extracted, cudaEventDisableTiming));
-	CU(cudaEventCreateWithFlags(&h.got_p, cudaEventDisableTiming));
-	CU(cudaEventCreateWithFlags(&h.got_m, cudaEventDisableTiming));
-	CU(cudaEventCreateWithFlags(&h.inserted, cudaEventDisableTiming));
+	luw_domain::HaloAxis h; // built aside and handed over complete: after a failure the axis is still unset
+	DeviceMemory mem(&d->bytes);
+	h.bytes = face_area(d->c, axis)*(d->ddf_size==4u ? 20ull : 17ull);
+	CU(mem.alloc(&h.send_p, h.bytes));
+	CU(mem.alloc(&h.send_m, h.bytes));
+	CU(mem.alloc(&h.recv_p, h.bytes));
+	CU(mem.alloc(&h.recv_m, h.bytes));
+	CU(mem.event(&h.extracted));
+	CU(mem.event(&h.got_p));
+	CU(mem.event(&h.got_m));
+	CU(mem.event(&h.inserted));
+	d->mem.take(mem);
+	d->halo[axis] = h;
 	return LUW_OK;
 }
 // can a kernel on device `a` store into memory of device `b`? (peer access is switched on by luw_domain_create for every pair that allows it)
@@ -741,7 +796,7 @@ int luw_halo_ipc_export(luw_domain* d, uint32_t axis, void* handle_out) {
 		const uint64_t A = face_area(d->c, axis);
 		h->buf_bytes = (A*(d->ddf_size==4u ? 20ull : 17ull)+255ull)&~255ull; // the larger payload: 5 fpxx or rho_u_flags (17 B) per face cell
 		const uint64_t bytes = 256ull+4ull*h->buf_bytes;
-		if(const int rc = dev_alloc(d, &h->block, bytes)) return rc;
+		CU(d->mem.alloc(&h->block, bytes));
 		CU(cudaMemsetAsync(h->block, 0, bytes, d->stream));
 		CU(cudaStreamSynchronize(d->stream));
 	}
@@ -828,8 +883,8 @@ int luw_step_halo_ipc(luw_domain* d, uint64_t t, float fx, float fy, float fz, f
 	if(!d->halo_stream) {
 		int lo = 0, hi = 0;
 		CU(cudaDeviceGetStreamPriorityRange(&lo, &hi));
+		CU(d->mem.event(&d->halo_done)); // before the stream, whose presence marks the pair as set up
 		CU(cudaStreamCreateWithPriority(&d->halo_stream, cudaStreamNonBlocking, hi)); // its small kernels go ahead of the step kernel's remaining CTAs... which are resident anyway: they only need free thread slots
-		CU(cudaEventCreateWithFlags(&d->halo_done, cudaEventDisableTiming));
 	}
 	CU(enqueue_step(d, a, &order)); // boundary strips first, counted in *c.bdone
 	d->bdone_target += order.so_nb*per_strip;
@@ -865,41 +920,28 @@ int luw_run_steps_multi(luw_domain* const* doms, uint32_t count, uint64_t t0, ui
 int luw_vk_inlet_create(luw_domain* d, uint64_t P, uint64_t M, uint64_t V, const uint64_t* pc, const uint8_t* pf, const float* pd, const float* md, luw_vk_inlet** out) {
 	if(!d||!out||(P>0ull&&(!pc||!pf||!pd))||(V>0ull&&!md)) return fail(LUW_ERR_INVALID, "null argument");
 	*out = nullptr;
-	for(uint64_t i=0ull; i<P; i++) if(pc[i]>=d->ncells) return fail(LUW_ERR_INVALID, "inlet point outside the domain");
-	std::vector<uint64_t> pcd(pc, pc+P); // device indices of the cells
-	for(uint64_t i=0ull; i<P; i++) pcd[i] = device_index(d->c, pc[i]);
-	DeviceGuard guard(d->p.device);
-	luw_vk_inlet* v = new(std::nothrow) luw_vk_inlet();
-	if(!v) return fail(LUW_ERR_OOM, "host allocation failed");
-	memset(v, 0, sizeof(*v));
-	v->dom = d; v->P = P; v->M = M; v->V = V;
-	int rc = LUW_OK;
-	if(P>0ull) {
-		rc = dev_alloc(d, &v->point_cell, P);
-		if(rc==LUW_OK) rc = dev_alloc(d, &v->point_face, P);
-		if(rc==LUW_OK) rc = dev_alloc(d, &v->point_data, 7ull*P);
-	}
-	if(rc==LUW_OK&&V>0ull) rc = dev_alloc(d, &v->mode_data, 10ull*V);
-	if(rc==LUW_OK&&V>0ull) rc = dev_alloc(d, &v->mode_cs, 6ull*V);
+	std::vector<uint64_t> pcd;
+	if(const int rc = device_cells(d, pc, P, false, pcd)) return rc;
 	std::vector<float> cs(6ull*V);
 	for(uint64_t k=0ull; k<V; k++) for(uint32_t c=0u; c<3u; c++) { // amplitude (rows 4..6) times cos / sin of the phase (rows 7..9), in double, rounded once
 		const double A = md[(4ull+c)*V+k], ph = md[(7ull+c)*V+k];
 		cs[(2ull*c)*V+k] = (float)(A*cos(ph)); cs[(2ull*c+1ull)*V+k] = (float)(A*sin(ph));
 	}
-	if(rc==LUW_OK) {
-		cudaError_t e = cudaSuccess;
-		if(P>0ull) {
-			e = cudaMemcpyAsync(v->point_cell, pcd.data(), P*8ull, cudaMemcpyHostToDevice, d->stream);
-			if(e==cudaSuccess) e = cudaMemcpyAsync(v->point_face, pf, P, cudaMemcpyHostToDevice, d->stream);
-			if(e==cudaSuccess) e = cudaMemcpyAsync(v->point_data, pd, 7ull*P*4ull, cudaMemcpyHostToDevice, d->stream);
-		}
-		if(e==cudaSuccess&&V>0ull) e = cudaMemcpyAsync(v->mode_data, md, 10ull*V*4ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&V>0ull) e = cudaMemcpyAsync(v->mode_cs, cs.data(), 6ull*V*4ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // host arrays may be freed by the caller afterwards
-		if(e!=cudaSuccess) rc = cuda_fail(e, "upload inlet buffers");
+	DeviceGuard guard(d->p.device);
+	std::unique_ptr<luw_vk_inlet> v(new(std::nothrow) luw_vk_inlet());
+	if(!v) return fail(LUW_ERR_OOM, "host allocation failed");
+	v->dom = d; v->mem.charge = &d->bytes; v->P = P; v->M = M; v->V = V;
+	if(P>0ull) {
+		CU(v->mem.upload(&v->point_cell, pcd.data(), P, d->stream));
+		CU(v->mem.upload(&v->point_face, pf, P, d->stream));
+		CU(v->mem.upload(&v->point_data, pd, 7ull*P, d->stream));
 	}
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_vk_inlet_destroy(v); g_error = keep; return rc; }
-	*out = v;
+	if(V>0ull) {
+		CU(v->mem.upload(&v->mode_data, md, 10ull*V, d->stream));
+		CU(v->mem.upload(&v->mode_cs, cs.data(), 6ull*V, d->stream));
+	}
+	CU(cudaStreamSynchronize(d->stream)); // host arrays may be freed by the caller afterwards
+	*out = v.release();
 	return LUW_OK;
 }
 int luw_vk_inlet_apply(luw_vk_inlet* v, uint32_t use_interp, float t0, float t1, float alpha) {
@@ -914,7 +956,6 @@ int luw_vk_inlet_destroy(luw_vk_inlet* v) {
 	if(!v) return LUW_OK;
 	DeviceGuard guard(v->dom->p.device);
 	cudaStreamSynchronize(v->dom->stream);
-	cudaFree(v->point_cell); cudaFree(v->point_face); cudaFree(v->point_data); cudaFree(v->mode_data); cudaFree(v->mode_cs);
 	delete v;
 	return LUW_OK;
 }
@@ -929,16 +970,14 @@ int luw_voxelize_mesh(luw_domain* d, uint32_t direction, uint8_t flag, const flo
 	luw::VoxBins bins;
 	if(!(env&&env[0]=='0')) bins = luw::vox_build_bins(direction, d->c.Nx, d->c.Ny, d->c.Nz, d->c.Ox, d->c.Oy, d->c.Oz, p0, p1, p2, ntri);
 	const bool binned = bins.bins0>0u;
-	DeviceBuffers mem;
+	DeviceMemory mem;
 	float* tri = nullptr; uint32_t* bin_start = nullptr; uint32_t* bin_ids = nullptr;
-	CU(mem.get(&tri, 9ull*ntri)); // Memory<float3> p0, p1, p2 of FX/lbm.cpp:525-527: live for this call only
-	if(binned) { CU(mem.get(&bin_start, (uint64_t)bins.start.size())); CU(mem.get(&bin_ids, (uint64_t)bins.ids.size())); }
+	CU(mem.alloc(&tri, 9ull*ntri)); // Memory<float3> p0, p1, p2 of FX/lbm.cpp:525-527: live for this call only
+	if(binned) { CU(mem.upload(&bin_start, bins.start.data(), bins.start.size(), d->stream)); CU(mem.upload(&bin_ids, bins.ids.data(), bins.ids.size(), d->stream)); }
 	cudaError_t e = cudaMemcpyAsync(tri, p0, 3ull*ntri*4ull, cudaMemcpyHostToDevice, d->stream);
 	if(e==cudaSuccess) e = cudaMemcpyAsync(tri+3ull*ntri, p1, 3ull*ntri*4ull, cudaMemcpyHostToDevice, d->stream);
 	if(e==cudaSuccess) e = cudaMemcpyAsync(tri+6ull*ntri, p2, 3ull*ntri*4ull, cudaMemcpyHostToDevice, d->stream);
 	if(binned) {
-		if(e==cudaSuccess) e = cudaMemcpyAsync(bin_start, bins.start.data(), bins.start.size()*4ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&!bins.ids.empty()) e = cudaMemcpyAsync(bin_ids, bins.ids.data(), bins.ids.size()*4ull, cudaMemcpyHostToDevice, d->stream);
 		if(e==cudaSuccess) e = luw::kernels_strict().voxelize_binned(d->c, direction, flag, ntri, bbu+1, bins.bins0, bins.bins1, bin_start, bin_ids, tri, tri+3ull*ntri, tri+6ull*ntri, d->stream);
 	} else if(e==cudaSuccess) e = luw::kernels_strict().voxelize(d->c, direction, flag, ntri, bbu+1, tri, tri+3ull*ntri, tri+6ull*ntri, d->stream); // always the as-written arithmetic: flags are bit-exact
 	if(e==cudaSuccess) { d->launches++; e = cudaStreamSynchronize(d->stream); } // kernel.run() is synchronous in the reference, and the buffers are released on return
@@ -951,10 +990,10 @@ int luw_inlet_nearest(int device, uint64_t ncells, const float* cell_xyz, uint32
 	if(ncells==0ull) return LUW_OK;
 	DeviceGuard guard(device);
 	if(guard.err!=cudaSuccess) return cuda_fail(guard.err, "cudaSetDevice");
-	DeviceBuffers mem;
+	DeviceMemory mem;
 	const uint64_t B = ncells<kInletBatch ? ncells : kInletBatch;
 	float* dp = nullptr; float* dc = nullptr; uint32_t* dn = nullptr;
-	CU(mem.get(&dp, 3ull*npts)); CU(mem.get(&dc, 3ull*B)); CU(mem.get(&dn, B));
+	CU(mem.alloc(&dp, 3ull*npts)); CU(mem.alloc(&dc, 3ull*B)); CU(mem.alloc(&dn, B));
 	CU(cudaMemcpy(dp, point_xyz, 3ull*npts*sizeof(float), cudaMemcpyHostToDevice));
 	for(uint64_t c0=0ull; c0<ncells; c0+=B) {
 		const uint64_t n = ncells-c0<B ? ncells-c0 : B;
@@ -972,10 +1011,10 @@ int luw_inlet_knn(int device, uint64_t ncells, const float* cell_ab, uint32_t np
 	if(ncells==0ull) return LUW_OK;
 	DeviceGuard guard(device);
 	if(guard.err!=cudaSuccess) return cuda_fail(guard.err, "cudaSetDevice");
-	DeviceBuffers mem;
+	DeviceMemory mem;
 	const uint64_t B = ncells<kInletBatch ? ncells : kInletBatch, K = (uint64_t)luw::INLET_KNN_K;
 	float2* dp = nullptr; float* dc = nullptr; uint32_t* dk = nullptr; uint32_t* du = nullptr; float* dm = nullptr; int32_t* de = nullptr;
-	CU(mem.get(&dp, (uint64_t)npts)); CU(mem.get(&dc, 2ull*B)); CU(mem.get(&dk, K*B)); CU(mem.get(&du, B)); CU(mem.get(&dm, B)); CU(mem.get(&de, B));
+	CU(mem.alloc(&dp, (uint64_t)npts)); CU(mem.alloc(&dc, 2ull*B)); CU(mem.alloc(&dk, K*B)); CU(mem.alloc(&du, B)); CU(mem.alloc(&dm, B)); CU(mem.alloc(&de, B));
 	CU(cudaMemcpy(dp, point_ab, 2ull*npts*sizeof(float), cudaMemcpyHostToDevice));
 	for(uint64_t c0=0ull; c0<ncells; c0+=B) {
 		const uint64_t n = ncells-c0<B ? ncells-c0 : B;
@@ -1000,33 +1039,23 @@ int luw_inlet_launch_count(uint64_t* launches) {
 int luw_cellset_create(luw_domain* d, uint64_t count, const uint64_t* host_cell_index, luw_cellset** out) {
 	if(!d||!out||(count>0ull&&!host_cell_index)) return fail(LUW_ERR_INVALID, "null argument");
 	*out = nullptr;
-	for(uint64_t k=0ull; k<count; k++) if(host_cell_index[k]>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
-	std::vector<uint64_t> cd(host_cell_index, host_cell_index+count); // device indices
-	for(uint64_t k=0ull; k<count; k++) cd[k] = device_index(d->c, host_cell_index[k]);
+	std::vector<uint64_t> cd;
+	if(const int rc = device_cells(d, host_cell_index, count, false, cd)) return rc;
 	DeviceGuard guard(d->p.device);
-	luw_cellset* s = new(std::nothrow) luw_cellset();
+	std::unique_ptr<luw_cellset> s(new(std::nothrow) luw_cellset());
 	if(!s) return fail(LUW_ERR_OOM, "host allocation failed");
-	memset(s, 0, sizeof(*s));
-	s->dom = d; s->count = count;
-	int rc = LUW_OK;
+	s->dom = d; s->mem.charge = &d->bytes; s->count = count;
 	if(count>0ull) {
-		rc = dev_alloc(d, &s->cell, count);
-		for(int k=0; k<2&&rc==LUW_OK; k++) { rc = dev_alloc(d, &s->up[k], 3ull*count); if(rc==LUW_OK) rc = dev_alloc(d, &s->dn[k], 3ull*count); }
-		for(int k=0; k<2&&rc==LUW_OK; k++) {
-			cudaError_t e = cudaEventCreateWithFlags(&s->staged[k], cudaEventDisableTiming);
-			if(e==cudaSuccess) e = cudaEventCreateWithFlags(&s->scattered[k], cudaEventDisableTiming);
-			if(e==cudaSuccess) e = cudaEventCreateWithFlags(&s->gathered[k], cudaEventDisableTiming);
-			if(e==cudaSuccess) e = cudaEventCreateWithFlags(&s->drained[k], cudaEventDisableTiming);
-			if(e!=cudaSuccess) rc = cuda_fail(e, "cudaEventCreate");
+		DeviceMemory& m = s->mem;
+		CU(m.upload(&s->cell, cd.data(), count, d->stream));
+		for(int k=0; k<2; k++) {
+			CU(m.alloc(&s->up[k], 3ull*count));
+			CU(m.alloc(&s->dn[k], 3ull*count));
+			CU(m.event(&s->staged[k])); CU(m.event(&s->scattered[k])); CU(m.event(&s->gathered[k])); CU(m.event(&s->drained[k]));
 		}
-		if(rc==LUW_OK) {
-			cudaError_t e = cudaMemcpyAsync(s->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
-			if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream);
-			if(e!=cudaSuccess) rc = cuda_fail(e, "upload cell set");
-		}
+		CU(cudaStreamSynchronize(d->stream));
 	}
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_cellset_destroy(s); g_error = keep; return rc; }
-	*out = s;
+	*out = s.release();
 	return LUW_OK;
 }
 static int cellset_move(luw_cellset* s, int field, void* host, const bool up) {
@@ -1069,14 +1098,6 @@ int luw_cellset_destroy(luw_cellset* s) {
 	if(!s) return LUW_OK;
 	DeviceGuard guard(s->dom->p.device);
 	cudaStreamSynchronize(s->dom->stream); cudaStreamSynchronize(s->dom->copy_stream);
-	cudaFree(s->cell);
-	for(int k=0; k<2; k++) {
-		cudaFree(s->up[k]); cudaFree(s->dn[k]);
-		if(s->staged[k]) cudaEventDestroy(s->staged[k]);
-		if(s->scattered[k]) cudaEventDestroy(s->scattered[k]);
-		if(s->gathered[k]) cudaEventDestroy(s->gathered[k]);
-		if(s->drained[k]) cudaEventDestroy(s->drained[k]);
-	}
 	delete s;
 	return LUW_OK;
 }
@@ -1085,16 +1106,15 @@ int luw_stats_create(luw_domain* d, luw_stats** out) {
 	if(!d||!out) return fail(LUW_ERR_INVALID, "null argument");
 	*out = nullptr;
 	DeviceGuard guard(d->p.device);
-	luw_stats* st = new(std::nothrow) luw_stats();
+	std::unique_ptr<luw_stats> st(new(std::nothrow) luw_stats());
 	if(!st) return fail(LUW_ERR_OOM, "host allocation failed");
-	st->dom = d; st->count = 0ull; st->mean_u = st->m2_u = st->mean_rho = st->mean_T = nullptr;
-	int rc = dev_alloc(d, &st->mean_u, 3ull*d->c.N);
-	if(rc==LUW_OK) rc = dev_alloc(d, &st->m2_u, 3ull*d->c.N);
-	if(rc==LUW_OK) rc = dev_alloc(d, &st->mean_rho, d->c.N);
-	if(rc==LUW_OK&&d->c.T) rc = dev_alloc(d, &st->mean_T, d->c.N);
-	if(rc==LUW_OK) rc = luw_stats_reset(st);
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_stats_destroy(st); g_error = keep; return rc; }
-	*out = st;
+	st->dom = d; st->mem.charge = &d->bytes;
+	CU(st->mem.alloc(&st->mean_u, 3ull*d->c.N));
+	CU(st->mem.alloc(&st->m2_u, 3ull*d->c.N));
+	CU(st->mem.alloc(&st->mean_rho, d->c.N));
+	if(d->c.T) CU(st->mem.alloc(&st->mean_T, d->c.N));
+	if(const int rc = luw_stats_reset(st.get())) return rc;
+	*out = st.release();
 	return LUW_OK;
 }
 int luw_stats_reset(luw_stats* st) {
@@ -1114,11 +1134,11 @@ int luw_stats_accumulate(luw_stats* st) {
 	DeviceGuard guard(d->p.device);
 	st->count++;
 	const float inv_n = 1.0f/(float)st->count;
-	k_stats_accumulate<<<(unsigned)(4*d->sm_count>0 ? 8*d->sm_count : 1184), 256, 0, d->stream>>>(d->c.N, inv_n, d->c.rho, d->c.u, st->mean_u, st->m2_u, st->mean_rho);
+	k_stats_accumulate<<<lattice_grid(d), 256, 0, d->stream>>>(d->c.N, inv_n, d->c.rho, d->c.u, st->mean_u, st->m2_u, st->mean_rho);
 	CU(cudaGetLastError());
 	d->launches++;
 	if(st->mean_T) {
-		k_stats_mean<<<(unsigned)(4*d->sm_count>0 ? 8*d->sm_count : 1184), 256, 0, d->stream>>>(d->c.N, inv_n, d->c.T, st->mean_T);
+		k_stats_mean<<<lattice_grid(d), 256, 0, d->stream>>>(d->c.N, inv_n, d->c.T, st->mean_T);
 		CU(cudaGetLastError());
 		d->launches++;
 	}
@@ -1148,7 +1168,6 @@ int luw_stats_destroy(luw_stats* st) {
 	if(!st) return LUW_OK;
 	DeviceGuard guard(st->dom->p.device);
 	cudaStreamSynchronize(st->dom->stream);
-	cudaFree(st->mean_u); cudaFree(st->m2_u); cudaFree(st->mean_rho); cudaFree(st->mean_T);
 	delete st;
 	return LUW_OK;
 }
@@ -1163,12 +1182,12 @@ int luw_column_ground(luw_domain* d, uint32_t* host_ground) {
 	if(const int rc = require_device()) return rc;
 	if(!d||!host_ground) return fail(LUW_ERR_INVALID, "null argument");
 	const luw::DomainConst& c = d->c;
-	const uint32_t Hz = c.Dz>1u ? 1u : 0u;
+	const Box b = owned_box(c);
 	DeviceGuard guard(d->p.device);
-	DeviceBuffers mem;
+	DeviceMemory mem;
 	uint32_t* g = nullptr;
-	CU(mem.get(&g, (uint64_t)c.Nx*c.Ny));
-	luw::k_column_ground<<<dim3((c.Nx+255u)/256u, c.Ny), 256, 0, d->stream>>>(c.Nx, c.Px, c.Ny, Hz, c.Nz-Hz, c.Oz, c.flags, g);
+	CU(mem.alloc(&g, (uint64_t)c.Nx*c.Ny));
+	luw::k_column_ground<<<dim3((c.Nx+255u)/256u, c.Ny), 256, 0, d->stream>>>(c.Nx, c.Px, c.Ny, b.z0, b.z1, c.Oz, c.flags, g);
 	CU(cudaGetLastError());
 	d->launches++;
 	CU(cudaMemcpyAsync(host_ground, g, (uint64_t)c.Nx*c.Ny*4ull, cudaMemcpyDeviceToHost, d->stream));
@@ -1187,28 +1206,20 @@ int luw_wind_stats_create(luw_domain* d, uint64_t count, const uint64_t* host_ce
 		if(!(host_thresholds[j]>=0.0f)) return fail(LUW_ERR_INVALID, "thresholds must be non-negative numbers");
 		thr.t[j] = host_thresholds[j];
 	}
-	for(uint64_t k=0ull; k<count; k++) if(host_cell_index[k]>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
-	std::vector<uint64_t> cd(count);
-	for(uint64_t k=0ull; k<count; k++) cd[k] = device_index(d->c, host_cell_index[k]);
+	std::vector<uint64_t> cd;
+	if(const int rc = device_cells(d, host_cell_index, count, false, cd)) return rc;
 	DeviceGuard guard(d->p.device);
-	luw_wind_stats* st = new(std::nothrow) luw_wind_stats();
+	std::unique_ptr<luw_wind_stats> st(new(std::nothrow) luw_wind_stats());
 	if(!st) return fail(LUW_ERR_OOM, "host allocation failed");
-	memset(st, 0, sizeof(*st));
-	st->dom = d; st->count = count; st->thr = thr;
-	int rc = LUW_OK;
+	st->dom = d; st->mem.charge = &d->bytes; st->count = count; st->thr = thr;
 	if(count>0ull) {
-		rc = dev_alloc(d, &st->cell, count);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->acc, (uint64_t)luw::WIND_FLOAT_ACCUMULATORS*count);
-		if(rc==LUW_OK&&threshold_count>0u) rc = dev_alloc(d, &st->exceed, (uint64_t)threshold_count*count);
-		if(rc==LUW_OK) {
-			cudaError_t e = cudaMemcpyAsync(st->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
-			if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // the host list may be freed by the caller afterwards
-			if(e!=cudaSuccess) rc = cuda_fail(e, "upload cell list");
-		}
+		CU(st->mem.upload(&st->cell, cd.data(), count, d->stream));
+		CU(st->mem.alloc(&st->acc, (uint64_t)luw::WIND_FLOAT_ACCUMULATORS*count));
+		if(threshold_count>0u) CU(st->mem.alloc(&st->exceed, (uint64_t)threshold_count*count));
+		CU(cudaStreamSynchronize(d->stream)); // cd is freed on return
 	}
-	if(rc==LUW_OK) rc = luw_wind_stats_reset(st);
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_wind_stats_destroy(st); g_error = keep; return rc; }
-	*out = st;
+	if(const int rc = luw_wind_stats_reset(st.get())) return rc;
+	*out = st.release();
 	return LUW_OK;
 }
 int luw_wind_stats_reset(luw_wind_stats* st) {
@@ -1229,8 +1240,7 @@ int luw_wind_stats_accumulate(luw_wind_stats* st) {
 	st->samples++;
 	const float inv_n = 1.0f/(float)st->samples;
 	if(st->count==0ull) return LUW_OK;
-	const uint64_t want = (st->count+255ull)/256ull, cap = d->sm_count>0 ? 8ull*(uint64_t)d->sm_count : 1184ull;
-	luw::k_wind_stats_accumulate<<<(unsigned)(want<cap ? want : cap), 256, 0, d->stream>>>(st->count, d->c.N, inv_n, d->c.u, st->cell, st->thr, st->acc, st->exceed);
+	luw::k_wind_stats_accumulate<<<list_grid(d, st->count), 256, 0, d->stream>>>(st->count, d->c.N, inv_n, d->c.u, st->cell, st->thr, st->acc, st->exceed);
 	CU(cudaGetLastError());
 	d->launches++;
 	return LUW_OK;
@@ -1258,29 +1268,21 @@ int luw_wind_stats_destroy(luw_wind_stats* st) {
 	if(!st) return LUW_OK;
 	DeviceGuard guard(st->dom->p.device);
 	cudaStreamSynchronize(st->dom->stream);
-	cudaFree(st->cell); cudaFree(st->acc); cudaFree(st->exceed);
 	delete st;
 	return LUW_OK;
 }
 
-// owned range of a local axis: the halo layer at each end of a decomposed axis belongs to the neighbours
-static void owned_range(const uint32_t n, const uint32_t D, uint32_t& lo, uint32_t& hi) { lo = D>1u ? 1u : 0u; hi = n-lo; }
-static unsigned list_grid(const luw_domain* d, const uint64_t items) {
-	const uint64_t want = (items+255ull)/256ull, cap = d->sm_count>0 ? 8ull*(uint64_t)d->sm_count : 1184ull;
-	return (unsigned)(want<1ull ? 1ull : want<cap ? want : cap);
-}
 int luw_solid_surface(luw_domain* d, uint32_t periodic_mask, uint64_t capacity, uint64_t* host_cells, uint64_t* count) {
 	if(const int rc = require_device()) return rc;
 	if(!d||!count) return fail(LUW_ERR_INVALID, "null argument");
 	const luw::DomainConst& c = d->c;
-	uint32_t x0, x1, y0, y1, z0, z1;
-	owned_range(c.Nx, c.Dx, x0, x1); owned_range(c.Ny, c.Dy, y0, y1); owned_range(c.Nz, c.Dz, z0, z1);
-	const uint64_t rows = (uint64_t)(y1-y0)*(z1-z0);
+	const Box b = owned_box(c);
+	const uint64_t rows = (uint64_t)(b.y1-b.y0)*(b.z1-b.z0);
 	DeviceGuard guard(d->p.device);
-	DeviceBuffers mem;
+	DeviceMemory mem;
 	uint32_t* rc_dev = nullptr;
-	CU(mem.get(&rc_dev, rows));
-	luw::k_surface_rows<<<list_grid(d, rows), 256, 0, d->stream>>>(c, periodic_mask&7u, x0, x1, y0, y1, z0, z1, nullptr, rc_dev, nullptr);
+	CU(mem.alloc(&rc_dev, rows));
+	luw::k_surface_rows<<<list_grid(d, rows), 256, 0, d->stream>>>(c, periodic_mask&7u, b.x0, b.x1, b.y0, b.y1, b.z0, b.z1, nullptr, rc_dev, nullptr);
 	CU(cudaGetLastError());
 	d->launches++;
 	std::vector<uint32_t> rc(rows);
@@ -1294,10 +1296,9 @@ int luw_solid_surface(luw_domain* d, uint32_t periodic_mask, uint64_t capacity, 
 	if(capacity<total) return fail(LUW_ERR_INVALID, "capacity below the number of surface cells (call with host_cells == NULL for the count)");
 	if(total==0ull) return LUW_OK;
 	uint64_t* off_dev = nullptr; uint64_t* cells_dev = nullptr;
-	CU(mem.get(&off_dev, rows));
-	CU(mem.get(&cells_dev, total));
-	CU(cudaMemcpyAsync(off_dev, offset.data(), rows*8ull, cudaMemcpyHostToDevice, d->stream));
-	luw::k_surface_rows<<<list_grid(d, rows), 256, 0, d->stream>>>(c, periodic_mask&7u, x0, x1, y0, y1, z0, z1, off_dev, nullptr, cells_dev);
+	CU(mem.upload(&off_dev, offset.data(), rows, d->stream));
+	CU(mem.alloc(&cells_dev, total));
+	luw::k_surface_rows<<<list_grid(d, rows), 256, 0, d->stream>>>(c, periodic_mask&7u, b.x0, b.x1, b.y0, b.y1, b.z0, b.z1, off_dev, nullptr, cells_dev);
 	CU(cudaGetLastError());
 	d->launches++;
 	CU(cudaMemcpyAsync(host_cells, cells_dev, total*8ull, cudaMemcpyDeviceToHost, d->stream));
@@ -1312,22 +1313,16 @@ int luw_wall_loads_create(luw_domain* d, uint64_t count, const uint64_t* host_ce
 	if(label_count==0u) return fail(LUW_ERR_INVALID, "label_count must be at least 1");
 	if(sample_capacity==0u) return fail(LUW_ERR_INVALID, "sample_capacity must be at least 1");
 	for(uint64_t q=0ull; q<3ull*label_count; q++) if(!std::isfinite(host_ref_points[q])) return fail(LUW_ERR_INVALID, "reference points must be finite");
-	const luw::DomainConst& c = d->c;
-	uint32_t x0, x1, y0, y1, z0, z1;
-	owned_range(c.Nx, c.Dx, x0, x1); owned_range(c.Ny, c.Dy, y0, y1); owned_range(c.Nz, c.Dz, z0, z1);
-	std::vector<uint64_t> cd(count), chunk_begin;
+	std::vector<uint64_t> cd, chunk_begin;
+	if(const int rc = device_cells(d, host_cell_index, count, true, cd)) return rc;
 	std::vector<uint32_t> chunk_label;
 	std::vector<uint64_t> label_group(label_count+1ull, 0ull);
 	for(uint64_t k=0ull; k<count; k++) {
 		const uint64_t n = host_cell_index[k];
 		const uint32_t l = host_label[k];
-		if(n>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
-		const uint32_t x = (uint32_t)(n%c.Nx), y = (uint32_t)((n/c.Nx)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Nx*c.Ny));
-		if(x<x0||x>=x1||y<y0||y>=y1||z<z0||z>=z1) return fail(LUW_ERR_INVALID, "cell index in a halo layer");
 		if(l>=label_count) return fail(LUW_ERR_INVALID, "label outside [0, label_count)");
 		if(k>0ull&&!(l>host_label[k-1ull]||(l==host_label[k-1ull]&&n>host_cell_index[k-1ull]))) return fail(LUW_ERR_INVALID, "the list must be sorted by (label, cell index), strictly increasing");
 		if(k==0ull||l!=host_label[k-1ull]||k-chunk_begin.back()==(uint64_t)luw::WALL_CHUNK) { chunk_begin.push_back(k); chunk_label.push_back(l); }
-		cd[k] = device_index(c, n);
 	}
 	const uint64_t nchunks = chunk_label.size();
 	chunk_begin.push_back(count);
@@ -1342,42 +1337,32 @@ int luw_wall_loads_create(luw_domain* d, uint64_t count, const uint64_t* host_ce
 	group_begin.push_back(nchunks);
 	for(uint32_t l=1u; l<=label_count; l++) if(label_group[l]<label_group[l-1u]) label_group[l] = label_group[l-1u]; // labels without cells: empty ranges
 	DeviceGuard guard(d->p.device);
-	luw_wall_loads* st = new(std::nothrow) luw_wall_loads();
+	std::unique_ptr<luw_wall_loads> st(new(std::nothrow) luw_wall_loads());
 	if(!st) return fail(LUW_ERR_OOM, "host allocation failed");
-	memset(st, 0, sizeof(*st));
-	st->dom = d; st->count = count; st->nchunks = nchunks; st->ngroups = ngroups; st->L = label_count; st->capacity = sample_capacity; st->periodic = periodic_mask&7u;
-	int rc = dev_alloc(d, &st->ref, 3ull*label_count);
-	if(rc==LUW_OK) rc = dev_alloc(d, &st->label_group, label_count+1ull);
-	if(rc==LUW_OK) rc = dev_alloc(d, &st->ring, (uint64_t)sample_capacity*label_count*luw::WALL_COMPONENTS);
-	if(rc==LUW_OK&&count>0ull) {
-		rc = dev_alloc(d, &st->cell, count);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->links, count);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->F, 3ull*count);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->acc, 6ull*count);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->chunk_begin, nchunks+1ull);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->chunk_label, nchunks);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->partial, luw::WALL_COMPONENTS*nchunks);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->group_begin, ngroups+1ull);
-		if(rc==LUW_OK) rc = dev_alloc(d, &st->partial2, luw::WALL_COMPONENTS*ngroups);
+	st->dom = d; st->mem.charge = &d->bytes;
+	st->count = count; st->nchunks = nchunks; st->ngroups = ngroups; st->L = label_count; st->capacity = sample_capacity; st->periodic = periodic_mask&7u;
+	DeviceMemory& m = st->mem;
+	CU(m.upload(&st->ref, host_ref_points, 3ull*label_count, d->stream));
+	CU(m.upload(&st->label_group, label_group.data(), label_count+1ull, d->stream));
+	CU(m.alloc(&st->ring, (uint64_t)sample_capacity*label_count*luw::WALL_COMPONENTS));
+	if(count>0ull) {
+		CU(m.upload(&st->cell, cd.data(), count, d->stream));
+		CU(m.alloc(&st->links, count));
+		CU(m.alloc(&st->F, 3ull*count));
+		CU(m.alloc(&st->acc, 6ull*count));
+		CU(m.upload(&st->chunk_begin, chunk_begin.data(), nchunks+1ull, d->stream));
+		CU(m.upload(&st->chunk_label, chunk_label.data(), nchunks, d->stream));
+		CU(m.alloc(&st->partial, luw::WALL_COMPONENTS*nchunks));
+		CU(m.upload(&st->group_begin, group_begin.data(), ngroups+1ull, d->stream));
+		CU(m.alloc(&st->partial2, luw::WALL_COMPONENTS*ngroups));
+		// the links are classified once, from the device flags as they are now
+		luw::k_wall_links<<<list_grid(d, count), 256, 0, d->stream>>>(d->c, st->periodic, count, st->cell, st->links);
+		d->launches++;
+		CU(cudaGetLastError());
 	}
-	if(rc==LUW_OK) {
-		cudaError_t e = cudaMemcpyAsync(st->ref, host_ref_points, 3ull*label_count*8ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess) e = cudaMemcpyAsync(st->label_group, label_group.data(), (label_count+1ull)*8ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->group_begin, group_begin.data(), (ngroups+1ull)*8ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->chunk_begin, chunk_begin.data(), (nchunks+1ull)*8ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&count>0ull) e = cudaMemcpyAsync(st->chunk_label, chunk_label.data(), nchunks*4ull, cudaMemcpyHostToDevice, d->stream);
-		if(e==cudaSuccess&&count>0ull) { // the links are classified once, from the device flags as they are now
-			luw::k_wall_links<<<list_grid(d, count), 256, 0, d->stream>>>(c, st->periodic, count, st->cell, st->links);
-			e = cudaGetLastError();
-			d->launches++;
-		}
-		if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // the host arrays may be freed by the caller afterwards
-		if(e!=cudaSuccess) rc = cuda_fail(e, "set up the wall-load list");
-	}
-	if(rc==LUW_OK) rc = luw_wall_loads_reset(st);
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_wall_loads_destroy(st); g_error = keep; return rc; }
-	*out = st;
+	CU(cudaStreamSynchronize(d->stream)); // the host arrays may be freed by the caller afterwards
+	if(const int rc = luw_wall_loads_reset(st.get())) return rc;
+	*out = st.release();
 	return LUW_OK;
 }
 int luw_wall_loads_reset(luw_wall_loads* st) {
@@ -1441,8 +1426,6 @@ int luw_wall_loads_destroy(luw_wall_loads* st) {
 	if(!st) return LUW_OK;
 	DeviceGuard guard(st->dom->p.device);
 	cudaStreamSynchronize(st->dom->stream);
-	cudaFree(st->cell); cudaFree(st->links); cudaFree(st->F); cudaFree(st->acc); cudaFree(st->chunk_begin); cudaFree(st->chunk_label);
-	cudaFree(st->group_begin); cudaFree(st->label_group); cudaFree(st->ref); cudaFree(st->partial); cudaFree(st->partial2); cudaFree(st->ring);
 	delete st;
 	return LUW_OK;
 }
@@ -1452,34 +1435,18 @@ int luw_probes_create(luw_domain* d, uint64_t count, const uint64_t* host_cell_i
 	if(!d||!out||(count>0ull&&!host_cell_index)) return fail(LUW_ERR_INVALID, "null argument");
 	*out = nullptr;
 	if(sample_capacity==0u) return fail(LUW_ERR_INVALID, "sample_capacity must be at least 1");
-	const luw::DomainConst& c = d->c;
-	uint32_t x0, x1, y0, y1, z0, z1;
-	owned_range(c.Nx, c.Dx, x0, x1); owned_range(c.Ny, c.Dy, y0, y1); owned_range(c.Nz, c.Dz, z0, z1);
-	std::vector<uint64_t> cd(count);
-	for(uint64_t k=0ull; k<count; k++) {
-		const uint64_t n = host_cell_index[k];
-		if(n>=d->ncells) return fail(LUW_ERR_INVALID, "cell index outside the domain");
-		const uint32_t x = (uint32_t)(n%c.Nx), y = (uint32_t)((n/c.Nx)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Nx*c.Ny));
-		if(x<x0||x>=x1||y<y0||y>=y1||z<z0||z>=z1) return fail(LUW_ERR_INVALID, "cell index in a halo layer");
-		cd[k] = device_index(c, n);
-	}
+	std::vector<uint64_t> cd;
+	if(const int rc = device_cells(d, host_cell_index, count, true, cd)) return rc;
 	DeviceGuard guard(d->p.device);
-	luw_probes* pr = new(std::nothrow) luw_probes();
+	std::unique_ptr<luw_probes> pr(new(std::nothrow) luw_probes());
 	if(!pr) return fail(LUW_ERR_OOM, "host allocation failed");
-	memset(pr, 0, sizeof(*pr));
-	pr->dom = d; pr->count = count; pr->capacity = sample_capacity; pr->comps = (c.features&luw::F_TEMPERATURE) ? 5u : 4u;
-	int rc = LUW_OK;
+	pr->dom = d; pr->mem.charge = &d->bytes; pr->count = count; pr->capacity = sample_capacity; pr->comps = (d->c.features&luw::F_TEMPERATURE) ? 5u : 4u;
 	if(count>0ull) {
-		rc = dev_alloc(d, &pr->cell, count);
-		if(rc==LUW_OK) rc = dev_alloc(d, &pr->ring, (uint64_t)sample_capacity*pr->comps*count);
-		if(rc==LUW_OK) {
-			cudaError_t e = cudaMemcpyAsync(pr->cell, cd.data(), count*8ull, cudaMemcpyHostToDevice, d->stream);
-			if(e==cudaSuccess) e = cudaStreamSynchronize(d->stream); // cd is freed on return
-			if(e!=cudaSuccess) rc = cuda_fail(e, "upload the probe list");
-		}
+		CU(pr->mem.upload(&pr->cell, cd.data(), count, d->stream));
+		CU(pr->mem.alloc(&pr->ring, (uint64_t)sample_capacity*pr->comps*count));
+		CU(cudaStreamSynchronize(d->stream)); // cd is freed on return
 	}
-	if(rc!=LUW_OK) { const std::string keep = g_error; luw_probes_destroy(pr); g_error = keep; return rc; }
-	*out = pr;
+	*out = pr.release();
 	return LUW_OK;
 }
 int luw_probes_sample(luw_probes* pr, uint64_t t, float fx, float fy, float fz, float ox, float oy, float oz) {
@@ -1518,7 +1485,6 @@ int luw_probes_destroy(luw_probes* pr) {
 	if(!pr) return LUW_OK;
 	DeviceGuard guard(pr->dom->p.device);
 	cudaStreamSynchronize(pr->dom->stream);
-	cudaFree(pr->cell); cudaFree(pr->ring);
 	delete pr;
 	return LUW_OK;
 }
