@@ -280,6 +280,34 @@ int luw_probes_drain(luw_probes* pr, float* host_values, uint64_t* samples);
 int luw_probes_reset(luw_probes* pr);
 int luw_probes_destroy(luw_probes* pr);
 
+/* Lagrangian tracer particles. The reference's particle extension (PARTICLES, integrate_particles in FX/kernel.cpp) is compiled out of its urban-wind build; it
+ * moves float32 positions with the trilinearly interpolated stored u and can couple them back to the fluid. Here (csrc/lbm_particles.cuh): float64 positions in
+ * global lattice coordinates (cell centres at integers), u at the 8 cells around a particle as luw_probes_sample reads it (no update_fields over the lattice,
+ * nothing written into it), no back-coupling, plus box emitters, an optional uniform random walk, wall handling, open faces and concentration bins.
+ * Single domains only (Dx = Dy = Dz = 1). All work is stream-ordered on the domain's stream; only the downloads synchronise.
+ * luw_particles_create: a ring of `capacity` >= 1 slots, all FREE (state 0; 1 ACTIVE, 2 DEPOSITED, 3 LEFT, 4 BURIED). host_emitters[6e..6e+5] = centre x y z,
+ *   half-extents x y z (>= 0) of box emitter e < emitter_count, finite, inside [0, N-1] on every non-periodic axis. periodic_mask: bit a set = axis a periodic
+ *   (as in luw_wall_loads_create); a non-periodic axis needs N >= 2. wall_mode 0: a move whose nearest cell floor(p'+0.5) is solid is rejected (the particle
+ *   stays); 1: the particle is DEPOSITED there. seed: the Philox4x64-10 key (seed, 0). bin_size[3] >= 1 cells per concentration bin and axis.
+ * luw_particles_emit: releases emitter_count*per_emitter (<= capacity) particles into the next ring slots, order [emitter][i], overwriting the oldest, each
+ *   at centre + half*(2U-1) per axis (U from the counter (slot, emit call, 1, 0)), with release time t; one placed in a solid cell is BURIED.
+ * luw_particles_advance: the same arguments as luw_update_fields (the state of parity t is read) plus dt and sigma (finite, sigma >= 0): every ACTIVE particle
+ *   moves by u*dt + sigma*sqrt(3)*(2U-1) per axis (U from the counter (slot, advance call, 0, 0)); periodic axes wrap, leaving [0, N-1] on another makes it LEFT.
+ * luw_particles_count: adds every ACTIVE particle to bin floor(p+0.5)/bin_size per axis (integer counts) and counts one sample.
+ * luw_particles_download: synchronous; host_xyz[a*capacity + k], host_state[k], host_emitter[k], host_release_t[k]; NULL skips an array.
+ * luw_particles_download_bins: synchronous; host_bins[(iz*By + iy)*Bx + ix], B = ceil(N/bin_size), and the sample count. luw_particles_reset_bins zeroes both.
+ * Without a CUDA device every entry returns LUW_ERR_NO_DEVICE. */
+typedef struct luw_particles luw_particles;
+int luw_particles_create(luw_domain* dom, uint64_t capacity, uint32_t emitter_count, const double* host_emitters, uint32_t periodic_mask, uint32_t wall_mode,
+	uint64_t seed, const uint32_t* bin_size, luw_particles** out);
+int luw_particles_emit(luw_particles* pt, uint64_t t, uint32_t per_emitter);
+int luw_particles_advance(luw_particles* pt, uint64_t t, float fx, float fy, float fz, float omega_x, float omega_y, float omega_z, float dt, double sigma);
+int luw_particles_count(luw_particles* pt);
+int luw_particles_download(luw_particles* pt, double* host_xyz, uint8_t* host_state, uint32_t* host_emitter, uint64_t* host_release_t);
+int luw_particles_download_bins(luw_particles* pt, uint32_t* host_bins, uint64_t* samples);
+int luw_particles_reset_bins(luw_particles* pt);
+int luw_particles_destroy(luw_particles* pt);
+
 /* page-locked host memory for the mirrors (the reference's Memory<T> owns pageable new[] buffers, FX/opencl.hpp:354) */
 int luw_host_alloc(void** host_ptr, uint64_t bytes);
 int luw_host_free(void* host_ptr);

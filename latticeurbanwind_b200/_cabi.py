@@ -98,6 +98,14 @@ EXPORTS = {  # name -> argtypes; every symbol include/luw_cuda.h declares
     "luw_probes_drain": [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
     "luw_probes_reset": [C.c_void_p],
     "luw_probes_destroy": [C.c_void_p],
+    "luw_particles_create": [C.c_void_p, C.c_uint64, C.c_uint32, C.c_void_p, C.c_uint32, C.c_uint32, C.c_uint64, C.c_void_p, C.POINTER(C.c_void_p)],
+    "luw_particles_emit": [C.c_void_p, C.c_uint64, C.c_uint32],
+    "luw_particles_advance": [C.c_void_p, C.c_uint64] + [C.c_float] * 7 + [C.c_double],
+    "luw_particles_count": [C.c_void_p],
+    "luw_particles_download": [C.c_void_p] * 5,
+    "luw_particles_download_bins": [C.c_void_p, C.c_void_p, C.POINTER(C.c_uint64)],
+    "luw_particles_reset_bins": [C.c_void_p],
+    "luw_particles_destroy": [C.c_void_p],
     "luw_host_alloc": [C.POINTER(C.c_void_p), C.c_uint64],
     "luw_host_free": [C.c_void_p],
     "luw_sync": [C.c_void_p],

@@ -6,6 +6,7 @@
 #include "lbm_common.cuh"
 
 namespace luw {
+struct ParticleSet; // lbm_particles.cuh
 // Run-time value -> template argument: f is called with the matching value as a std::integral_constant (decltype(arg)::value names the instantiation).
 // precision p; unknown values take FP16C
 template<class F> auto with_precision(const int p, F&& f) {
@@ -50,6 +51,8 @@ struct KernelSet { // one per arithmetic mode; every function enqueues exactly o
 	cudaError_t (*thermal_g)(const DomainConst& c, const StepArgs& a, cudaStream_t s); // the TEMPERATURE block alone, after a tiled momentum step that filled c.upre
 	// probe sample (lbm_probes.cuh): rho, u (and T) of `count` listed cells (device indices), as update_fields + a read would give them, into out[c*count + k]
 	cudaError_t (*probe_sample)(const DomainConst& c, const StepArgs& a, uint64_t count, const uint64_t* cell, float* out, unsigned grid, cudaStream_t s);
+	// tracer particles (lbm_particles.cuh): one advance of the ACTIVE particles of `s` by dt with the cell velocities probe_sample reads; call: the ring's advance count
+	cudaError_t (*particles_advance)(const DomainConst& c, const StepArgs& a, const ParticleSet& s, uint64_t call, float dt, double sigma, unsigned grid, cudaStream_t st);
 };
 const KernelSet& kernels_strict(); // lbm_strict.cu: -fmad=false
 const KernelSet& kernels_fast(); // lbm_fast.cu: contraction allowed

@@ -14,24 +14,31 @@
 namespace luw {
 namespace {
 
-// FEAT: F_UPDATE_FIELDS alone, or a subset of F_VOLUME_FORCE | F_EQUILIBRIUM (the bits update_fields depends on). cell[k]: device (pitched) indices of owned cells.
+// rho, u (and, TH, T) at the cell with device index n, as update_fields + a read gives them. FEAT: F_UPDATE_FIELDS alone, or a subset of
+// F_VOLUME_FORCE | F_EQUILIBRIUM (the bits update_fields depends on). k_probe_sample and k_particles_advance (lbm_particles.cuh) read cells through this.
+template<int P, uint32_t FEAT, bool TH> __device__ __forceinline__ void probe_cell(const DomainConst& c, const StepArgs& a, const uint64_t n,
+	float& rhon, float& uxn, float& uyn, float& uzn, float& Tn) {
+	constexpr bool UF = (FEAT&F_UPDATE_FIELDS)!=0u, EQ = (FEAT&F_EQUILIBRIUM)!=0u;
+	const uint32_t fl = c.flags[n], bo = fl&TYPE_BO;
+	const bool computed = !UF&&bo!=TYPE_S&&(fl&TYPE_SU)!=TYPE_G;
+	if(computed) {
+		const uint32_t x = (uint32_t)(n%c.Px), y = (uint32_t)((n/c.Px)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Px*c.Ny));
+		uint64_t j[Q];
+		neighbors(c, x, y, z, j);
+		update_fields_cell<P, FEAT, TH>(c, a, j, x, y, z, fl, rhon, uxn, uyn, uzn, Tn);
+	}
+	if(!computed||(EQ&&bo==TYPE_E)) { rhon = c.rho[n]; uxn = c.u[n]; uyn = c.u[c.N+n]; uzn = c.u[2ull*c.N+n]; }
+	if constexpr(TH) { if(!computed) Tn = c.T[n]; } // update_fields_thermal stores T of every executing cell (a TYPE_T cell's T is its preset)
+}
+
+// cell[k]: device (pitched) indices of owned cells.
 template<int P, uint32_t FEAT, bool TH> __global__ void __launch_bounds__(256) k_probe_sample(const __grid_constant__ DomainConst c, const __grid_constant__ StepArgs a,
 	const uint64_t count, const uint64_t* __restrict__ cell, float* __restrict__ out) {
-	constexpr bool UF = (FEAT&F_UPDATE_FIELDS)!=0u, EQ = (FEAT&F_EQUILIBRIUM)!=0u;
 	for(uint64_t k=(uint64_t)blockIdx.x*blockDim.x+threadIdx.x; k<count; k+=(uint64_t)gridDim.x*blockDim.x) {
-		const uint64_t n = cell[k];
-		const uint32_t fl = c.flags[n], bo = fl&TYPE_BO;
-		const bool computed = !UF&&bo!=TYPE_S&&(fl&TYPE_SU)!=TYPE_G;
 		float rhon, uxn, uyn, uzn, Tn;
-		if(computed) {
-			const uint32_t x = (uint32_t)(n%c.Px), y = (uint32_t)((n/c.Px)%c.Ny), z = (uint32_t)(n/((uint64_t)c.Px*c.Ny));
-			uint64_t j[Q];
-			neighbors(c, x, y, z, j);
-			update_fields_cell<P, FEAT, TH>(c, a, j, x, y, z, fl, rhon, uxn, uyn, uzn, Tn);
-		}
-		if(!computed||(EQ&&bo==TYPE_E)) { rhon = c.rho[n]; uxn = c.u[n]; uyn = c.u[c.N+n]; uzn = c.u[2ull*c.N+n]; }
+		probe_cell<P, FEAT, TH>(c, a, cell[k], rhon, uxn, uyn, uzn, Tn);
 		out[k] = rhon; out[count+k] = uxn; out[2ull*count+k] = uyn; out[3ull*count+k] = uzn;
-		if constexpr(TH) out[4ull*count+k] = computed ? Tn : c.T[n]; // update_fields_thermal stores T of every executing cell (a TYPE_T cell's T is its preset)
+		if constexpr(TH) out[4ull*count+k] = Tn;
 	}
 }
 

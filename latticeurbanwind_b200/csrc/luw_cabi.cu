@@ -5,6 +5,7 @@
 #include "lbm_inlet.cuh"
 #include "lbm_wind_stats.cuh"
 #include "lbm_wall_loads.cuh"
+#include "lbm_particles.cuh"
 #include "vox_bins.h"
 
 #include <climits>
@@ -170,6 +171,16 @@ struct luw_probes {
 	uint32_t comps; // 4: rho ux uy uz; 5: and T
 	uint64_t* cell; // device indices of the listed cells
 	float* ring; // [capacity][comps][count]: samples not drained yet
+};
+struct luw_particles {
+	luw_domain* dom;
+	DeviceMemory mem;
+	luw::ParticleSet s; // device arrays, capacity, seed, periodic mask, wall mode
+	uint32_t E;
+	double* emitters; // device [6E]
+	uint32_t b[3], B[3]; // bin size and bins per axis
+	uint32_t* bins; // [B2][B1][B0]
+	uint64_t head, emit_calls, advance_calls, samples; // next ring slot, Philox call counters, count() calls since the last reset_bins
 };
 struct luw_vk_inlet {
 	luw_domain* dom;
@@ -1486,6 +1497,130 @@ int luw_probes_destroy(luw_probes* pr) {
 	DeviceGuard guard(pr->dom->p.device);
 	cudaStreamSynchronize(pr->dom->stream);
 	delete pr;
+	return LUW_OK;
+}
+
+int luw_particles_create(luw_domain* d, uint64_t capacity, uint32_t emitter_count, const double* host_emitters, uint32_t periodic_mask, uint32_t wall_mode,
+	uint64_t seed, const uint32_t* bin_size, luw_particles** out) {
+	if(const int rc = require_device()) return rc;
+	if(!d||!out||!bin_size||(emitter_count>0u&&!host_emitters)) return fail(LUW_ERR_INVALID, "null argument");
+	*out = nullptr;
+	const luw::DomainConst& c = d->c;
+	if(c.Dx>1u||c.Dy>1u||c.Dz>1u) return fail(LUW_ERR_INVALID, "particles need a single domain (D = 1, 1, 1)");
+	if(capacity==0ull) return fail(LUW_ERR_INVALID, "capacity must be at least 1");
+	if(wall_mode>1u) return fail(LUW_ERR_INVALID, "wall_mode must be 0 or 1");
+	const uint32_t Nd[3] = { c.Nx, c.Ny, c.Nz }, per = periodic_mask&7u;
+	for(int a=0; a<3; a++) {
+		if(bin_size[a]==0u) return fail(LUW_ERR_INVALID, "bin sizes must be at least 1");
+		if(!((per>>a)&1u)&&Nd[a]<2u) return fail(LUW_ERR_INVALID, "a non-periodic axis needs at least 2 cells");
+	}
+	for(uint32_t e=0u; e<emitter_count; e++) for(int a=0; a<3; a++) {
+		const double ce = host_emitters[6u*e+a], h = host_emitters[6u*e+3u+a];
+		if(!std::isfinite(ce)||!std::isfinite(h)||h<0.0) return fail(LUW_ERR_INVALID, "emitter centres and half-extents must be finite, half-extents >= 0");
+		if(!((per>>a)&1u)&&(ce-h<0.0||ce+h>(double)(Nd[a]-1u))) return fail(LUW_ERR_INVALID, "emitter box outside [0, N-1] on a non-periodic axis");
+	}
+	DeviceGuard guard(d->p.device);
+	std::unique_ptr<luw_particles> pt(new(std::nothrow) luw_particles());
+	if(!pt) return fail(LUW_ERR_OOM, "host allocation failed");
+	pt->dom = d; pt->mem.charge = &d->bytes; pt->E = emitter_count;
+	luw::ParticleSet& s = pt->s;
+	s.capacity = capacity; s.seed = seed; s.periodic = per; s.wall_mode = wall_mode;
+	uint64_t nbins = 1ull;
+	for(int a=0; a<3; a++) { pt->b[a] = bin_size[a]; pt->B[a] = (Nd[a]+bin_size[a]-1u)/bin_size[a]; nbins *= pt->B[a]; }
+	DeviceMemory& m = pt->mem;
+	CU(m.alloc(&s.p, 3ull*capacity));
+	CU(m.alloc(&s.state, capacity));
+	CU(m.alloc(&s.emitter, capacity));
+	CU(m.alloc(&s.release, capacity));
+	CU(m.upload(&pt->emitters, host_emitters, 6ull*emitter_count, d->stream));
+	CU(m.alloc(&pt->bins, nbins));
+	CU(cudaMemsetAsync(s.p, 0, 3ull*capacity*8ull, d->stream));
+	CU(cudaMemsetAsync(s.state, luw::PT_FREE, capacity, d->stream));
+	CU(cudaMemsetAsync(s.emitter, 0, capacity*4ull, d->stream));
+	CU(cudaMemsetAsync(s.release, 0, capacity*8ull, d->stream));
+	CU(cudaMemsetAsync(pt->bins, 0, nbins*4ull, d->stream));
+	CU(cudaStreamSynchronize(d->stream)); // the caller may free host_emitters on return
+	*out = pt.release();
+	return LUW_OK;
+}
+int luw_particles_emit(luw_particles* pt, uint64_t t, uint32_t per_emitter) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return fail(LUW_ERR_INVALID, "null particles object");
+	const uint64_t total = (uint64_t)pt->E*per_emitter;
+	if(total>pt->s.capacity) return fail(LUW_ERR_INVALID, "emitter_count * per_emitter exceeds the capacity");
+	if(total>0ull) {
+		luw_domain* d = pt->dom;
+		DeviceGuard guard(d->p.device);
+		luw::k_particles_emit<<<list_grid(d, total), 256, 0, d->stream>>>(d->c, pt->s, pt->emitters, per_emitter, total, pt->head, pt->emit_calls, t);
+		CU(cudaGetLastError());
+		d->launches++;
+		pt->head = (pt->head+total)%pt->s.capacity;
+	}
+	pt->emit_calls++;
+	return LUW_OK;
+}
+int luw_particles_advance(luw_particles* pt, uint64_t t, float fx, float fy, float fz, float ox, float oy, float oz, float dt, double sigma) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return fail(LUW_ERR_INVALID, "null particles object");
+	if(!std::isfinite(dt)) return fail(LUW_ERR_INVALID, "dt must be finite");
+	if(!std::isfinite(sigma)||sigma<0.0) return fail(LUW_ERR_INVALID, "sigma must be finite and >= 0");
+	luw_domain* d = pt->dom;
+	DeviceGuard guard(d->p.device);
+	const luw::StepArgs a = { t, fx, fy, fz, ox, oy, oz };
+	CU(d->ks->particles_advance(d->c, a, pt->s, pt->advance_calls, dt, sigma, list_grid(d, pt->s.capacity), d->stream));
+	d->launches++;
+	pt->advance_calls++;
+	return LUW_OK;
+}
+int luw_particles_count(luw_particles* pt) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return fail(LUW_ERR_INVALID, "null particles object");
+	luw_domain* d = pt->dom;
+	DeviceGuard guard(d->p.device);
+	luw::k_particles_count<<<list_grid(d, pt->s.capacity), 256, 0, d->stream>>>(d->c, pt->s, pt->b[0], pt->b[1], pt->b[2], pt->B[0], pt->B[1], pt->bins);
+	CU(cudaGetLastError());
+	d->launches++;
+	pt->samples++;
+	return LUW_OK;
+}
+int luw_particles_download(luw_particles* pt, double* host_xyz, uint8_t* host_state, uint32_t* host_emitter, uint64_t* host_release_t) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return fail(LUW_ERR_INVALID, "null particles object");
+	luw_domain* d = pt->dom;
+	DeviceGuard guard(d->p.device);
+	const uint64_t K = pt->s.capacity;
+	if(host_xyz) CU(cudaMemcpyAsync(host_xyz, pt->s.p, 3ull*K*8ull, cudaMemcpyDeviceToHost, d->stream));
+	if(host_state) CU(cudaMemcpyAsync(host_state, pt->s.state, K, cudaMemcpyDeviceToHost, d->stream));
+	if(host_emitter) CU(cudaMemcpyAsync(host_emitter, pt->s.emitter, K*4ull, cudaMemcpyDeviceToHost, d->stream));
+	if(host_release_t) CU(cudaMemcpyAsync(host_release_t, pt->s.release, K*8ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	return LUW_OK;
+}
+int luw_particles_download_bins(luw_particles* pt, uint32_t* host_bins, uint64_t* samples) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return fail(LUW_ERR_INVALID, "null particles object");
+	luw_domain* d = pt->dom;
+	DeviceGuard guard(d->p.device);
+	if(host_bins) CU(cudaMemcpyAsync(host_bins, pt->bins, (uint64_t)pt->B[0]*pt->B[1]*pt->B[2]*4ull, cudaMemcpyDeviceToHost, d->stream));
+	CU(cudaStreamSynchronize(d->stream));
+	if(samples) *samples = pt->samples;
+	return LUW_OK;
+}
+int luw_particles_reset_bins(luw_particles* pt) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return fail(LUW_ERR_INVALID, "null particles object");
+	luw_domain* d = pt->dom;
+	DeviceGuard guard(d->p.device);
+	CU(cudaMemsetAsync(pt->bins, 0, (uint64_t)pt->B[0]*pt->B[1]*pt->B[2]*4ull, d->stream));
+	pt->samples = 0ull;
+	return LUW_OK;
+}
+int luw_particles_destroy(luw_particles* pt) {
+	if(const int rc = require_device()) return rc;
+	if(!pt) return LUW_OK;
+	DeviceGuard guard(pt->dom->p.device);
+	cudaStreamSynchronize(pt->dom->stream);
+	delete pt;
 	return LUW_OK;
 }
 

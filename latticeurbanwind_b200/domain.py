@@ -449,6 +449,62 @@ class Probes:
             self._h = C.c_void_p()
 
 
+
+class Particles:
+    """Lagrangian tracer particles on a single domain (luw_particles_*): a device ring of `capacity` slots filled by box emitters, advected with the velocity
+    update_fields + a read would give at the 8 cells around each particle, plus an optional uniform random walk, and binned into concentration counts.
+    `emitters` [E, 6]: centre x y z and half-extents x y z in lattice coordinates; `periodic_mask` bits x y z; wall_mode 0 (a move into a solid cell is
+    rejected) or 1 (the particle is deposited); `bins` (bx, by, bz) cells per bin."""
+    STATES = ("FREE", "ACTIVE", "DEPOSITED", "LEFT", "BURIED")
+
+    def __init__(self, domain, emitters, capacity, periodic_mask=0, wall_mode=0, seed=0, bins=(1, 1, 1)):
+        self.domain = domain
+        self.emitters = np.ascontiguousarray(emitters, np.float64).reshape(-1, 6)
+        self.capacity = int(capacity)
+        self.bin_size = np.ascontiguousarray(bins, np.uint32).reshape(3)
+        shape = (domain.Nx, domain.Ny, domain.Nz)
+        self.bin_shape = tuple(int((n + b - 1) // b) for n, b in zip(shape, self.bin_size))[::-1] if (self.bin_size > 0).all() else (0, 0, 0)
+        self._h = C.c_void_p()
+        A.check(A.lib().luw_particles_create(domain._h, self.capacity, self.emitters.shape[0], _ptr(self.emitters), int(periodic_mask), int(wall_mode), int(seed),
+                                             _ptr(self.bin_size), C.byref(self._h)))
+
+    def emit(self, per_emitter, t=None):
+        """Release per_emitter particles from every emitter into the next ring slots (overwriting the oldest), with release time t (default: the domain's)."""
+        A.check(A.lib().luw_particles_emit(self._h, self.domain.t if t is None else int(t), int(per_emitter)))
+
+    def advance(self, dt=1.0, sigma=0.0, t=None):
+        """Move every ACTIVE particle by u*dt plus a uniform step of standard deviation sigma per axis, u read from the state of time step t (default: the
+        domain's) with the domain's force and Coriolis, the arguments enqueue_update_fields passes. Stream-ordered, no synchronisation."""
+        d = self.domain
+        A.check(A.lib().luw_particles_advance(self._h, d.t if t is None else int(t), *map(float, d.f), *map(float, d.omega), float(dt), float(sigma)))
+
+    def count(self):
+        """Add every ACTIVE particle to its concentration bin (one sample)."""
+        A.check(A.lib().luw_particles_count(self._h))
+
+    def state(self):
+        """-> dict: xyz float64 [capacity, 3], state uint8, emitter uint32, release_t uint64 [capacity]; synchronous."""
+        xyz = np.empty((3, self.capacity), np.float64)
+        st, em, rel = np.empty(self.capacity, np.uint8), np.empty(self.capacity, np.uint32), np.empty(self.capacity, np.uint64)
+        A.check(A.lib().luw_particles_download(self._h, _ptr(xyz), _ptr(st), _ptr(em), _ptr(rel)))
+        return {"xyz": xyz.T.copy(), "state": st, "emitter": em, "release_t": rel}
+
+    def bins(self):
+        """-> (uint32 [Bz, By, Bx] counts, samples); synchronous."""
+        out = np.empty(self.bin_shape, np.uint32)
+        n = C.c_uint64()
+        A.check(A.lib().luw_particles_download_bins(self._h, _ptr(out), C.byref(n)))
+        return out, int(n.value)
+
+    def reset_bins(self):
+        A.check(A.lib().luw_particles_reset_bins(self._h))
+
+    def close(self):
+        if self._h:
+            A.lib().luw_particles_destroy(self._h)
+            self._h = C.c_void_p()
+
+
 def pinned_empty(count, dtype):
     """numpy array over page-locked host memory (luw_host_alloc). The array keeps the allocation alive through its base object."""
     dtype = np.dtype(dtype)

@@ -11,6 +11,9 @@
 //   samples u64, L u32, K u64, series[samples*L*6] f64, ref_points[3L] f64, column_labels[Nx*Ny] u32, cell[K] u64, label[K] u32, mean_F[3K], m2_F[3K] f32
 //   LUW_CASE_PROBES=x0,y0,z0,x1,y1,z1,... (global lattice points) with LUW_CASE_PROBES_OUT=<file>: LBM_Probes sampled after every step of the same window as
 //   LUW_CASE_STATS (capacity LUW_CASE_PROBES_CAP, default 256); the file gets samples u64, comps u32, P u64, t[samples] u64, values[samples*comps*P] f32
+//   LUW_CASE_PARTICLES=cx,cy,cz,hx,hy,hz,... (box emitters, lattice coordinates) with LUW_CASE_PARTICLES_ARGS=capacity,per_emitter,periodic_mask,wall_mode,seed,
+//   bx,by,bz,dt,sigma and LUW_CASE_PARTICLES_OUT=<file>: LBM_Particles over the same window as LUW_CASE_STATS, after every step emit(per_emitter), advance(dt, sigma),
+//   count(); the file gets capacity u64, xyz[3*capacity] f64, state[capacity] u8, emitter[capacity] u32, release_t[capacity] u64, samples u64, bins[Bz*By*Bx] u32
 //   with LUW_TEMPERATURE in `features`: in.bin carries T[N] f32 after u, out.bin ends with T[N] f32; alpha / beta of the LBM constructor from LUW_CASE_ALPHA / LUW_CASE_BETA
 #include "lbm.hpp"
 #include <fstream>
@@ -84,7 +87,27 @@ int main(int argc, char** argv) {
 	LBM_WallLoads* wall = wall_out ? new LBM_WallLoads(lbm, getenv("LUW_CASE_WALL_GROUND") ? (uint)atoi(getenv("LUW_CASE_WALL_GROUND")) : 0u) : nullptr;
 	const char* probes_out = getenv("LUW_CASE_PROBES_OUT");
 	LBM_Probes* probes = probes_out ? new LBM_Probes(lbm, env_list<uint>("LUW_CASE_PROBES"), getenv("LUW_CASE_PROBES_CAP") ? (uint)atoi(getenv("LUW_CASE_PROBES_CAP")) : 256u) : nullptr;
-	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) { lbm.run(1ull); if(probes) probes->sample(); stats->accumulate(); if(wind) wind->accumulate(); if(wall) wall->accumulate(); }
+	const char* particles_out = getenv("LUW_CASE_PARTICLES_OUT");
+	const std::vector<double> pargs = env_list<double>("LUW_CASE_PARTICLES_ARGS");
+	if(particles_out&&pargs.size()!=10u) print_error("LUW_CASE_PARTICLES_ARGS needs 10 values");
+	LBM_Particles* particles = particles_out ? new LBM_Particles(lbm, env_list<double>("LUW_CASE_PARTICLES"), (ulong)pargs[0], (uint)pargs[2], (uint)pargs[3], (ulong)pargs[4],
+		(uint)pargs[5], (uint)pargs[6], (uint)pargs[7]) : nullptr;
+	for(ulong k=0ull; k<(samples<steps ? samples : steps); k++) {
+		lbm.run(1ull);
+		if(probes) probes->sample();
+		if(particles) { particles->emit((uint)pargs[1]); particles->advance((float)pargs[8], pargs[9]); particles->count(); }
+		stats->accumulate(); if(wind) wind->accumulate(); if(wall) wall->accumulate();
+	}
+	if(particles) {
+		std::vector<double> xyz; std::vector<uchar> state; std::vector<uint> emitter, bins; std::vector<ulong> release_t;
+		particles->download(xyz, state, emitter, release_t);
+		const uint64_t count = (uint64_t)particles->download_bins(bins), K = (uint64_t)particles->capacity;
+		std::ofstream pf(particles_out, std::ios::binary);
+		pf.write((const char*)&K, 8); pf.write((const char*)xyz.data(), (std::streamsize)(8u*xyz.size())); pf.write((const char*)state.data(), (std::streamsize)state.size());
+		pf.write((const char*)emitter.data(), (std::streamsize)(4u*emitter.size())); pf.write((const char*)release_t.data(), (std::streamsize)(8u*release_t.size()));
+		pf.write((const char*)&count, 8); pf.write((const char*)bins.data(), (std::streamsize)(4u*bins.size()));
+		delete particles;
+	}
 	if(probes) {
 		std::vector<float> values;
 		const uint64_t count = (uint64_t)probes->series(values), P = (uint64_t)probes->points;

@@ -851,3 +851,48 @@ public:
 		return (ulong)t.size();
 	}
 };
+
+// ---------------------------------------------------------------------------------------------------------------- tracer particles
+// Lagrangian tracers of a single-domain LBM (luw_particles_*; csrc/lbm_particles.cuh): released from box emitters into a device ring, advected with the
+// velocity update_fields + a read would give at the 8 cells around each particle (t / f / omega taken from the domain as enqueue_update_fields takes them),
+// an optional uniform random walk, open faces, wall modes and concentration bins. The reference compiles its particle extension (PARTICLES) out; a decomposed
+// LBM is an error (particles crossing block faces would need a migration step). Same semantics as lbm.Particles in Python.
+class LBM_Particles {
+private:
+	LBM* lbm = nullptr;
+	luw_particles* h = nullptr;
+	const LBM_Domain* dom() const { return lbm->lbm_domain[0]; }
+public:
+	ulong capacity = 0ull;
+	uint B[3] = { 0u, 0u, 0u }; // bins per axis
+	// emitters[6e..6e+5]: centre x y z, half-extents x y z (lattice coordinates); periodic_mask bits x y z; wall_mode 0 reject, 1 deposit; bin[3] cells per bin
+	LBM_Particles(LBM& lbm_, const std::vector<double>& emitters, const ulong capacity_, const uint periodic_mask=0u, const uint wall_mode=0u, const ulong seed=0ull,
+		const uint bx=1u, const uint by=1u, const uint bz=1u) : lbm(&lbm_), capacity(capacity_) {
+		if(lbm->get_D()!=1u) print_error("LBM_Particles: needs a single domain (D = 1)");
+		const uint bin[3] = { bx, by, bz };
+		luw_check(luw_particles_create(dom()->get_handle(), capacity, (uint32_t)(emitters.size()/6u), emitters.data(), periodic_mask, wall_mode, seed, bin, &h));
+		B[0] = (lbm->get_Nx()+bx-1u)/bx; B[1] = (lbm->get_Ny()+by-1u)/by; B[2] = (lbm->get_Nz()+bz-1u)/bz;
+	}
+	~LBM_Particles() { if(h) luw_particles_destroy(h); }
+	LBM_Particles(const LBM_Particles&) = delete;
+	LBM_Particles& operator=(const LBM_Particles&) = delete;
+	void emit(const uint per_emitter) { luw_check(luw_particles_emit(h, dom()->get_t(), per_emitter)); }
+	void advance(const float dt=1.0f, const double sigma=0.0) {
+		const LBM_Domain* d = dom();
+		luw_check(luw_particles_advance(h, d->get_t(), d->get_fx(), d->get_fy(), d->get_fz(), d->get_omega_x(), d->get_omega_y(), d->get_omega_z(), dt, sigma));
+	}
+	void count() { luw_check(luw_particles_count(h)); }
+	// xyz[a*capacity + k], state[k] (0 FREE, 1 ACTIVE, 2 DEPOSITED, 3 LEFT, 4 BURIED), emitter[k], release time step[k]
+	void download(std::vector<double>& xyz, std::vector<uchar>& state, std::vector<uint>& emitter, std::vector<ulong>& release_t) {
+		xyz.resize(3ull*capacity); state.resize(capacity); emitter.resize(capacity); release_t.resize(capacity);
+		luw_check(luw_particles_download(h, xyz.data(), state.data(), emitter.data(), (uint64_t*)release_t.data()));
+	}
+	// bins[(iz*B[1] + iy)*B[0] + ix]; returns the sample count
+	ulong download_bins(std::vector<uint>& bins) {
+		bins.resize((ulong)B[0]*B[1]*B[2]);
+		uint64_t samples = 0ull;
+		luw_check(luw_particles_download_bins(h, bins.data(), &samples));
+		return (ulong)samples;
+	}
+	void reset_bins() { luw_check(luw_particles_reset_bins(h)); }
+};

@@ -20,6 +20,7 @@ from . import cases
 from .domain import CellSet, Domain, WindStats
 from .domain import WallLoads as DomainWallLoads
 from .domain import Probes as DomainProbes
+from .domain import Particles as DomainParticles
 
 AXES = (0, 1, 2)
 
@@ -515,6 +516,70 @@ class Probes:
         for pr in self._probes:
             pr.close()
 
+
+
+def particle_args(Ng, emitters, capacity, periodic, wall_mode, bins):
+    """Checks of lbm.Particles' arguments -> (emitters float64 [E, 6], periodic_mask, bins uint32 [3]); ValueError for what luw_particles_create rejects."""
+    Ng = np.asarray(Ng, np.int64)
+    em = np.asarray(emitters, np.float64).reshape(-1, 6)
+    per = [bool(v) for v in periodic]
+    b = np.asarray(bins, np.int64).reshape(-1)
+    if len(per) != 3 or b.size != 3:
+        raise ValueError("periodic and bins take one value per axis")
+    if int(capacity) < 1:
+        raise ValueError("capacity must be at least 1")
+    if int(wall_mode) not in (0, 1):
+        raise ValueError("wall_mode must be 0 (reject the move) or 1 (deposit)")
+    if (b < 1).any():
+        raise ValueError("bin sizes must be at least 1")
+    for a in range(3):
+        if not per[a] and Ng[a] < 2:
+            raise ValueError("a non-periodic axis needs at least 2 cells")
+    if not np.isfinite(em).all() or (em[:, 3:] < 0).any():
+        raise ValueError("emitter centres and half-extents must be finite, half-extents >= 0")
+    for a in range(3):
+        if not per[a] and ((em[:, a] - em[:, 3 + a] < 0) | (em[:, a] + em[:, 3 + a] > Ng[a] - 1)).any():
+            raise ValueError("emitter boxes must lie inside [0, N-1] on non-periodic axes")
+    return em, sum(1 << a for a in range(3) if per[a]), b.astype(np.uint32)
+
+
+class Particles:
+    """Lagrangian tracer particles in an in-process `LBM` of one domain (D == (1, 1, 1); a decomposed LBM raises ValueError, as particles crossing block
+    faces would need a migration step). `emitters` [E, 6]: box centre x y z and half-extents x y z in global lattice coordinates; `capacity` ring slots;
+    `periodic` one bool per axis (open faces elsewhere: a particle that leaves [0, N-1] becomes LEFT); wall_mode 0 rejects a move into a solid cell, 1 deposits
+    the particle there; `seed` keys the random numbers; `bins` cells per concentration bin and axis. Everything is stream-ordered on the domain's stream;
+    state() and bins() synchronise."""
+
+    def __init__(self, lbm, emitters, capacity, periodic=(False, False, False), wall_mode=0, seed=0, bins=(1, 1, 1)):
+        if tuple(lbm.D) != (1, 1, 1):
+            raise ValueError("lbm.Particles needs a single domain, D == (1, 1, 1)")
+        em, mask, b = particle_args(lbm.Ng, emitters, capacity, periodic, wall_mode, bins)
+        self.lbm = lbm
+        self._pt = DomainParticles(lbm.domains[0], em, int(capacity), mask, int(wall_mode), int(seed), b)
+
+    def emit(self, per_emitter):
+        self._pt.emit(per_emitter, t=self.lbm.t)
+
+    def advance(self, dt=1.0, sigma=0.0):
+        """One move with the lattice's current t, force and Coriolis."""
+        lbm, d = self.lbm, self.lbm.domains[0]
+        d.f, d.omega = lbm.f, lbm.omega
+        self._pt.advance(dt, sigma, t=lbm.t)
+
+    def count(self):
+        self._pt.count()
+
+    def state(self):
+        return self._pt.state()
+
+    def bins(self):
+        return self._pt.bins()
+
+    def reset_bins(self):
+        self._pt.reset_bins()
+
+    def close(self):
+        self._pt.close()
 
 class DistributedLBM(_Base):
     """One domain per rank (torch.distributed); rank r owns domain r of the split. Works with NCCL (GPU) and, for the host logic, with
